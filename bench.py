@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- segment-propagations/s (fp64 state + STM) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic segments.  Default
 workload (BASELINE.json configs[2]): 65,536 direct-method segments per GPU, 7-state + STM
@@ -13,6 +13,8 @@ collective (segments are independent).
 Prints ONE JSON line (rank 0).  `value` times the kernel(s) with inputs resident in HBM
 (CUDA events on the launching stream, L2 flushed between iterations); `e2e` times the
 C-ABI host-buffer call (pinned host memory, H2D + kernels + D2H inside the timed region).
+`--dump-outputs DIR` writes what the timed path returned in its last step (dump_outputs); the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -46,6 +48,7 @@ BYTES_PER_SEG = {"direct7": 1360.0, "direct6": (2 * 6 + 6 + 2 + 6 + 1 + 6 * 18) 
 WORKLOADS = ["direct7_fixed", "direct6_fixed", "direct7_adaptive", "indirect12", "indirect14", "indirect12_1m", "continuation",
              "continuation_solve"]
 SHARDED = ("indirect12_1m", "continuation")      # strong-scaling workloads: fixed total, sharded + all-gathered (lowthrustopt_b200/sharded.py)
+DUMP_BYTES = 60_000_000                          # --dump-outputs: data of all files together (the .npy headers keep it under 64 MB)
 
 
 def parse():
@@ -68,7 +71,31 @@ def parse():
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"],
                     help="sharded workloads: deliver results to the solver rank by the kernels' own stores into its HBM over NVLink "
                          "peer memory (fused, default) or by a chunked NCCL all-gather")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the arrays the timed path returned in its last step as DIR/<name>.npy (float64; "
+                         "a fixed, seeded sample of units when they exceed 60 MB)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
+    return a
+
+
+def dump_outputs(directory, arrays, seed=20180005):
+    """DIR/<name>.npy in float64 for every array the timed path returned in its last step.  Every array is indexed by unit (segment or
+    trajectory) along its first axis; when together they exceed DUMP_BYTES, the same seeded sample of units is kept of each, and the
+    sampled unit indices are written as DIR/sample_index.npy."""
+    host = {k: (v.cpu().numpy() if hasattr(v, "cpu") else np.asarray(v)).astype(np.float64) for k, v in arrays.items()}
+    n = len(next(iter(host.values())))
+    if sum(a.nbytes for a in host.values()) > DUMP_BYTES:
+        per_unit = sum(a[0].nbytes for a in host.values()) + 8
+        keep = np.sort(np.random.default_rng(seed).choice(n, DUMP_BYTES // per_unit, replace=False))
+        host = {k: a[keep] for k, a in host.items()}
+        host["sample_index"] = keep.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(directory, k + ".npy"), a)
 
 
 def make_batch(workload, n_seg, rank):
@@ -489,6 +516,8 @@ def run_sharded(args):
     if world > 1:
         dist.all_reduce(t_total, op=dist.ReduceOp.MAX)
     ms_per_step = float(t_total.item()) / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     if peer:
         # the dominant kernel alone: this rank's STM launch into its own (local) scratch, CUDA events on the library stream
         u0, u1 = sh.pg.slab()
@@ -735,6 +764,8 @@ def run_solve(args):
         dev_ms += h.last_kernel_ms
     wall = time.perf_counter() - t0
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r)
     launches = h.launches - l0
     tm = torch.tensor([dev_ms, wall * 1e3], dtype=torch.float64, device=dev)
     if world > 1:
@@ -925,6 +956,9 @@ def run_ours(args):
         dist.all_reduce(t_total, op=dist.ReduceOp.MAX)
     ms_per_step = float(t_total.item()) / args.steps
     value = n_seg * world / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(defect=d_def, errors=d_err, status=d_st, jac=d_jac) if direct else
+                     dict(defect=d_def, status=d_st, nsteps=d_ns, phi=d_phi))
     if not direct:
         nst = d_ns.cpu().numpy()
         attempted = float(nst[:, 1].mean()); accepted = float(nst[:, 0].mean())
@@ -1039,7 +1073,7 @@ def run_single_process(args):
     n_seg = (args.n_seg or (65536 if direct else 131072)) * n_dev         # weak scaling, like the multi-process default
     batch = make_batch(wl, n_seg, 0)
     res = {}
-    for devs in ([0], list(range(n_dev))):
+    for last, devs in ((False, [0]), (True, list(range(n_dev)))):
         h = capi.Handle(devs)
         pin_in = {k: capi.PinnedBuffer(v.shape) for k, v in batch.items()}
         for k, v in batch.items():
@@ -1066,6 +1100,8 @@ def run_single_process(args):
         for _ in range(args.steps):
             r = call()
         dt = time.perf_counter() - t0
+        if args.dump_outputs and last:
+            dump_outputs(args.dump_outputs, r)
         res[len(devs)] = {"value": n_seg * args.steps / dt, "ms_per_step": 1e3 * dt / args.steps, "launches": int(h.launches - l0),
                           "checksum": float(np.asarray(r["defect"]).sum())}
         h.close()

@@ -175,13 +175,12 @@ h.close()
 def test_k3_experimental_layouts_match_default(layout, lto, oracle, tmp_path):
     """The two round-2 rebuilds of K3 that were measured and not adopted (DESIGN.md section 4: hc = second-order half-column formulation with
     setmaxnreg and three tiles; wl = warp-local, every warp owns 8 slots) live in tools/experiments/ and are NOT in the product library; a library
-    built by tools/experiments/build_variant.sh contains them.  Each runs in a child process (the layout is selected once per process) and is held
-    to the same bars against the oracle as the default K3, and to 1e-10 against the default K3."""
+    built by build.build_experiments() (tools/experiments/lib/liblto_k3x.so, made by build()) contains them.  Each runs in a child process (the
+    layout is selected once per process) and is held to the same bars against the oracle as the default K3, and to 1e-10 against the default K3."""
     import subprocess
     import sys
-    xlib = os.path.join(ROOT, "tools", "experiments", "lib", "liblto_k3x.so")
-    if not os.path.exists(xlib):
-        pytest.skip("tools/experiments/lib/liblto_k3x.so not built (bash tools/experiments/build_variant.sh k3x)")
+    from lowthrustopt_b200 import build
+    xlib = build.build_experiments()
     laws = LAWS[:3]
     f = str(tmp_path / "hc.npz")
     env = dict(os.environ, LTO_K3=layout, LTO_B200_LIB=xlib)
