@@ -230,6 +230,27 @@ int lto_indirect_solve_batch(lto_handle* h, const lto_indirect_params* p, int64_
                              const double* thrustLimit_traj, const double* rho_traj,
                              double* defect, int32_t* status_flag, int32_t* iters, double* er_out);
 
+/* The same four entry points for either system, ndim = 12 or 14 (anything else: LTO_ERR_ARG).  Every "12" above becomes ndim:
+ * phi ndim x ndim column-major per segment, defect ndim x (n_nodes-1), xc_update / XC_all ndim x n_nodes per trajectory.  The
+ * functions above are these with ndim = 12.
+ *   ndim = 12  [r v | lr lv]: the end pins of :141-142 / :324-325 -- r, v (components 0..5) of the first and of the last node.
+ *   ndim = 14  [r v m | lr lv lm] (the 14-dim system of lto_indirect_dev, p->Isp / p->g0 in the mass flow):
+ *              first node r, v, m (components 0..6); last node r, v, lm (components 0..5 and 13).  The final mass is free and is
+ *              solved for; lm, which enters no right-hand side, is held by its end value (otherwise the band is rank deficient).
+ *              flag_adjointsOnly: the unknowns are the costates (7..13) of nodes 0..n_nodes-2 and m, lr, lv (6..12) of the last node.
+ * Pinned components get exact-zero updates, so the batched solver leaves them bit-identical to the input ("the end states cannot
+ * have moved").  A resolve must match the factorisation the handle holds in shape, mode AND ndim, or it is refused (LTO_ERR_ARG). */
+int lto_indirect_newton_nd(lto_handle* h, int ndim, int64_t n_traj, int n_nodes, int flag_adjointsOnly,
+                           const double* phi, const double* defect, double* xc_update, int32_t* status);
+int lto_indirect_newton_nd_dev(lto_handle* h, int ndim, int64_t n_traj, int n_nodes, int flag_adjointsOnly,
+                               const double* phi, const double* defect, double* xc_update, int32_t* status);
+int lto_indirect_newton_resolve_nd_dev(lto_handle* h, int ndim, int64_t n_traj, int n_nodes, int flag_adjointsOnly,
+                                       const double* defect, double* xc_update, int32_t* status);
+int lto_indirect_solve_batch_nd(lto_handle* h, const lto_indirect_params* p, int ndim, int64_t n_traj, int n_nodes, int max_iter,
+                                int flag_adjointsOnly, double* XC_all, const double* t_TU,
+                                const double* thrustLimit_traj, const double* rho_traj,
+                                double* defect, int32_t* status_flag, int32_t* iters, double* er_out);
+
 /* ---- the linear subproblem of the direct solver (device-side; SURVEY 8(f) row 4) ------------------------
  * lto_direct_qp: optimizeTraj of src/multiShoot_CRTBP_direct.jl:248-403 in the setting the demo runs (flagEnd = false,
  * allowImpulsive = false): with tf_jump, p1_jump, p2_jump and the dV jumps pinned by their bounds (:288-302) the JuMP / Ipopt model is

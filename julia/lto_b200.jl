@@ -124,7 +124,8 @@ function densify(XC_all::Matrix{Float64}, t_TU::Vector{Float64}, params, n_desir
 end
 
 # ---- indirect: the linear step of optimizeTraj_OLS (multiShoot_CRTBP_indirect.jl:181-182, :207) on the device.
-# `phi` is what jacobianCalc_blocks returns (m x m x (n_nodes-1)); Jac_full is never formed.
+# `phi` is what jacobianCalc_blocks returns (m x m x (n_nodes-1)); Jac_full is never formed.  m = 12, or 14 for the system with mass
+# ([r v m | lr lv lm]; end pins r, v, m first / r, v, lm last, see lto_b200.h): the dimension is taken from the arrays.
 function jacobianCalc_blocks(XC_all, t_TU, nstate, n_nodes, params)
     m = 2 * nstate; defect = pinned_array(Float64, m, n_nodes - 1); status = pinned_array(Int32, n_nodes - 1); phi = pinned_array(Float64, m, m, n_nodes - 1)
     GC.@preserve XC_all t_TU defect status phi check(ccall((:lto_indirect_defect_jac_traj, lib), Cint,
@@ -133,24 +134,27 @@ function jacobianCalc_blocks(XC_all, t_TU, nstate, n_nodes, params)
     phi
 end
 function newtonUpdate(phi::Array{Float64,3}, defect::Matrix{Float64}, n_nodes, flag_adjointsOnly::Bool)
-    xc_update = zeros(12, n_nodes); status = zeros(Int32, 1)              # == reshape(xc_update2, 2*nstate, n_nodes) (:185)
-    GC.@preserve phi defect xc_update status check(ccall((:lto_indirect_newton, lib), Cint,
-        (Ptr{Cvoid}, Int64, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
-        handle[], 1, n_nodes, flag_adjointsOnly ? 1 : 0, phi, defect, xc_update, status))
+    m = size(phi, 1)
+    (size(phi) == (m, m, n_nodes - 1) && size(defect) == (m, n_nodes - 1)) || throw(ArgumentError("phi must be m x m x (n_nodes-1), defect m x (n_nodes-1)"))
+    xc_update = zeros(m, n_nodes); status = zeros(Int32, 1)               # == reshape(xc_update2, 2*nstate, n_nodes) (:185)
+    GC.@preserve phi defect xc_update status check(ccall((:lto_indirect_newton_nd, lib), Cint,
+        (Ptr{Cvoid}, Cint, Int64, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+        handle[], m, 1, n_nodes, flag_adjointsOnly ? 1 : 0, phi, defect, xc_update, status))
     xc_update
 end
 
 # ---- indirect: multiShoot_CRTBP_indirect (:58-345) for a BATCH of trajectories, iterated on the device.
-# XC_batch: 12 x n_nodes x n_traj, t_batch: n_nodes x n_traj; thrustLimit / rho: per-trajectory vectors (continuation ladders).
+# XC_batch: m x n_nodes x n_traj (m = 12, or 14 with mass: Isp enters its mass flow), t_batch: n_nodes x n_traj; thrustLimit / rho:
+# per-trajectory vectors (continuation ladders).
 function multiShoot_CRTBP_indirect_batch(XC_batch::Array{Float64,3}, t_batch::Matrix{Float64}, MU, DU, TU, mass0, thrustLimit::Vector{Float64},
-                                         flag_adjointsOnly::Bool, maxIter, p, rho::Vector{Float64})
-    n_nodes = size(XC_batch, 2); n_traj = size(XC_batch, 3)
-    XC = copy(XC_batch); defect = zeros(12, n_nodes - 1, n_traj)
+                                         flag_adjointsOnly::Bool, maxIter, p, rho::Vector{Float64}; Isp = 2000.0)
+    m = size(XC_batch, 1); n_nodes = size(XC_batch, 2); n_traj = size(XC_batch, 3)
+    XC = copy(XC_batch); defect = zeros(m, n_nodes - 1, n_traj)
     status_flag = zeros(Int32, n_traj); iters = zeros(Int32, n_traj); er = zeros(n_traj)
-    prm = iparams((MU, DU, TU, thrustLimit[1], mass0, 1.0, p, rho[1]))
-    GC.@preserve XC t_batch thrustLimit rho defect status_flag iters er check(ccall((:lto_indirect_solve_batch, lib), Cint,
-        (Ptr{Cvoid}, Ref{IndirectParams}, Int64, Cint, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}),
-        handle[], prm, n_traj, n_nodes, maxIter, flag_adjointsOnly ? 1 : 0, XC, t_batch, thrustLimit, rho, defect, status_flag, iters, er))
+    prm = iparams((MU, DU, TU, thrustLimit[1], mass0, 1.0, p, rho[1])); prm.Isp = Isp
+    GC.@preserve XC t_batch thrustLimit rho defect status_flag iters er check(ccall((:lto_indirect_solve_batch_nd, lib), Cint,
+        (Ptr{Cvoid}, Ref{IndirectParams}, Cint, Int64, Cint, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}),
+        handle[], prm, m, n_traj, n_nodes, maxIter, flag_adjointsOnly ? 1 : 0, XC, t_batch, thrustLimit, rho, defect, status_flag, iters, er))
     (XC, defect, status_flag)
 end
 # ---- direct: multiShoot_CRTBP_direct (:465-594) for a BATCH of trajectories, iterated on the device (flagEnd = false, allowImpulsive = false).

@@ -31,6 +31,7 @@ EXPORTS = [
     "lto_direct_dev", "lto_indirect_dev", "lto_sumsq_dev", "lto_dev_alloc", "lto_dev_free", "lto_ipc_export", "lto_ipc_open", "lto_ipc_close",
     "lto_push_async", "lto_sync_copies", "lto_signal_dev", "lto_wait_dev", "lto_fp64_peak_probe", "lto_debug_profile",
     "lto_indirect_newton", "lto_indirect_newton_dev", "lto_indirect_newton_resolve_dev", "lto_indirect_solve_batch", "lto_direct_qp", "lto_direct_qp_dev", "lto_direct_solve_batch",
+    "lto_indirect_newton_nd", "lto_indirect_newton_nd_dev", "lto_indirect_newton_resolve_nd_dev", "lto_indirect_solve_batch_nd",
 ]
 
 
@@ -107,6 +108,10 @@ def lib():
         L.lto_indirect_newton_dev.argtypes = [vp, i64, ci, ci] + [vp] * 4
         L.lto_indirect_newton_resolve_dev.argtypes = [vp, i64, ci, ci] + [vp] * 3
         L.lto_indirect_solve_batch.argtypes = [vp, vp, i64, ci, ci, ci] + [vp] * 8
+        L.lto_indirect_newton_nd.argtypes = [vp, ci, i64, ci, ci] + [vp] * 4
+        L.lto_indirect_newton_nd_dev.argtypes = [vp, ci, i64, ci, ci] + [vp] * 4
+        L.lto_indirect_newton_resolve_nd_dev.argtypes = [vp, ci, i64, ci, ci] + [vp] * 3
+        L.lto_indirect_solve_batch_nd.argtypes = [vp, vp, ci, i64, ci, ci, ci] + [vp] * 8
         L.lto_direct_qp.argtypes = [vp, i64, ci, ci] + [vp] * 9
         L.lto_direct_qp_dev.argtypes = [vp, i64, ci, ci] + [vp] * 9
         L.lto_direct_solve_batch.argtypes = [vp, vp, i64, ci, ci, ci, ci] + [vp] * 5 + [C.c_double] + [vp] * 3
@@ -487,32 +492,37 @@ class Handle:
     # ---- Newton update / batched solver of the indirect method (device side) ----
     def indirect_newton(self, phi, defect, flag_adjointsOnly=False):
         """xc_update = -sparse(Jac_full) \\ defect_vec (multiShoot_CRTBP_indirect.jl:181-182) for a batch of trajectories.
-        phi: (n_traj, n_nodes-1, 12, 12) column-major blocks as the propagation returns them ([.., col, row]);
-        defect: (n_traj, n_nodes-1, 12).  Returns (xc_update (n_traj, n_nodes, 12), status (n_traj,))."""
+        phi: (n_traj, n_nodes-1, m, m) column-major blocks as the propagation returns them ([.., col, row]), m = 12 or 14 (the
+        14-dim system with mass; end pins in include/lto_b200.h); defect: (n_traj, n_nodes-1, m).
+        Returns (xc_update (n_traj, n_nodes, m), status (n_traj,))."""
         phi, defect = _f64(phi), _f64(defect)
         if phi.ndim == 3:
             phi, defect = phi[None], defect[None]
+        if phi.ndim != 4:
+            raise ValueError("phi must be (n_traj, n_nodes-1, m, m) with m = 12 or 14")
         n_traj, nseg, m, m2 = phi.shape
-        if m != 12 or m2 != 12 or defect.shape != (n_traj, nseg, 12):
-            raise ValueError("phi must be (n_traj, n_nodes-1, 12, 12) and defect (n_traj, n_nodes-1, 12)")
-        upd = np.empty((n_traj, nseg + 1, 12)); status = np.empty(n_traj, dtype=np.int32)
-        self._ck(lib().lto_indirect_newton(self._h, n_traj, nseg + 1, int(bool(flag_adjointsOnly)), _ptr(phi), _ptr(defect), _ptr(upd),
-                                           _ptr(status)))
+        if m not in (12, 14) or m2 != m or defect.shape != (n_traj, nseg, m):
+            raise ValueError("phi must be (n_traj, n_nodes-1, m, m) and defect (n_traj, n_nodes-1, m) with m = 12 or 14 "
+                             "(got phi %s, defect %s)" % (phi.shape, defect.shape))
+        upd = np.empty((n_traj, nseg + 1, m)); status = np.empty(n_traj, dtype=np.int32)
+        self._ck(lib().lto_indirect_newton_nd(self._h, m, n_traj, nseg + 1, int(bool(flag_adjointsOnly)), _ptr(phi), _ptr(defect), _ptr(upd),
+                                              _ptr(status)))
         return upd, status
 
-    def indirect_newton_dev(self, n_traj, n_nodes, flag_adjointsOnly, phi, defect, xc_update, status=None):
-        self._ck(lib().lto_indirect_newton_dev(self._h, int(n_traj), int(n_nodes), int(bool(flag_adjointsOnly)), _ptr(phi), _ptr(defect),
-                                               _ptr(xc_update), _ptr(status)))
+    def indirect_newton_dev(self, n_traj, n_nodes, flag_adjointsOnly, phi, defect, xc_update, status=None, ndim=12):
+        self._ck(lib().lto_indirect_newton_nd_dev(self._h, int(ndim), int(n_traj), int(n_nodes), int(bool(flag_adjointsOnly)), _ptr(phi),
+                                                  _ptr(defect), _ptr(xc_update), _ptr(status)))
 
-    def indirect_newton_resolve_dev(self, n_traj, n_nodes, flag_adjointsOnly, defect, xc_update, status=None):
-        """Same matrix as the preceding indirect_newton_dev call, new defects (the second-order correction, :207)."""
-        self._ck(lib().lto_indirect_newton_resolve_dev(self._h, int(n_traj), int(n_nodes), int(bool(flag_adjointsOnly)), _ptr(defect),
-                                                       _ptr(xc_update), _ptr(status)))
+    def indirect_newton_resolve_dev(self, n_traj, n_nodes, flag_adjointsOnly, defect, xc_update, status=None, ndim=12):
+        """Same matrix as the preceding indirect_newton_dev call (same shape, mode and ndim), new defects (the second-order correction, :207)."""
+        self._ck(lib().lto_indirect_newton_resolve_nd_dev(self._h, int(ndim), int(n_traj), int(n_nodes), int(bool(flag_adjointsOnly)),
+                                                          _ptr(defect), _ptr(xc_update), _ptr(status)))
 
     def indirect_solve_batch(self, XC_all, t_TU, params=None, thrustLimit=None, rho=None, max_iter=50, flag_adjointsOnly=False, inplace=False,
                              out=None):
         """multiShoot_CRTBP_indirect (:58-345) for n_traj trajectories at once, iterated on the device.
-        XC_all: (n_traj, n_nodes, 12); t_TU: (n_traj, n_nodes).  Returns dict(XC_all, defect, status_flag, iters, er).
+        XC_all: (n_traj, n_nodes, m), m = 12 (the reference's system) or 14 ([r v m | lr lv lm], params.Isp in the mass flow; end pins
+        in include/lto_b200.h); t_TU: (n_traj, n_nodes).  Returns dict(XC_all, defect, status_flag, iters, er).
         inplace: work directly on XC_all (must be a C-contiguous float64 array, e.g. pinned) as the C entry point does;
         out: optional preallocated arrays under the keys defect / status_flag / iters / er."""
         p = params or indirect_params()
@@ -526,8 +536,8 @@ class Handle:
         if XC.ndim == 2:
             XC, t_TU = XC[None], t_TU[None]
         n_traj, n_nodes, nd = XC.shape
-        if nd != 12:
-            raise ValueError("the reference's indirect solver is 12-dimensional (multiShoot_CRTBP_indirect.jl:258)")
+        if nd not in (12, 14):
+            raise ValueError("XC_all must have 12 (the reference's system, multiShoot_CRTBP_indirect.jl:258) or 14 columns (got %d)" % nd)
         t_TU = _shaped("t_TU", t_TU, (n_traj, n_nodes))
         tl = _per_unit("thrustLimit", thrustLimit, n_traj)
         rh = _per_unit("rho", rho, n_traj)
@@ -536,8 +546,8 @@ class Handle:
         flag = _out(o, "status_flag", (n_traj,), np.int32)
         iters = _out(o, "iters", (n_traj,), np.int32)
         er = _out(o, "er", (n_traj,))
-        self._ck(lib().lto_indirect_solve_batch(self._h, C.addressof(p), n_traj, n_nodes, int(max_iter), int(bool(flag_adjointsOnly)),
-                                                _ptr(XC), _ptr(t_TU), _ptr(tl), _ptr(rh), _ptr(defect), _ptr(flag), _ptr(iters), _ptr(er)))
+        self._ck(lib().lto_indirect_solve_batch_nd(self._h, C.addressof(p), nd, n_traj, n_nodes, int(max_iter), int(bool(flag_adjointsOnly)),
+                                                   _ptr(XC), _ptr(t_TU), _ptr(tl), _ptr(rh), _ptr(defect), _ptr(flag), _ptr(iters), _ptr(er)))
         return dict(XC_all=XC, defect=defect, status_flag=flag, iters=iters, er=er)
 
     # ---- direct method: the QP of optimizeTraj on the device ----

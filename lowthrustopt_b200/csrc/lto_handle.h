@@ -24,6 +24,7 @@ struct lto_handle {
     unsigned long long* d_prof;                 // LTO_ICW_PROF=1: per-warp cycle counters of the last indirect throughput launch
     void* d_nwt; size_t d_nwt_cap;              // factor workspace of the Newton update (lto_newton.cu)
     long long nwt_traj; int nwt_nodes, nwt_adj;  // shape / mode of the factorisation it holds (0 trajectories: none)
+    int nwt_ndim;                               // and its system dimension (12 or 14)
     void* d_slv; size_t d_slv_cap;              // arrays of the batched solver (lto_solve.cu)
     int64_t launches;
     double last_ms;

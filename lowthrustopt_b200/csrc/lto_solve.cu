@@ -9,6 +9,7 @@
 //                               order correction (:187-214), 20-point line search (:221-246), end-state pins (:324-325),
 //                               defect check (:328-336).  Per iteration the host reads back ONE integer (how many
 //                               trajectories are still iterating).
+//   The *_nd forms take the system dimension (12: the reference's system; 14: with mass, see lto_b200.h); the others are ndim = 12.
 // Built on the public device-pointer entry points (lto_indirect_dev, lto_sumsq_dev) and a few row-wise helper kernels.
 #include "lto_internal.h"
 #include "lto_handle.h"
@@ -18,11 +19,11 @@
 #include <vector>
 
 namespace lto {
-size_t indirect_newton_workspace_bytes(long long n_traj, int n_nodes);
+size_t indirect_newton_workspace_bytes(long long n_traj, int n_nodes, int ndim);
 cudaError_t launch_indirect_newton(const double* phi, const double* defect, double* work, double* update, int32_t* status,
-                                   long long n_traj, int n_nodes, bool adjoints_only, cudaStream_t st);
+                                   long long n_traj, int n_nodes, int ndim, bool adjoints_only, cudaStream_t st);
 cudaError_t launch_indirect_newton_resolve(const double* defect, double* work, double* update, int32_t* status, long long n_traj, int n_nodes,
-                                           bool adjoints_only, cudaStream_t st);
+                                           int ndim, bool adjoints_only, cudaStream_t st);
 
 size_t direct_qp_workspace_bytes(long long n_traj, int n_nodes, int nstate);
 cudaError_t launch_direct_qp(const double* jac, const double* defect, const double* X_all, const double* u_all, const double* t,
@@ -203,11 +204,14 @@ static int split_trajectories(lto_handle* h, long long n_traj, F&& call) {
 
 extern "C" {
 
-int lto_indirect_newton_dev(lto_handle* h, int64_t n_traj, int n_nodes, int flag_adjointsOnly, const double* phi,
-                            const double* defect, double* xc_update, int32_t* status) {
+static inline bool valid_ndim(int ndim) { return ndim == 12 || ndim == 14; }
+
+int lto_indirect_newton_nd_dev(lto_handle* h, int ndim, int64_t n_traj, int n_nodes, int flag_adjointsOnly, const double* phi,
+                               const double* defect, double* xc_update, int32_t* status) {
     LTO_NVTX();
     if (!h) return fail(nullptr, LTO_ERR_ARG, "null handle");
     if (h->n_child > 0) return fail(h, LTO_ERR_ARG, "device-pointer entry points need a single-device handle (lto_init)");
+    if (!valid_ndim(ndim)) return fail(h, LTO_ERR_ARG, "ndim must be 12 or 14 (got %d)", ndim);
     if (n_traj < 0) return fail(h, LTO_ERR_ARG, "negative trajectory count");
     if (n_nodes < 2) return fail(h, LTO_ERR_ARG, "n_nodes must be >= 2");
     if (n_traj == 0) return LTO_SUCCESS;
@@ -215,62 +219,83 @@ int lto_indirect_newton_dev(lto_handle* h, int64_t n_traj, int n_nodes, int flag
     if (((uintptr_t)phi & 15u) != 0) return fail(h, LTO_ERR_ARG, "phi must be 16-byte aligned");
     CK(h, cudaSetDevice(h->device));
     h->nwt_traj = 0;
-    int rc = ensure(h, &h->d_nwt, &h->d_nwt_cap, indirect_newton_workspace_bytes(n_traj, n_nodes)); if (rc) return rc;
-    cudaError_t e = launch_indirect_newton(phi, defect, (double*)h->d_nwt, xc_update, status, n_traj, n_nodes, flag_adjointsOnly != 0, h->s_compute);
+    int rc = ensure(h, &h->d_nwt, &h->d_nwt_cap, indirect_newton_workspace_bytes(n_traj, n_nodes, ndim)); if (rc) return rc;
+    cudaError_t e = launch_indirect_newton(phi, defect, (double*)h->d_nwt, xc_update, status, n_traj, n_nodes, ndim, flag_adjointsOnly != 0,
+                                           h->s_compute);
     if (e != cudaSuccess) return fail(h, LTO_ERR_CUDA, "newton kernel launch: %s", cudaGetErrorString(e));
     h->launches += 1;
-    h->nwt_traj = n_traj; h->nwt_nodes = n_nodes; h->nwt_adj = flag_adjointsOnly != 0;
+    h->nwt_traj = n_traj; h->nwt_nodes = n_nodes; h->nwt_adj = flag_adjointsOnly != 0; h->nwt_ndim = ndim;
     return LTO_SUCCESS;
 }
 
-int lto_indirect_newton_resolve_dev(lto_handle* h, int64_t n_traj, int n_nodes, int flag_adjointsOnly, const double* defect,
-                                    double* xc_update, int32_t* status) {
+int lto_indirect_newton_dev(lto_handle* h, int64_t n_traj, int n_nodes, int flag_adjointsOnly, const double* phi,
+                            const double* defect, double* xc_update, int32_t* status) {
+    return lto_indirect_newton_nd_dev(h, 12, n_traj, n_nodes, flag_adjointsOnly, phi, defect, xc_update, status);
+}
+
+int lto_indirect_newton_resolve_nd_dev(lto_handle* h, int ndim, int64_t n_traj, int n_nodes, int flag_adjointsOnly, const double* defect,
+                                       double* xc_update, int32_t* status) {
     LTO_NVTX();
     if (!h) return fail(nullptr, LTO_ERR_ARG, "null handle");
     if (h->n_child > 0) return fail(h, LTO_ERR_ARG, "device-pointer entry points need a single-device handle (lto_init)");
+    if (!valid_ndim(ndim)) return fail(h, LTO_ERR_ARG, "ndim must be 12 or 14 (got %d)", ndim);
     if (n_traj == 0) return LTO_SUCCESS;
     if (!defect || !xc_update) return fail(h, LTO_ERR_ARG, "null array argument");
-    if (h->nwt_traj != n_traj || h->nwt_nodes != n_nodes || h->nwt_adj != (flag_adjointsOnly != 0) || !h->d_nwt)
-        return fail(h, LTO_ERR_ARG, "lto_indirect_newton_resolve_dev: no factorisation of this shape and mode is held (call lto_indirect_newton_dev first)");
+    if (h->nwt_traj != n_traj || h->nwt_nodes != n_nodes || h->nwt_adj != (flag_adjointsOnly != 0) || h->nwt_ndim != ndim || !h->d_nwt)
+        return fail(h, LTO_ERR_ARG, "lto_indirect_newton_resolve_dev: no factorisation of this shape, dimension and mode is held "
+                                    "(call lto_indirect_newton_dev first)");
     if (((uintptr_t)defect & 15u) != 0) return fail(h, LTO_ERR_ARG, "defect must be 16-byte aligned");
     CK(h, cudaSetDevice(h->device));
-    cudaError_t e = launch_indirect_newton_resolve(defect, (double*)h->d_nwt, xc_update, status, n_traj, n_nodes, flag_adjointsOnly != 0, h->s_compute);
+    cudaError_t e = launch_indirect_newton_resolve(defect, (double*)h->d_nwt, xc_update, status, n_traj, n_nodes, ndim, flag_adjointsOnly != 0,
+                                                   h->s_compute);
     if (e != cudaSuccess) return fail(h, LTO_ERR_CUDA, "newton resolve kernel launch: %s", cudaGetErrorString(e));
     h->launches += 1;
     return LTO_SUCCESS;
 }
 
-int lto_indirect_newton(lto_handle* h, int64_t n_traj, int n_nodes, int flag_adjointsOnly, const double* phi,
-                        const double* defect, double* xc_update, int32_t* status) {
+int lto_indirect_newton_resolve_dev(lto_handle* h, int64_t n_traj, int n_nodes, int flag_adjointsOnly, const double* defect,
+                                    double* xc_update, int32_t* status) {
+    return lto_indirect_newton_resolve_nd_dev(h, 12, n_traj, n_nodes, flag_adjointsOnly, defect, xc_update, status);
+}
+
+int lto_indirect_newton_nd(lto_handle* h, int ndim, int64_t n_traj, int n_nodes, int flag_adjointsOnly, const double* phi,
+                           const double* defect, double* xc_update, int32_t* status) {
     LTO_NVTX();
     if (!h) return fail(nullptr, LTO_ERR_ARG, "null handle");
+    if (!valid_ndim(ndim)) return fail(h, LTO_ERR_ARG, "ndim must be 12 or 14 (got %d)", ndim);
     if (n_traj < 0) return fail(h, LTO_ERR_ARG, "negative trajectory count");
     if (n_nodes < 2) return fail(h, LTO_ERR_ARG, "n_nodes must be >= 2");
     if (n_traj == 0) return LTO_SUCCESS;
     if (!phi || !defect || !xc_update) return fail(h, LTO_ERR_ARG, "null array argument");
+    const long long ND = ndim;
     if (h->n_child > 0) {
         const long long N = n_nodes;
         return split_trajectories(h, n_traj, [&](lto_handle* c, long long u0, long long nu) {
-            return lto_indirect_newton(c, nu, n_nodes, flag_adjointsOnly, phi + u0 * (N - 1) * 144, defect + u0 * (N - 1) * 12, xc_update + u0 * N * 12,
-                                       status ? status + u0 : nullptr);
+            return lto_indirect_newton_nd(c, ndim, nu, n_nodes, flag_adjointsOnly, phi + u0 * (N - 1) * ND * ND, defect + u0 * (N - 1) * ND,
+                                          xc_update + u0 * N * ND, status ? status + u0 : nullptr);
         });
     }
     CK(h, cudaSetDevice(h->device));
     const long long ns = n_traj * (long long)(n_nodes - 1), nn = n_traj * (long long)n_nodes;
-    const size_t bP = al(ns * 144 * 8), bD = al(ns * 12 * 8), bU = al(nn * 12 * 8), bS = al(n_traj * 4);
+    const size_t bP = al(ns * ND * ND * 8), bD = al(ns * ND * 8), bU = al(nn * ND * 8), bS = al(n_traj * 4);
     int rc = ensure(h, &h->d_out, &h->d_out_cap, bP + bD + bU + bS); if (rc) return rc;
     char* q = (char*)h->d_out;
     double* dP = (double*)q; q += bP; double* dD = (double*)q; q += bD; double* dU = (double*)q; q += bU; int32_t* dS = (int32_t*)q;
-    CK(h, cudaMemcpyAsync(dP, phi, ns * 144 * 8, cudaMemcpyHostToDevice, h->s_compute));
-    CK(h, cudaMemcpyAsync(dD, defect, ns * 12 * 8, cudaMemcpyHostToDevice, h->s_compute));
+    CK(h, cudaMemcpyAsync(dP, phi, ns * ND * ND * 8, cudaMemcpyHostToDevice, h->s_compute));
+    CK(h, cudaMemcpyAsync(dD, defect, ns * ND * 8, cudaMemcpyHostToDevice, h->s_compute));
     CK(h, cudaEventRecord(h->ev_t0, h->s_compute));
-    rc = lto_indirect_newton_dev(h, n_traj, n_nodes, flag_adjointsOnly, dP, dD, dU, dS); if (rc) return rc;
+    rc = lto_indirect_newton_nd_dev(h, ndim, n_traj, n_nodes, flag_adjointsOnly, dP, dD, dU, dS); if (rc) return rc;
     CK(h, cudaEventRecord(h->ev_t1, h->s_compute));
-    CK(h, cudaMemcpyAsync(xc_update, dU, nn * 12 * 8, cudaMemcpyDeviceToHost, h->s_compute));
+    CK(h, cudaMemcpyAsync(xc_update, dU, nn * ND * 8, cudaMemcpyDeviceToHost, h->s_compute));
     if (status) CK(h, cudaMemcpyAsync(status, dS, n_traj * 4, cudaMemcpyDeviceToHost, h->s_compute));
     CK(h, cudaStreamSynchronize(h->s_compute));
     float ms = 0.f; CK(h, cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1)); h->last_ms = ms;
     return LTO_SUCCESS;
+}
+
+int lto_indirect_newton(lto_handle* h, int64_t n_traj, int n_nodes, int flag_adjointsOnly, const double* phi,
+                        const double* defect, double* xc_update, int32_t* status) {
+    return lto_indirect_newton_nd(h, 12, n_traj, n_nodes, flag_adjointsOnly, phi, defect, xc_update, status);
 }
 
 // ---- direct method: the QP of optimizeTraj (multiShoot_CRTBP_direct.jl:248-403, flagEnd = false, allowImpulsive = false) ----
@@ -486,12 +511,13 @@ int lto_direct_solve_batch(lto_handle* h, const lto_direct_params* p, int64_t n_
     return LTO_SUCCESS;
 }
 
-int lto_indirect_solve_batch(lto_handle* h, const lto_indirect_params* p, int64_t n_traj, int n_nodes, int max_iter,
-                             int flag_adjointsOnly, double* XC_all, const double* t_TU, const double* thrustLimit_traj,
-                             const double* rho_traj, double* defect, int32_t* status_flag, int32_t* iters, double* er_out) {
+int lto_indirect_solve_batch_nd(lto_handle* h, const lto_indirect_params* p, int ndim, int64_t n_traj, int n_nodes, int max_iter,
+                                int flag_adjointsOnly, double* XC_all, const double* t_TU, const double* thrustLimit_traj,
+                                const double* rho_traj, double* defect, int32_t* status_flag, int32_t* iters, double* er_out) {
     LTO_NVTX();
     if (!h) return fail(nullptr, LTO_ERR_ARG, "null handle");
     if (!p) return fail(h, LTO_ERR_ARG, "null params");
+    if (!valid_ndim(ndim)) return fail(h, LTO_ERR_ARG, "ndim must be 12 or 14 (got %d)", ndim);
     if (n_traj < 0) return fail(h, LTO_ERR_ARG, "negative trajectory count");
     if (n_nodes < 2) return fail(h, LTO_ERR_ARG, "n_nodes must be >= 2");
     if (max_iter < 0) return fail(h, LTO_ERR_ARG, "negative max_iter");
@@ -500,14 +526,14 @@ int lto_indirect_solve_batch(lto_handle* h, const lto_indirect_params* p, int64_
     if (h->n_child > 0) {                                                 // independent solver instances: no communication between the devices
         const long long N = n_nodes;
         return split_trajectories(h, n_traj, [&](lto_handle* c, long long u0, long long nu) {
-            return lto_indirect_solve_batch(c, p, nu, n_nodes, max_iter, flag_adjointsOnly, XC_all + u0 * N * 12, t_TU + u0 * N,
-                                            thrustLimit_traj ? thrustLimit_traj + u0 : nullptr, rho_traj ? rho_traj + u0 : nullptr,
-                                            defect ? defect + u0 * (N - 1) * 12 : nullptr, status_flag ? status_flag + u0 : nullptr,
-                                            iters ? iters + u0 : nullptr, er_out ? er_out + u0 : nullptr);
+            return lto_indirect_solve_batch_nd(c, p, ndim, nu, n_nodes, max_iter, flag_adjointsOnly, XC_all + u0 * N * ndim, t_TU + u0 * N,
+                                               thrustLimit_traj ? thrustLimit_traj + u0 : nullptr, rho_traj ? rho_traj + u0 : nullptr,
+                                               defect ? defect + u0 * (N - 1) * ndim : nullptr, status_flag ? status_flag + u0 : nullptr,
+                                               iters ? iters + u0 : nullptr, er_out ? er_out + u0 : nullptr);
         });
     }
     CK(h, cudaSetDevice(h->device));
-    const int ND = 12, N = n_nodes, NA = slv::NA;
+    const int ND = ndim, N = n_nodes, NA = slv::NA;
     const long long T = n_traj, ns = T * (N - 1), nn = T * N;
     if (T > 0x7fffffffll) return fail(h, LTO_ERR_ARG, "too many trajectories");
     const long long LX = (long long)N * ND, LD = (long long)(N - 1) * ND;      // row lengths: states / defects of one trajectory
@@ -613,13 +639,13 @@ int lto_indirect_solve_batch(lto_handle* h, const lto_indirect_params* p, int64_
         // jacobianCalc (:290): one launch, Phi_i of every segment of every trajectory still iterating (and the defects, unchanged)
         rc = lto_indirect_dev(h, p, nc * (N - 1), N, ND, dXC, dT, nullptr, nullptr, dTL, dRH, dDef, nullptr, nullptr, dPhi); if (rc) return rc;
         // optimizeTraj_OLS (:149-183)
-        rc = lto_indirect_newton_dev(h, nc, N, flag_adjointsOnly, dPhi, dDef, dUp, nullptr); if (rc) return rc;
+        rc = lto_indirect_newton_nd_dev(h, ND, nc, N, flag_adjointsOnly, dPhi, dDef, dUp, nullptr); if (rc) return rc;
         // second-order correction (:187-214), only where norm(xc_update, Inf) < 1e-1
         rowmax(dUp, nc, LX, dUmax);
         slv::k_soc_mask<<<slv::nblk(nc, 256), 256, 0, st>>>(dUmax, dActive, dMask, nc); h->launches += 1;
         axpy(dXC, dUp, dMask, dXS, nc, LX, 1);                                                 // XC_all_soc (:194)
         rc = defect_pass(dXS, dT, dTL, dRH, nc, dDs); if (rc) return rc;                       // :197
-        rc = lto_indirect_newton_resolve_dev(h, nc, N, flag_adjointsOnly, dDs, dUp2, nullptr); if (rc) return rc;   // :207 (same Jacobian: stored reflections replayed)
+        rc = lto_indirect_newton_resolve_nd_dev(h, ND, nc, N, flag_adjointsOnly, dDs, dUp2, nullptr); if (rc) return rc;   // :207 (same Jacobian: stored reflections replayed)
         axpy(dUp, dUp2, dMask, dUp, nc, LX, 1);                                                // xc_update += xc_update_soc (:213)
         // line search (:298-302)
         const int use_ls = it > 3;
@@ -631,7 +657,7 @@ int lto_indirect_solve_batch(lto_handle* h, const lto_indirect_params* p, int64_
         }
         slv::k_pick_alpha<<<slv::nblk(nc, 256), 256, 0, st>>>(dErs, dAlphaAll, dActive, dAlpha, dScale, nc, use_ls); h->launches += 1;
         axpy(dXC, dUp, dScale, dXC, nc, LX, 1);                                                // XC_all = XC_all + xc_update*alpha (:304)
-        // the end states cannot have moved (:324-325): their update entries are exact zeros (lto_newton.cu)
+        // the end states cannot have moved (:324-325): their update entries are exact zeros (lto_newton.cu; 14-dim: the 7-element pins)
         rc = defect_pass(dXC, dT, dTL, dRH, nc, dDef); if (rc) return rc;                      // :328
         rowmax(dDef, nc, LD, dEr);                                                             // :332
         rc = iter_end(it, &n_next); if (rc) return rc;
@@ -650,6 +676,13 @@ int lto_indirect_solve_batch(lto_handle* h, const lto_indirect_params* p, int64_
         for (long long j = 0; j < T; ++j) status_flag[j] = flag[(size_t)j];                    // (non-finite nodes were flagged when the row was retired)
     }
     return LTO_SUCCESS;
+}
+
+int lto_indirect_solve_batch(lto_handle* h, const lto_indirect_params* p, int64_t n_traj, int n_nodes, int max_iter,
+                             int flag_adjointsOnly, double* XC_all, const double* t_TU, const double* thrustLimit_traj,
+                             const double* rho_traj, double* defect, int32_t* status_flag, int32_t* iters, double* er_out) {
+    return lto_indirect_solve_batch_nd(h, p, 12, n_traj, n_nodes, max_iter, flag_adjointsOnly, XC_all, t_TU, thrustLimit_traj, rho_traj,
+                                       defect, status_flag, iters, er_out);
 }
 
 }  // extern "C"

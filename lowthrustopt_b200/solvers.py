@@ -412,7 +412,7 @@ def _band_indirect(phi, nstate, N):
 def multiShoot_CRTBP_indirect(XC_all, t_TU, MU, DU, TU, n_nodes, mass0, thrustLimit, plot_yn=False, flag_adjointsOnly=False,
                               maxIter=50, p=1.0, rho=1.0, backend=None, log=None, device_newton=False, Isp=2000.0):
     """(XC_all, defect, status_flag) = multiShoot_CRTBP_indirect(...)   (:58-59, :344).
-    device_newton: solve the update on the GPU (lto_indirect_newton) instead of the dense host least squares.
+    device_newton: solve the update on the GPU (lto_indirect_newton_nd, either system) instead of the dense host least squares.
 
     XC_all with 12 rows is the reference's system.  With 14 rows ([r v m | lr lv lm], BASELINE configs[1] as north_star words it) the
     same loop runs on the 14-dim system with mass: nstate = 7, the band blocks are 14 x 14, and the end pins of :324-325 become
@@ -424,8 +424,6 @@ def multiShoot_CRTBP_indirect(XC_all, t_TU, MU, DU, TU, n_nodes, mass0, thrustLi
     nstate = XC_all.shape[0] // 2; m = 2 * nstate; N = n_nodes
     if nstate not in (6, 7):
         raise ValueError("XC_all must have 12 rows (the reference's system) or 14 ([r v m | lr lv lm])")
-    if nstate == 7 and device_newton:
-        raise NotImplementedError("the device-side Newton update (lto_indirect_newton) is 12-dim; the 14-dim loop solves the update on the host")
     params = (MU, DU, TU, thrustLimit, mass0, 1.0, p, rho) + ((Isp,) if nstate == 7 else ())              # :260
     status_flag = 0
     pin0, pinf = _end_pins(nstate)
@@ -489,17 +487,20 @@ def multiShoot_CRTBP_indirect(XC_all, t_TU, MU, DU, TU, n_nodes, mass0, thrustLi
 
 
 def multiShoot_CRTBP_indirect_batch(XC_all, t_TU, MU, DU, TU, n_nodes, mass0, thrustLimit, flag_adjointsOnly=False, maxIter=50, p=1.0,
-                                    rho=1.0, backend=None):
+                                    rho=1.0, backend=None, Isp=2000.0):
     """multiShoot_CRTBP_indirect for a BATCH of independent trajectories, iterated entirely on the device
-    (lto_indirect_solve_batch).  XC_all: (n_traj, 12, n_nodes) in the reference's per-trajectory shape; t_TU: (n_traj, n_nodes);
-    thrustLimit / rho: scalars or per-trajectory arrays (continuation ladders).  Returns (XC_all, defect (n_traj, 12, n_nodes-1),
+    (lto_indirect_solve_batch_nd).  XC_all: (n_traj, m, n_nodes) in the reference's per-trajectory shape, m = 12 or 14 (the system
+    with mass, same end pins as multiShoot_CRTBP_indirect; `Isp` enters its mass flow); t_TU: (n_traj, n_nodes);
+    thrustLimit / rho: scalars or per-trajectory arrays (continuation ladders).  Returns (XC_all, defect (n_traj, m, n_nodes-1),
     status_flag (n_traj,), iters (n_traj,))."""
     be = backend or default_backend()
     XC = np.ascontiguousarray(np.asarray(XC_all, dtype=np.float64).transpose(0, 2, 1))
-    T = XC.shape[0]
+    T, _, m = XC.shape
+    if m not in (12, 14):
+        raise ValueError("XC_all must be (n_traj, 12 or 14, n_nodes) (got %s)" % (np.shape(XC_all),))
     tl = np.broadcast_to(np.asarray(thrustLimit, dtype=np.float64), (T,)).copy()
     rh = np.broadcast_to(np.asarray(rho, dtype=np.float64), (T,)).copy()
-    params = (MU, DU, TU, float(tl[0]), mass0, 1.0, p, float(rh[0]))
+    params = (MU, DU, TU, float(tl[0]), mass0, 1.0, p, float(rh[0])) + ((Isp,) if m == 14 else ())
     r = be.indirect_solve_batch(XC, np.asarray(t_TU, dtype=np.float64), params, thrustLimit=tl, rho=rh, max_iter=maxIter,
                                 flag_adjointsOnly=flag_adjointsOnly)
     return r["XC_all"].transpose(0, 2, 1).copy(), r["defect"].transpose(0, 2, 1).copy(), r["status_flag"], r["iters"]
@@ -537,13 +538,14 @@ def _reduceFuel_steps(XC_all, rho_current, rho_target, rng):
 
 
 def reduceFuel_indirect(XC_all, t_TU, MU, DU, TU, n_nodes, mass, thrustLimit, rho_current, rho_target, backend=None, rng=None,
-                        log=None):
-    """rho-continuation driver (HelperFunctions.jl:105-193).  `rng` supplies the rand() of the back-off (:182)."""
+                        log=None, Isp=2000.0):
+    """rho-continuation driver (HelperFunctions.jl:105-193).  `rng` supplies the rand() of the back-off (:182).
+    XC_all: 12 or 14 rows (multiShoot_CRTBP_indirect); `Isp` enters the mass flow of the 14-dim system."""
     gen = _reduceFuel_steps(np.array(XC_all, dtype=np.float64), rho_current, rho_target, rng or np.random.default_rng(0))
     req = next(gen)
     while True:
         XC, rho = req
-        out = multiShoot_CRTBP_indirect(XC, t_TU, MU, DU, TU, n_nodes, mass, thrustLimit, False, False, 10, 1.0, rho, backend=backend)
+        out = multiShoot_CRTBP_indirect(XC, t_TU, MU, DU, TU, n_nodes, mass, thrustLimit, False, False, 10, 1.0, rho, backend=backend, Isp=Isp)
         if log is not None:
             log.append(dict(rho=rho, status=out[2], er=float(np.max(np.abs(out[1])))))
         try:
@@ -553,12 +555,13 @@ def reduceFuel_indirect(XC_all, t_TU, MU, DU, TU, n_nodes, mass, thrustLimit, rh
 
 
 def reduceFuel_indirect_batch(XC_all, t_TU, MU, DU, TU, n_nodes, mass, thrustLimit, rho_current, rho_target, backend=None, rngs=None,
-                              log=None):
+                              log=None, Isp=2000.0):
     """reduceFuel_indirect for a BATCH of independent trajectories (SURVEY 8(f) row 3): every trajectory walks its own rho ladder
     (halving on success, x 3(1 + rand) back-off on failure, :155-187); each round, the solver calls all unfinished trajectories
     ask for are issued as ONE lto_indirect_solve_batch call with per-trajectory rho / thrustLimit.
-    XC_all: (n_traj, 12, n_nodes); t_TU: (n_traj, n_nodes); thrustLimit, rho_current, rho_target: scalars or (n_traj,).
-    Returns (XC_new (n_traj, 12, n_nodes), defect (n_traj, 12, n_nodes-1), status (n_traj,), rounds)."""
+    XC_all: (n_traj, m, n_nodes), m = 12 or 14 (`Isp` enters the mass flow of the 14-dim system); t_TU: (n_traj, n_nodes);
+    thrustLimit, rho_current, rho_target: scalars or (n_traj,).
+    Returns (XC_new (n_traj, m, n_nodes), defect (n_traj, m, n_nodes-1), status (n_traj,), rounds)."""
     be = backend or default_backend()
     XC_all = np.asarray(XC_all, dtype=np.float64); t_TU = np.asarray(t_TU, dtype=np.float64)
     T = XC_all.shape[0]
@@ -573,7 +576,8 @@ def reduceFuel_indirect_batch(XC_all, t_TU, MU, DU, TU, n_nodes, mass, thrustLim
         rounds += 1
         idx = sorted(req)
         XC = np.stack([req[j][0] for j in idx]); rho = np.array([req[j][1] for j in idx])
-        Xn, dn, st, it = multiShoot_CRTBP_indirect_batch(XC, t_TU[idx], MU, DU, TU, n_nodes, mass, tl[idx], False, 10, 1.0, rho, backend=be)
+        Xn, dn, st, it = multiShoot_CRTBP_indirect_batch(XC, t_TU[idx], MU, DU, TU, n_nodes, mass, tl[idx], False, 10, 1.0, rho, backend=be,
+                                                         Isp=Isp)
         if log is not None:
             log.append(dict(round=rounds, n=len(idx), rho=rho.copy(), status=np.asarray(st).copy()))
         for k, j in enumerate(idx):
