@@ -40,8 +40,8 @@ struct Cfg {
     static constexpr int NCOL = NS + 3;
     static constexpr int NW = NTILE + NCOL;
     static constexpr int NTHREADS = 32 * NW;
-    static constexpr int SVAL = (NS == 7) ? 10 : 6;          // U[6] (+ k/m, am[3]) per stage and leg
-    static constexpr int OFF_H = 13 * SVAL;                  // h
+    static constexpr int SVAL = (NS == 7) ? 10 : 6;          // U[6] (+ k/m, am[3]) per stage and leg, lane-contiguous (128-bit accesses)
+    static constexpr int OFF_H = 13 * SVAL;                  // h (lane-strided, as bm)
     static constexpr int OFF_BM = OFF_H + 1;                 // bm[3] (nstate 7)
     static constexpr int STEP_DOUBLES = OFF_BM + ((NS == 7) ? 3 : 0);
     static constexpr size_t REC_BYTES = (size_t)NTILE * NSLOT * STEP_DOUBLES * 32 * sizeof(double);
@@ -50,18 +50,54 @@ struct Cfg {
     static constexpr size_t OUT_BYTES = (size_t)NTILE * OUT_TILE_BYTES;
     static constexpr size_t BAR_OFF = REC_BYTES + OUT_BYTES;
     static constexpr size_t FLAG_OFF = BAR_OFF + (size_t)NTILE * NSLOT * 2 * sizeof(unsigned long long);
-    static constexpr size_t SMEM = FLAG_OFF + (size_t)NTILE * NSLOT * sizeof(int);      // ADAPTIVE: "last step of this tile" per ring slot
+    static constexpr size_t PARK_OFF = (FLAG_OFF + (size_t)NTILE * NSLOT * sizeof(int) + 15) & ~(size_t)15;   // after the ADAPTIVE "last step" flags
+    static constexpr int NPARK = (NS == 7) ? 7 : 6;                                    // sr[3] sv[3] (sm) of one column thread
+    static constexpr size_t SMEM = PARK_OFF + (size_t)NTILE * NCOL * NPARK * 32 * sizeof(double);   // column state of every tile, lane-strided
 };
+
+// ---------------------------------------------------------------------------
+// -DLTO_K1_PROF: per-warp clock64() spans of K1 / K2, written to k1_prof[block][warp][K1P_N] when the warp retires
+// (tools/k1_phase_clocks.py reads them through lto_k1_prof_read).  Without the switch every method is empty.
+// ---------------------------------------------------------------------------
+enum { K1P_WORK, K1P_BAR, K1P_PACE, K1P_STORE, K1P_TOTAL, K1P_STEPS, K1P_N };
+#ifdef LTO_K1_PROF
+constexpr int K1P_MAX_BLOCKS = 1024, K1P_MAX_WARPS = 16;
+__device__ unsigned long long k1_prof[K1P_MAX_BLOCKS * K1P_MAX_WARPS * K1P_N];
+struct K1Prof {
+    long long c[K1P_N], t, t_begin;
+    __device__ __forceinline__ void start() {
+        for (int i = 0; i < K1P_N; ++i) c[i] = 0;
+        t = t_begin = clock64();
+    }
+    __device__ __forceinline__ void mark() { t = clock64(); }
+    __device__ __forceinline__ void add(int i) { const long long n = clock64(); c[i] += n - t; t = n; }
+    __device__ __forceinline__ void step() { ++c[K1P_STEPS]; }
+    __device__ __forceinline__ void flush(int warp, int lane) {
+        c[K1P_TOTAL] = clock64() - t_begin;
+        if (lane == 0 && blockIdx.x < K1P_MAX_BLOCKS)
+            for (int i = 0; i < K1P_N; ++i) k1_prof[((size_t)blockIdx.x * K1P_MAX_WARPS + warp) * K1P_N + i] = (unsigned long long)c[i];
+    }
+};
+#else
+struct K1Prof {
+    __device__ __forceinline__ void start() {}
+    __device__ __forceinline__ void mark() {}
+    __device__ __forceinline__ void add(int) {}
+    __device__ __forceinline__ void step() {}
+    __device__ __forceinline__ void flush(int, int) {}
+};
+#endif
 
 using namespace cwc;
 
 // ---------------------------------------------------------------------------
-// State warp: one RK step of x = [r v (m)] in Nystrom form; publishes the stage
-// linearisations of this step into `rec` (lane-strided) and accumulates maxErr.
+// State warp: one RK step of x = [r v (m)] in Nystrom form; publishes h into `rec` (lane-strided)
+// and the stage linearisations of this step into `stg` (lane-contiguous), and accumulates maxErr.
 // ---------------------------------------------------------------------------
 template <int NS, bool PUB = true>
 __device__ __forceinline__ double x_step(double (&r)[3], double (&v)[3], double& m, const double (&u)[3], double omega,
-                                         double mdot, double h, const EPConst& c, double* __restrict__ rec, double& maxErr) {
+                                         double mdot, double h, const EPConst& c, double* __restrict__ rec, double* __restrict__ stg,
+                                         double& maxErr) {
     constexpr int SVAL = Cfg<NS>::SVAL;
     const double h2 = h * h;
     const double w2 = 2.0 * omega;
@@ -103,18 +139,14 @@ __device__ __forceinline__ double x_step(double (&r)[3], double (&v)[3], double&
             const double p1 = a51 * dx1, p2 = a52 * dx2;
             const double t = p1 + p2;
             const double s5y = s5 * R[1];
-            double* w = rec + j * SVAL * 32;
-            w[0 * 32] = fma(p1, dx1, fma(p2, dx2, gg1));
-            w[1 * 32] = fma(s5y, R[1], gg1);
-            w[2 * 32] = fma(s5 * R[2], R[2], gg1 - 1.0);
-            w[3 * 32] = t * R[1];
-            w[4 * 32] = t * R[2];
-            w[5 * 32] = s5y * R[2];
+            double2* w = reinterpret_cast<double2*>(stg + j * SVAL * 32);
+            w[0] = make_double2(fma(p1, dx1, fma(p2, dx2, gg1)), fma(s5y, R[1], gg1));
+            w[1] = make_double2(fma(s5 * R[2], R[2], gg1 - 1.0), t * R[1]);
+            w[2] = make_double2(t * R[2], s5y * R[2]);
             if (NS == 7) {
-                w[6 * 32] = kom;
                 const double k2 = -kom * im;
-#pragma unroll
-                for (int q = 0; q < 3; ++q) w[(7 + q) * 32] = k2 * u[q];
+                w[3] = make_double2(kom, k2 * u[0]);
+                w[4] = make_double2(k2 * u[1], k2 * u[2]);
             }
         }
         if (lto_tab::PSIf(j) != 0.0) {
@@ -145,14 +177,14 @@ __device__ __forceinline__ double x_step(double (&r)[3], double (&v)[3], double&
 // Column warp: one RK step of one column s = [s_r s_v (s_m)] of S = [Phi | Gamma].
 // ONE instruction stream serves every column (the instruction cache is shared by the
 // whole SM): what distinguishes the columns is data --
-//   Phi column of r or v : s_m == 0,            no forcing      (bm = 0, ec = 0)
-//   Phi column of m      : s_m == 1,            no forcing      (bm = 0, ec = 0, sm = 1)
-//   Gamma column c       : s_m = bm*(t - t0),   forcing (k/m) e_c on s_v, bm on s_m
-// MASS = (NS == 7): rows/columns of the mass exist.
+//   Phi column of r or v : s_m == 0,            no forcing      (bm = 0, gc < 0)
+//   Phi column of m      : s_m == 1,            no forcing      (bm = 0, gc < 0, sm = 1)
+//   Gamma column gc      : s_m = bm*(t - t0),   forcing (k/m) e_gc on s_v, bm on s_m
+// MASS = (NS == 7): rows/columns of the mass exist.  `rec`: h (lane-strided), `stg`: this lane's stage records.
 // ---------------------------------------------------------------------------
 template <int NS>
-__device__ __forceinline__ void col_step(double (&sr)[3], double (&sv)[3], double& sm, double bm, const double (&ec)[3],
-                                         double omega, double kom6, const double* __restrict__ rec) {
+__device__ __forceinline__ void col_step(double (&sr)[3], double (&sv)[3], double& sm, double bm, int gc,
+                                         double omega, double kom6, const double* __restrict__ rec, const double* __restrict__ stg) {
     constexpr int SVAL = Cfg<NS>::SVAL;
     constexpr bool MASS = (NS == 7);
     const double h = rec[Cfg<NS>::OFF_H * 32];
@@ -174,19 +206,22 @@ __device__ __forceinline__ void col_step(double (&sr)[3], double (&sv)[3], doubl
             V[q] = (j == 0) ? sv[q] : fma(h, accv, sv[q]);
             R[q] = (j == 0) ? sr[q] : fma(h2, accr, fma(h * lto_tab::Cf(j), sv[q], sr[q]));
         }
-        const double* w = rec + j * SVAL * 32;
-        double U[6];
-#pragma unroll
-        for (int q = 0; q < 6; ++q) U[q] = w[q * 32];
-        const double kom = MASS ? w[6 * 32] : kom6;
+        const double2* w = reinterpret_cast<const double2*>(stg + j * SVAL * 32);
+        const double2 w0 = w[0], w1 = w[1], w2v = w[2];
+        const double U[6] = {w0.x, w0.y, w1.x, w1.y, w2v.x, w2v.y};
+        double2 w3 = make_double2(kom6, 0.0), w4 = make_double2(0.0, 0.0);
+        if (MASS) { w3 = w[3]; w4 = w[4]; }
+        const double kom = w3.x;
+        // forcing (k/m) e_gc: selected, not multiplied by a unit vector (w2 = +-2, so w2 * V is exact and the sums are unchanged)
         double acc[3];
-        acc[0] = fma(ec[0], kom, w2 * V[1]);
-        acc[1] = fma(ec[1], kom, -w2 * V[0]);
-        acc[2] = ec[2] * kom;
+        acc[0] = fma(w2, V[1], gc == 0 ? kom : 0.0);
+        acc[1] = fma(-w2, V[0], gc == 1 ? kom : 0.0);
+        acc[2] = gc == 2 ? kom : 0.0;
         if (MASS) {
             const double smj = fma(h * lto_tab::Cf(j), bm, sm);
+            const double am[3] = {w3.y, w4.x, w4.y};
 #pragma unroll
-            for (int q = 0; q < 3; ++q) acc[q] = fma(w[(7 + q) * 32], smj, acc[q]);
+            for (int q = 0; q < 3; ++q) acc[q] = fma(am[q], smj, acc[q]);
         }
         sym3_mul_acc(U, R, acc);
 #pragma unroll
@@ -206,15 +241,29 @@ __device__ __forceinline__ void col_step(double (&sr)[3], double (&sv)[3], doubl
     if (MASS) sm = fma(h, bm, sm);
 }
 
-// One column thread's state for one tile in flight.
-struct ColState { double sr[3], sv[3], sm, bm; };
+// One column thread's state for one tile in flight.  Between its steps it is parked in shared memory (lane-strided), so a
+// column thread holds one tile's state in registers, not NTILE.
+struct ColState { double sr[3], sv[3], sm; };
 
 template <int NS>
 __device__ __forceinline__ void col_init(ColState& c, int col) {
 #pragma unroll
     for (int q = 0; q < 3; ++q) { c.sr[q] = (col == q) ? 1.0 : 0.0; c.sv[q] = (col == q + 3) ? 1.0 : 0.0; }
     c.sm = (NS == 7 && col == 6) ? 1.0 : 0.0;                // S(0) = [I | 0]
-    c.bm = 0.0;
+}
+
+template <int NS>
+__device__ __forceinline__ void col_park(double* __restrict__ p, const ColState& c) {
+#pragma unroll
+    for (int q = 0; q < 3; ++q) { p[q * 32] = c.sr[q]; p[(3 + q) * 32] = c.sv[q]; }
+    if (NS == 7) p[6 * 32] = c.sm;
+}
+
+template <int NS>
+__device__ __forceinline__ void col_unpark(const double* __restrict__ p, ColState& c) {
+#pragma unroll
+    for (int q = 0; q < 3; ++q) { c.sr[q] = p[q * 32]; c.sv[q] = p[(3 + q) * 32]; }
+    c.sm = (NS == 7) ? p[6 * 32] : 0.0;
 }
 
 // Store this column of the segment's Jacobian block, in the defect's frame:
@@ -234,71 +283,111 @@ __device__ __forceinline__ void col_store(double* __restrict__ stage, const ColS
     if (NS == 7) J[6] = sp * c.sm;
 }
 
+// This column thread's parked state of tile t.
 template <int NS>
-__device__ __forceinline__ void column_warp(const DirectArgs& a, long long n_tiles, int col, int lane, double* recs, double* outs, unsigned bars) {
+__device__ __forceinline__ double* col_park_at(double* parks, int t, int col, int lane) {
+    return parks + (size_t)(t * Cfg<NS>::NCOL + col) * Cfg<NS>::NPARK * 32 + lane;
+}
+
+// One column step of tile t: wait for the state warp's record, step the parked column, release the record.
+// ADAPT: returns whether this was the tile's last step (K2's per-slot flag).
+template <int NS, bool ADAPT>
+__device__ __forceinline__ bool col_tile_step(int t, unsigned g, int col, int gc, int lane, double omega, double kom6, double* recs, double* parks,
+                                              unsigned bars, volatile int* lastf, K1Prof& pf) {
+    typedef Cfg<NS> C;
+    const unsigned slot = g & (NSLOT - 1), par = (g / NSLOT) & 1;
+    const double* slotp = recs + (size_t)(t * NSLOT + slot) * C::STEP_DOUBLES * 32;
+    const double* rec = slotp + lane;
+    const unsigned full = bars + (unsigned)((t * NSLOT + slot) * 16), empty = full + 8;
+    mbar_wait(full, par);
+    pf.add(K1P_BAR);
+    double* park = col_park_at<NS>(parks, t, col, lane);
+    ColState cs;
+    col_unpark<NS>(park, cs);
+    const double bm = (NS == 7 && gc >= 0) ? rec[(C::OFF_BM + gc) * 32] : 0.0;   // the state warp republishes bm with every step
+    const bool last = ADAPT && lastf[t * NSLOT + slot] != 0;
+    col_step<NS>(cs.sr, cs.sv, cs.sm, bm, gc, omega, kom6, rec, slotp + lane * C::SVAL);
+    mbar_arrive(empty);
+    col_park<NS>(park, cs);
+    pf.add(K1P_WORK);
+    pf.step();
+    return last;
+}
+
+// Both tiles of the pair are through: their 16 Jacobian blocks each are one contiguous run of the output.  Stage them in shared memory in
+// the output's own layout and let the TMA engine write each run (one bulk store, fully coalesced, also when `jac` is NVLink peer memory of
+// another GPU).
+template <int NS>
+__device__ __forceinline__ void col_tiles_store(const DirectArgs& a, long long pair, int col, int lane, double* outs, double* parks) {
+    typedef Cfg<NS> C;
+    const bool leader = (col == 0 && lane == 0);
+#pragma unroll 1
+    for (int t = 0; t < NTILE; ++t) {
+        const long long seg0 = (pair * NTILE + t) * 16;
+        double* stage = outs + (size_t)t * (C::OUT_TILE_BYTES / sizeof(double));
+        // the previous store from THIS buffer has been read out: it is the oldest of the NTILE stores in flight (one per tile and
+        // pair, issued in tile order), so the younger ones -- the other tile's, issued a moment ago -- need not be waited for.
+        // Matters when `jac` is peer memory behind a saturated NVLink port (8 GPUs delivering to one): a store then takes tens
+        // of microseconds to leave, and waiting for all of them stalled the CTA once per tile.
+        if (leader) bulk_store_wait_read_but<NTILE - 1>();
+        asm volatile("bar.sync 2, %0;" ::"n"(32 * C::NCOL) : "memory");
+        ColState cs;
+        col_unpark<NS>(col_park_at<NS>(parks, t, col, lane), cs);
+        col_store<NS>(stage, cs, col, lane);
+        fence_proxy_async();
+        asm volatile("bar.sync 2, %0;" ::"n"(32 * C::NCOL) : "memory");
+        if (leader && seg0 < a.n_seg) {
+            const long long nseg = (a.n_seg - seg0 < 16) ? (a.n_seg - seg0) : 16;
+            bulk_store(a.jac + seg0 * (long long)(NS * C::NV), smem_u32(stage), (unsigned)(nseg * NS * C::NV * sizeof(double)));
+        }
+    }
+}
+
+template <int NS>
+__device__ __forceinline__ void column_warp(const DirectArgs& a, long long n_tiles, int warp, int col, int lane, double* recs, double* outs, double* parks,
+                                            unsigned bars) {
     typedef Cfg<NS> C;
     const int nstep = a.cfg.nsteps - 1;
     const double omega = (lane & 1) ? -1.0 : 1.0;
     const double kom6 = a.c.kthr / a.c.default_mass;
     const int gc = col - NS;                             // >= 0: control component of a Gamma column
-    const double ec[3] = {gc == 0 ? 1.0 : 0.0, gc == 1 ? 1.0 : 0.0, gc == 2 ? 1.0 : 0.0};
-    ColState cs[NTILE];
+    K1Prof pf;
+    pf.start();
     unsigned g = 0;                                      // step counter of each tile stream (same for both)
     for (long long pair = blockIdx.x; pair * NTILE < n_tiles; pair += gridDim.x) {
-#pragma unroll
-        for (int t = 0; t < NTILE; ++t) col_init<NS>(cs[t], col);
+#pragma unroll 1
+        for (int t = 0; t < NTILE; ++t) { ColState c; col_init<NS>(c, col); col_park<NS>(col_park_at<NS>(parks, t, col, lane), c); }
         for (int k = 0; k < nstep; ++k, ++g) {
-            const unsigned slot = g & (NSLOT - 1), par = (g / NSLOT) & 1;
+            pf.mark();
 #ifndef LTO_K1_NO_PACE
-            // the column warps walk the ~25 KB step body together (shared instruction fetches): without this the column warp that shares its
+            // the column warps walk the step body together (shared instruction fetches): without this the column warp that shares its
             // sub-partition with a state warp and no second column warp (nstate 6) runs ahead and the instruction-cache hit rate drops
             // (78 % against 95 %).  Measured: nstate 6 0.707 -> 0.611 ms, nstate 7 unchanged (0.682 ms); a second barrier between the two
             // tiles of a step is no better for 6 and costs 8 % for 7.
             asm volatile("bar.sync 3, %0;" ::"n"(32 * C::NCOL) : "memory");
 #endif
-#pragma unroll
-            for (int t = 0; t < NTILE; ++t) {
-                const double* rec = recs + (size_t)(t * NSLOT + slot) * C::STEP_DOUBLES * 32 + lane;
-                const unsigned full = bars + (unsigned)((t * NSLOT + slot) * 16), empty = full + 8;
-                mbar_wait(full, par);
-                if (NS == 7 && k == 0 && gc >= 0) cs[t].bm = rec[(C::OFF_BM + gc) * 32];
-                col_step<NS>(cs[t].sr, cs[t].sv, cs[t].sm, cs[t].bm, ec, omega, kom6, rec);
-                mbar_arrive(empty);
-                if (k == nstep - 1) {
-                    // ---- this tile's 16 Jacobian blocks are one contiguous run of the output: stage them in shared memory in
-                    // the output's own layout and let the TMA engine write the run (one bulk store, fully coalesced, also when
-                    // `jac` is NVLink peer memory of another GPU).
-                    const long long tile = pair * NTILE + t;
-                    const long long seg0 = tile * 16;
-                    double* stage = outs + (size_t)t * (C::OUT_TILE_BYTES / sizeof(double));
-                    const bool leader = (col == 0 && lane == 0);
-                    // the previous store from THIS buffer has been read out: it is the oldest of the NTILE stores in flight (one per tile and
-                    // pair, issued in tile order), so the younger ones -- the other tile's, issued a moment ago -- need not be waited for.
-                    // Matters when `jac` is peer memory behind a saturated NVLink port (8 GPUs delivering to one): a store then takes tens
-                    // of microseconds to leave, and waiting for all of them stalled the CTA once per tile.
-                    if (leader) bulk_store_wait_read_but<NTILE - 1>();
-                    asm volatile("bar.sync 2, %0;" ::"n"(32 * C::NCOL) : "memory");
-                    col_store<NS>(stage, cs[t], col, lane);
-                    fence_proxy_async();
-                    asm volatile("bar.sync 2, %0;" ::"n"(32 * C::NCOL) : "memory");
-                    if (leader && seg0 < a.n_seg) {
-                        const long long nseg = (a.n_seg - seg0 < 16) ? (a.n_seg - seg0) : 16;
-                        bulk_store(a.jac + seg0 * (long long)(NS * C::NV), smem_u32(stage), (unsigned)(nseg * NS * C::NV * sizeof(double)));
-                    }
-                }
-            }
+            pf.add(K1P_PACE);
+            // one copy of the step body for both tiles: half the instruction footprint, and only one tile's column state live
+#pragma unroll 1
+            for (int t = 0; t < NTILE; ++t) col_tile_step<NS, false>(t, g, col, gc, lane, omega, kom6, recs, parks, bars, nullptr, pf);
         }
+        pf.mark();
+        col_tiles_store<NS>(a, pair, col, lane, outs, parks);
+        pf.add(K1P_STORE);
     }
     if (col == 0 && lane == 0) bulk_store_wait_all();        // the last bulk stores must have completed before the CTA retires
+    pf.flush(warp, lane);
 }
 
 template <int NS>
-__device__ __forceinline__ void state_warp(const DirectArgs& a, long long n_tiles, int t, int lane, double* recs, unsigned bars) {
+__device__ __forceinline__ void state_warp(const DirectArgs& a, long long n_tiles, int warp, int t, int lane, double* recs, unsigned bars) {
     typedef Cfg<NS> C;
     const int nsteps = a.cfg.nsteps, nstep = nsteps - 1;
     const int back = lane & 1;
     const double omega = back ? -1.0 : 1.0;
     double r[3], v[3], m = a.c.default_mass, u[3], bm[3] = {0.0, 0.0, 0.0}, mdot = 0.0, t0 = 0.0, t1 = 1.0, maxErr = 0.0;
+    K1Prof pf;
+    pf.start();
     unsigned g = 0;
     for (long long pair = blockIdx.x; pair * NTILE < n_tiles; pair += gridDim.x) {
         // ---- load this tile's legs (multiShoot_CRTBP_direct.jl:82-95)
@@ -328,16 +417,21 @@ __device__ __forceinline__ void state_warp(const DirectArgs& a, long long n_tile
         }
         for (int k = 0; k < nstep; ++k, ++g) {
             const unsigned slot = g & (NSLOT - 1), use = g / NSLOT;
-            double* rec = recs + (size_t)(t * NSLOT + slot) * C::STEP_DOUBLES * 32 + lane;
+            double* slotp = recs + (size_t)(t * NSLOT + slot) * C::STEP_DOUBLES * 32;
+            double* rec = slotp + lane;
             const unsigned full = bars + (unsigned)((t * NSLOT + slot) * 16), empty = full + 8;
+            pf.mark();
             if (use > 0) mbar_wait(empty, (use - 1) & 1);               // every column thread is done with this slot
+            pf.add(K1P_BAR);
             const double h = linrange_at(t0, t1, nsteps, k + 1) - linrange_at(t0, t1, nsteps, k);   // ode.jl:904
             if (NS == 7) {
 #pragma unroll
                 for (int q = 0; q < 3; ++q) rec[(C::OFF_BM + q) * 32] = bm[q];
             }
-            x_step<NS>(r, v, m, u, omega, mdot, h, a.c, rec, maxErr);
+            x_step<NS>(r, v, m, u, omega, mdot, h, a.c, rec, slotp + lane * C::SVAL, maxErr);
             mbar_arrive(full);
+            pf.add(K1P_WORK);
+            pf.step();
         }
         // ---- defect = forward end - R * backward end (:98-101), errors (:104)
         const unsigned fullmask = 0xffffffffu;
@@ -359,6 +453,7 @@ __device__ __forceinline__ void state_warp(const DirectArgs& a, long long n_tile
             if (a.status) a.status[seg] = bad ? LTO_ST_NAN : LTO_OK;
         }
     }
+    pf.flush(warp, lane);
 }
 
 
@@ -370,6 +465,19 @@ __device__ __forceinline__ void state_warp(const DirectArgs& a, long long n_tile
 // linearisation: the column is left unchanged) until the slowest leg of the tile is through; a per-slot flag tells the
 // column warps which step is the tile's last.
 // ---------------------------------------------------------------------------
+// h = 0 and a zero linearisation: a column step leaves the column unchanged
+template <int NS>
+__device__ __forceinline__ void zero_step_record(double* rec, double* stg) {
+    constexpr int SVAL = Cfg<NS>::SVAL;
+#pragma unroll
+    for (int j = 0; j < 13; ++j) {
+        double2* w = reinterpret_cast<double2*>(stg + j * SVAL * 32);
+#pragma unroll
+        for (int p = 0; p < SVAL / 2; ++p) w[p] = make_double2(0.0, 0.0);
+    }
+    rec[Cfg<NS>::OFF_H * 32] = 0.0;
+}
+
 template <int NS>
 __device__ __forceinline__ void state_warp_adapt(const DirectArgs& a, long long n_tiles, int t, int lane, double* recs, unsigned bars, volatile int* lastf) {
     typedef Cfg<NS> C;
@@ -404,7 +512,9 @@ __device__ __forceinline__ void state_warp_adapt(const DirectArgs& a, long long 
         bool done = !((tt < tfinal) && (h >= hmin));
         while (true) {
             const unsigned slot = g & (NSLOT - 1), use = g / NSLOT;
-            double* rec = recs + (size_t)(t * NSLOT + slot) * C::STEP_DOUBLES * 32 + lane;
+            double* slotp = recs + (size_t)(t * NSLOT + slot) * C::STEP_DOUBLES * 32;
+            double* rec = slotp + lane;
+            double* stg = slotp + lane * C::SVAL;
             const unsigned full = bars + (unsigned)((t * NSLOT + slot) * 16), empty = full + 8;
             if (use > 0) mbar_wait(empty, (use - 1) & 1);
             if (NS == 7) {
@@ -413,9 +523,7 @@ __device__ __forceinline__ void state_warp_adapt(const DirectArgs& a, long long 
             }
             bool pending = !done;
             if (done) {                                                      // zero-length step: leaves the column unchanged
-#pragma unroll
-                for (int j = 0; j < 13 * C::SVAL; ++j) rec[j * 32] = 0.0;
-                rec[C::OFF_H * 32] = 0.0;
+                zero_step_record<NS>(rec, stg);
             }
             while (__any_sync(fullmask, pending)) {
                 if (pending) {
@@ -426,7 +534,7 @@ __device__ __forceinline__ void state_warp_adapt(const DirectArgs& a, long long 
                     ++nt;
                     double r2[3] = {r[0], r[1], r[2]}, v2[3] = {v[0], v[1], v[2]}, m2 = m;
                     const double xn = fmax(fmax(fmax(fabs(r[0]), fabs(r[1])), fmax(fabs(r[2]), fabs(v[0]))), fmax(fmax(fabs(v[1]), fabs(v[2])), NS == 7 ? fabs(m) : 0.0));
-                    double delta = x_step<NS>(r2, v2, m2, u, omega, mdot, h, a.c, rec, dummy);
+                    double delta = x_step<NS>(r2, v2, m2, u, omega, mdot, h, a.c, rec, stg, dummy);
                     if (!(delta == delta)) { status = LTO_ST_NAN; done = true; pending = false; }
                     else {
                         const double tau = a.cfg.tol * fmax(xn, 1.0);
@@ -441,11 +549,7 @@ __device__ __forceinline__ void state_warp_adapt(const DirectArgs& a, long long 
                     }
                 }
             }
-            if (status != 0) {                                               // a failed leg must not hand a rejected attempt to the columns
-#pragma unroll
-                for (int j = 0; j < 13 * C::SVAL; ++j) rec[j * 32] = 0.0;
-                rec[C::OFF_H * 32] = 0.0;
-            }
+            if (status != 0) zero_step_record<NS>(rec, stg);               // a failed leg must not hand a rejected attempt to the columns
             const bool all_done = __all_sync(fullmask, done);
             if (lane == 0) lastf[t * NSLOT + slot] = all_done ? 1 : 0;
             mbar_arrive(full);
@@ -474,60 +578,39 @@ __device__ __forceinline__ void state_warp_adapt(const DirectArgs& a, long long 
 }
 
 template <int NS>
-__device__ __forceinline__ void column_warp_adapt(const DirectArgs& a, long long n_tiles, int col, int lane, double* recs, double* outs, unsigned bars,
-                                                  volatile int* lastf) {
-    typedef Cfg<NS> C;
+__device__ __forceinline__ void column_warp_adapt(const DirectArgs& a, long long n_tiles, int warp, int col, int lane, double* recs, double* outs,
+                                                  double* parks, unsigned bars, volatile int* lastf) {
     const double omega = (lane & 1) ? -1.0 : 1.0;
     const double kom6 = a.c.kthr / a.c.default_mass;
     const int gc = col - NS;
-    const double ec[3] = {gc == 0 ? 1.0 : 0.0, gc == 1 ? 1.0 : 0.0, gc == 2 ? 1.0 : 0.0};
-    ColState cs[NTILE];
+    K1Prof pf;
+    pf.start();
     unsigned g[NTILE];
 #pragma unroll
     for (int t = 0; t < NTILE; ++t) g[t] = 0;
     for (long long pair = blockIdx.x; pair * NTILE < n_tiles; pair += gridDim.x) {
-#pragma unroll
-        for (int t = 0; t < NTILE; ++t) col_init<NS>(cs[t], col);
-        unsigned alive = (1u << NTILE) - 1u, first = alive;
+#pragma unroll 1
+        for (int t = 0; t < NTILE; ++t) { ColState c; col_init<NS>(c, col); col_park<NS>(col_park_at<NS>(parks, t, col, lane), c); }
+        unsigned alive = (1u << NTILE) - 1u;
         while (alive) {
+            pf.mark();
 #ifndef LTO_K1_NO_PACE
-            asm volatile("bar.sync 3, %0;" ::"n"(32 * C::NCOL) : "memory");     // keep the column warps on the same instructions (see column_warp)
+            asm volatile("bar.sync 3, %0;" ::"n"(32 * Cfg<NS>::NCOL) : "memory");     // keep the column warps on the same instructions (see column_warp)
 #endif
+            pf.add(K1P_PACE);
 #pragma unroll
             for (int t = 0; t < NTILE; ++t) {
                 if (!(alive & (1u << t))) continue;
-                const unsigned slot = g[t] & (NSLOT - 1), par = (g[t] / NSLOT) & 1;
-                const double* rec = recs + (size_t)(t * NSLOT + slot) * C::STEP_DOUBLES * 32 + lane;
-                const unsigned full = bars + (unsigned)((t * NSLOT + slot) * 16), empty = full + 8;
-                mbar_wait(full, par);
-                if (NS == 7 && (first & (1u << t)) && gc >= 0) cs[t].bm = rec[(C::OFF_BM + gc) * 32];
-                first &= ~(1u << t);
-                const bool last = lastf[t * NSLOT + slot] != 0;
-                col_step<NS>(cs[t].sr, cs[t].sv, cs[t].sm, cs[t].bm, ec, omega, kom6, rec);
-                mbar_arrive(empty);
+                if (col_tile_step<NS, true>(t, g[t], col, gc, lane, omega, kom6, recs, parks, bars, lastf, pf)) alive &= ~(1u << t);
                 ++g[t];
-                if (last) alive &= ~(1u << t);
             }
         }
-        // ---- both tiles of the pair are through: stage and bulk-store their Jacobian blocks (as in column_warp)
-#pragma unroll
-        for (int t = 0; t < NTILE; ++t) {
-            const long long tile = pair * NTILE + t;
-            const long long seg0 = tile * 16;
-            double* stage = outs + (size_t)t * (C::OUT_TILE_BYTES / sizeof(double));
-            const bool leader = (col == 0 && lane == 0);
-            if (leader) bulk_store_wait_read_but<NTILE - 1>();
-            asm volatile("bar.sync 2, %0;" ::"n"(32 * C::NCOL) : "memory");
-            col_store<NS>(stage, cs[t], col, lane);
-            fence_proxy_async();
-            asm volatile("bar.sync 2, %0;" ::"n"(32 * C::NCOL) : "memory");
-            if (leader && seg0 < a.n_seg) {
-                const long long nseg = (a.n_seg - seg0 < 16) ? (a.n_seg - seg0) : 16;
-                bulk_store(a.jac + seg0 * (long long)(NS * C::NV), smem_u32(stage), (unsigned)(nseg * NS * C::NV * sizeof(double)));
-            }
-        }
+        pf.mark();
+        col_tiles_store<NS>(a, pair, col, lane, outs, parks);
+        pf.add(K1P_STORE);
     }
     if (col == 0 && lane == 0) bulk_store_wait_all();
+    pf.flush(warp, lane);
 }
 
 template <int NS, bool ADAPT>
@@ -536,6 +619,7 @@ __global__ void __launch_bounds__(Cfg<NS>::NTHREADS, 1) k_direct_cw(DirectArgs a
     extern __shared__ __align__(16) unsigned char smem_raw[];
     double* recs = reinterpret_cast<double*>(smem_raw);
     double* outs = reinterpret_cast<double*>(smem_raw + C::REC_BYTES);
+    double* parks = reinterpret_cast<double*>(smem_raw + C::PARK_OFF);
     const unsigned bars = smem_u32(smem_raw + C::BAR_OFF);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (threadIdx.x == 0) {
@@ -549,11 +633,11 @@ __global__ void __launch_bounds__(Cfg<NS>::NTHREADS, 1) k_direct_cw(DirectArgs a
     volatile int* lastf = reinterpret_cast<volatile int*>(smem_raw + C::FLAG_OFF);
     if (warp >= XW0 && warp < XW0 + NTILE) {
         if (ADAPT) state_warp_adapt<NS>(a, n_tiles, warp - XW0, lane, recs, bars, lastf);
-        else state_warp<NS>(a, n_tiles, warp - XW0, lane, recs, bars);
+        else state_warp<NS>(a, n_tiles, warp, warp - XW0, lane, recs, bars);
     } else {
         const int col = warp < XW0 ? warp : warp - NTILE;
-        if (ADAPT) column_warp_adapt<NS>(a, n_tiles, col, lane, recs, outs, bars, lastf);
-        else column_warp<NS>(a, n_tiles, col, lane, recs, outs, bars);
+        if (ADAPT) column_warp_adapt<NS>(a, n_tiles, warp, col, lane, recs, outs, parks, bars, lastf);
+        else column_warp<NS>(a, n_tiles, warp, col, lane, recs, outs, parks, bars);
     }
 }
 
@@ -584,7 +668,7 @@ __global__ void __launch_bounds__(128) k_direct_state(DirectArgs a) {
         const double mdot = -omega * un * a.c.cmdot;                       // CRTBP_prop_EP_deriv.jl:42
         for (int k = 0; k < nstep; ++k) {
             const double h = linrange_at(t0, t1, nsteps, k + 1) - linrange_at(t0, t1, nsteps, k);   // ode.jl:904
-            x_step<NS, false>(r, v, m, u, omega, mdot, h, a.c, nullptr, maxErr);
+            x_step<NS, false>(r, v, m, u, omega, mdot, h, a.c, nullptr, nullptr, maxErr);
         }
         const unsigned fullmask = 0xffffffffu;
         double xe[NS];
@@ -643,6 +727,14 @@ static cudaError_t launch_cw(const DirectArgs& a, cudaStream_t st) {
     cw::k_direct_cw<NS, ADAPT><<<grid, C::NTHREADS, C::SMEM, st>>>(a, n_tiles);
     return cudaGetLastError();
 }
+
+#ifdef LTO_K1_PROF
+// counters of the last K1 / K2 launch (each warp overwrites its own): [block < 1024][warp < 16][K1P_N] (K1P_WORK, _BAR, _PACE, _STORE, _TOTAL, _STEPS)
+extern "C" int lto_k1_prof_read(unsigned long long* out, int n_words) {
+    const size_t n = std::min<size_t>((size_t)n_words, sizeof(cw::k1_prof) / sizeof(unsigned long long));
+    return (int)cudaMemcpyFromSymbol(out, cw::k1_prof, n * sizeof(unsigned long long));
+}
+#endif
 
 cudaError_t launch_direct_cw(const DirectArgs& a, int nstate, cudaStream_t st, int* n_launch) {
     *n_launch = 0;
