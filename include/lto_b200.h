@@ -251,6 +251,27 @@ int lto_indirect_solve_batch_nd(lto_handle* h, const lto_indirect_params* p, int
                                 const double* thrustLimit_traj, const double* rho_traj,
                                 double* defect, int32_t* status_flag, int32_t* iters, double* er_out);
 
+/* lto_indirect_reduce_fuel_batch: the rho continuation of reduceFuel_indirect (src/HelperFunctions.jl:105-193) for n_traj independent
+ * ladders in one call, every solver call on the device.  Each call is lto_indirect_solve_batch_nd's (maxIter = max_iter per call --
+ * the reference uses 10 --, p = 1, flag_adjointsOnly = 0, per-trajectory rho and thrustLimit); the ladder logic runs on the device
+ * between calls, and a ladder's next call starts as soon as its last one ended (not once per round):
+ *   target = min(rho_target, rho_current); first call at rho_current from the start, done if it converges and rho_current == target;
+ *   while calls fail and rho < 1: rho = min(5 rho, 1), from the start again (a failure at rho = 1 ends the ladder with that call);
+ *   then, up to 100 rungs: after a success accept XC_new as the start and rho = max(rho / 2, target); after a failure
+ *   rho *= 3 (1 + u) with u the trajectory's next back-off draw (:182); done on a success at rho <= target.
+ *   ndim          12 or 14 (the 14-dim system with the pins and p->Isp described above)
+ *   XC_all        in/out, ndim x n_nodes per trajectory: the starts on entry, the last call's XC_new on return
+ *   t_TU          n_nodes per trajectory;  thrustLimit_traj: optional per-trajectory override of p->thrustLimit
+ *   rho_current, rho_target: n_traj each;  backoff_uniform: n_traj x 100 doubles in [0, 1), consumed in order (at most 100 a ladder)
+ *   defect        out, ndim x (n_nodes-1) per trajectory at the returned XC_all
+ *   status        out, n_traj: the last call's status_flag (0, 1, 2), or 3 when the ladder gave up after 100 rungs
+ *   calls, newton_iters, rho_last: out, n_traj: solver calls, Newton iterations over all calls, rho of the last call; may be NULL
+ * p->p must be 1 (rho only means something there): anything else is LTO_ERR_ARG. */
+int lto_indirect_reduce_fuel_batch(lto_handle* h, const lto_indirect_params* p, int ndim, int64_t n_traj, int n_nodes, int max_iter,
+                                   double* XC_all, const double* t_TU, const double* thrustLimit_traj,
+                                   const double* rho_current, const double* rho_target, const double* backoff_uniform,
+                                   double* defect, int32_t* status, int32_t* calls, int32_t* newton_iters, double* rho_last);
+
 /* ---- the linear subproblem of the direct solver (device-side; SURVEY 8(f) row 4) ------------------------
  * lto_direct_qp: optimizeTraj of src/multiShoot_CRTBP_direct.jl:248-403 in the setting the demo runs (flagEnd = false,
  * allowImpulsive = false): with tf_jump, p1_jump, p2_jump and the dV jumps pinned by their bounds (:288-302) the JuMP / Ipopt model is

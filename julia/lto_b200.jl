@@ -157,6 +157,22 @@ function multiShoot_CRTBP_indirect_batch(XC_batch::Array{Float64,3}, t_batch::Ma
         handle[], prm, m, n_traj, n_nodes, maxIter, flag_adjointsOnly ? 1 : 0, XC, t_batch, thrustLimit, rho, defect, status_flag, iters, er))
     (XC, defect, status_flag)
 end
+# ---- indirect: reduceFuel_indirect (HelperFunctions.jl:105-193) for a BATCH of rho ladders in ONE call; the ladder logic runs on the device.
+# XC_batch: m x n_nodes x n_traj starts (m = 12, or 14 with mass), t_batch: n_nodes x n_traj; thrustLimit, rho_current, rho_target: per-trajectory
+# vectors; backoff: 100 x n_traj draws in [0, 1) for the back-off rho *= 3(1 + rand()) (:182), consumed in order (rand(rng, 100) per trajectory).
+# maxIter is per solver call (the reference uses 10).  status: the last call's status_flag, or 3 when a ladder gave up after 100 rungs.
+function reduceFuel_indirect_batch(XC_batch::Array{Float64,3}, t_batch::Matrix{Float64}, MU, DU, TU, mass, thrustLimit::Vector{Float64},
+                                   rho_current::Vector{Float64}, rho_target::Vector{Float64}, backoff::Matrix{Float64}; maxIter = 10, Isp = 2000.0)
+    m = size(XC_batch, 1); n_nodes = size(XC_batch, 2); n_traj = size(XC_batch, 3)
+    XC = copy(XC_batch); defect = zeros(m, n_nodes - 1, n_traj); status = zeros(Int32, n_traj)
+    calls = zeros(Int32, n_traj); newton_iters = zeros(Int32, n_traj); rho_last = zeros(n_traj)
+    prm = iparams((MU, DU, TU, thrustLimit[1], mass, 1.0, 1.0, 1.0)); prm.Isp = Isp
+    GC.@preserve XC t_batch thrustLimit rho_current rho_target backoff defect status calls newton_iters rho_last check(ccall((:lto_indirect_reduce_fuel_batch, lib), Cint,
+        (Ptr{Cvoid}, Ref{IndirectParams}, Cint, Int64, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Int32}, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}),
+        handle[], prm, m, n_traj, n_nodes, maxIter, XC, t_batch, thrustLimit, rho_current, rho_target, backoff, defect, status, calls, newton_iters, rho_last))
+    (XC, defect, status, calls)
+end
 # ---- direct: multiShoot_CRTBP_direct (:465-594) for a BATCH of trajectories, iterated on the device (flagEnd = false, allowImpulsive = false).
 # X_batch: nstate x n_nodes x n_traj, u_batch: 3 x n_nodes x n_traj, t_batch: n_nodes x n_traj, state_0 / state_f: 6 x n_traj (interpEndStates, :483)
 function multiShoot_CRTBP_direct_batch(X_batch::Array{Float64,3}, u_batch::Array{Float64,3}, t_batch::Matrix{Float64}, state_0::Matrix{Float64},

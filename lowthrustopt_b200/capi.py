@@ -32,6 +32,7 @@ EXPORTS = [
     "lto_push_async", "lto_sync_copies", "lto_signal_dev", "lto_wait_dev", "lto_fp64_peak_probe", "lto_debug_profile",
     "lto_indirect_newton", "lto_indirect_newton_dev", "lto_indirect_newton_resolve_dev", "lto_indirect_solve_batch", "lto_direct_qp", "lto_direct_qp_dev", "lto_direct_solve_batch",
     "lto_indirect_newton_nd", "lto_indirect_newton_nd_dev", "lto_indirect_newton_resolve_nd_dev", "lto_indirect_solve_batch_nd",
+    "lto_indirect_reduce_fuel_batch",
 ]
 
 
@@ -112,6 +113,7 @@ def lib():
         L.lto_indirect_newton_nd_dev.argtypes = [vp, ci, i64, ci, ci] + [vp] * 4
         L.lto_indirect_newton_resolve_nd_dev.argtypes = [vp, ci, i64, ci, ci] + [vp] * 3
         L.lto_indirect_solve_batch_nd.argtypes = [vp, vp, ci, i64, ci, ci, ci] + [vp] * 8
+        L.lto_indirect_reduce_fuel_batch.argtypes = [vp, vp, ci, i64, ci, ci] + [vp] * 11
         L.lto_direct_qp.argtypes = [vp, i64, ci, ci] + [vp] * 9
         L.lto_direct_qp_dev.argtypes = [vp, i64, ci, ci] + [vp] * 9
         L.lto_direct_solve_batch.argtypes = [vp, vp, i64, ci, ci, ci, ci] + [vp] * 5 + [C.c_double] + [vp] * 3
@@ -549,6 +551,28 @@ class Handle:
         self._ck(lib().lto_indirect_solve_batch_nd(self._h, C.addressof(p), nd, n_traj, n_nodes, int(max_iter), int(bool(flag_adjointsOnly)),
                                                    _ptr(XC), _ptr(t_TU), _ptr(tl), _ptr(rh), _ptr(defect), _ptr(flag), _ptr(iters), _ptr(er)))
         return dict(XC_all=XC, defect=defect, status_flag=flag, iters=iters, er=er)
+
+    def indirect_reduce_fuel_batch(self, XC_all, t_TU, rho_current, rho_target, backoff_uniform, params=None, thrustLimit=None, max_iter=10):
+        """reduceFuel_indirect (HelperFunctions.jl:105-193) for n_traj independent rho ladders in one call, every solver call and the
+        ladder logic on the device (lto_indirect_reduce_fuel_batch).  XC_all: (n_traj, n_nodes, m), m = 12 or 14; t_TU: (n_traj, n_nodes);
+        rho_current, rho_target, thrustLimit: scalars or (n_traj,); backoff_uniform: (n_traj, 100) draws in [0, 1) for the back-off
+        rho *= 3(1 + u) (:182), consumed in order; params.p must be 1; max_iter: maxIter of every solver call.
+        Returns dict(XC_all, defect, status (3: gave up after 100 rungs), calls, newton_iters, rho_last)."""
+        p = params or indirect_params()
+        XC = np.array(XC_all, dtype=np.float64, order="C")
+        if XC.ndim != 3 or XC.shape[2] not in (12, 14):
+            raise ValueError("XC_all must be (n_traj, n_nodes, 12 or 14) (got %s)" % (XC.shape,))
+        n_traj, n_nodes, nd = XC.shape
+        t_TU = _shaped("t_TU", t_TU, (n_traj, n_nodes))
+        r0 = _per_unit("rho_current", rho_current, n_traj); r1 = _per_unit("rho_target", rho_target, n_traj)
+        tl = _per_unit("thrustLimit", thrustLimit, n_traj)
+        draws = _shaped("backoff_uniform", backoff_uniform, (n_traj, 100))
+        defect = np.empty((n_traj, n_nodes - 1, nd)); status = np.empty(n_traj, dtype=np.int32)
+        calls = np.empty(n_traj, dtype=np.int32); nit = np.empty(n_traj, dtype=np.int32); rho_last = np.empty(n_traj)
+        self._ck(lib().lto_indirect_reduce_fuel_batch(self._h, C.addressof(p), nd, n_traj, n_nodes, int(max_iter), _ptr(XC), _ptr(t_TU), _ptr(tl),
+                                                      _ptr(r0), _ptr(r1), _ptr(draws), _ptr(defect), _ptr(status), _ptr(calls), _ptr(nit),
+                                                      _ptr(rho_last)))
+        return dict(XC_all=XC, defect=defect, status=status, calls=calls, newton_iters=nit, rho_last=rho_last)
 
     # ---- direct method: the QP of optimizeTraj on the device ----
     def direct_qp(self, jac, defect, u_all, t_TU, b0, bf):

@@ -10,9 +10,12 @@
 //                               defect check (:328-336).  Per iteration the host reads back ONE integer (how many
 //                               trajectories are still iterating).
 //   The *_nd forms take the system dimension (12: the reference's system; 14: with mass, see lto_b200.h); the others are ndim = 12.
+//   lto_indirect_reduce_fuel_batch   reduceFuel_indirect's rho continuation (HelperFunctions.jl:105-193) for n_traj ladders: the
+//                               same iteration engine, with the ladder state machine (lto_ladder.h) run on the device when a call ends.
 // Built on the public device-pointer entry points (lto_indirect_dev, lto_sumsq_dev) and a few row-wise helper kernels.
 #include "lto_internal.h"
 #include "lto_handle.h"
+#include "lto_ladder.h"
 #include <cmath>
 #include <cstring>
 #include <thread>
@@ -66,21 +69,151 @@ __global__ void k_soc_mask(const double* __restrict__ umax, const int* __restric
     if (j < n) mask[j] = (active[j] && umax[j] < 1e-1) ? 1.0 : 0.0;
 }
 
-// line search (:243-245): alpha = alpha_all[er .== minimum(er)][1]; scale = alpha for iterating trajectories, 0 otherwise
+// line search (:243-245): alpha = alpha_all[er .== minimum(er)][1] of row j, whose trials are ers[a*n + j]
+__device__ __forceinline__ double best_alpha(const double* __restrict__ ers, const double* __restrict__ alpha_all, long long n, long long j,
+                                             int n_alpha) {
+    // minimum() propagates NaN in Julia, and then no entry compares equal: the reference would throw.  Here a NaN merit
+    // value never wins; if all are NaN the full step is taken and the NaN surfaces in the defect check.
+    double best = INFINITY; int ib = -1;
+    for (int a = 0; a < n_alpha; ++a) { const double e = ers[(long long)a * n + j]; if (e < best) { best = e; ib = a; } }
+    return ib >= 0 ? alpha_all[ib] : 1.0;
+}
+// scale = alpha for iterating trajectories, 0 otherwise
 __global__ void k_pick_alpha(const double* __restrict__ ers, const double* __restrict__ alpha_all, const int* __restrict__ active,
                              double* __restrict__ alpha, double* __restrict__ scale, long long n, int use_ls, int n_alpha = NA) {
     const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= n) return;
-    double al = 1.0;
-    if (use_ls) {
-        // minimum() propagates NaN in Julia, and then no entry compares equal: the reference would throw.  Here a NaN merit
-        // value never wins; if all are NaN the full step is taken and the NaN surfaces in the defect check.
-        double best = INFINITY; int ib = -1;
-        for (int a = 0; a < n_alpha; ++a) { const double e = ers[(long long)a * n + j]; if (e < best) { best = e; ib = a; } }
-        al = ib >= 0 ? alpha_all[ib] : 1.0;
-    }
+    const double al = use_ls ? best_alpha(ers, alpha_all, n, j, n_alpha) : 1.0;
     alpha[j] = al;
     scale[j] = active[j] ? al : 0.0;
+}
+// the same for the nsel work-set rows idx[k] of a gathered line search (ers[a*nsel + k])
+__global__ void k_pick_alpha_sel(const double* __restrict__ ers, const double* __restrict__ alpha_all, const int* __restrict__ idx,
+                                 double* __restrict__ scale, long long nsel) {
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < nsel) scale[idx[k]] = best_alpha(ers, alpha_all, nsel, k, NA);
+}
+
+// Rows of the work set a gathered pass takes: those at their nominal pass (wit < 0), or those due a line search (wit >= 3, :300).
+__global__ void k_select(const int* __restrict__ wit, int* __restrict__ sel, long long n, int line_search) {
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < n) sel[j] = line_search ? (wit[j] >= 3) : (wit[j] < 0);
+}
+// idx[k] = the k-th selected row (pos: exclusive prefix sum of sel)
+__global__ void k_index_of(const int* __restrict__ sel, const int* __restrict__ pos, int* __restrict__ idx, long long n) {
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < n && sel[j]) idx[pos[j]] = (int)j;
+}
+// dst[a][k][e] = src[idx[k]][e] for a < reps
+__global__ void __launch_bounds__(256) k_gather_rows(const double* __restrict__ src, const int* __restrict__ idx, double* __restrict__ dst,
+                                                     long long nsel, long long len, int reps) {
+    const long long total = nsel * len;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total * reps; i += (long long)gridDim.x * blockDim.x) {
+        const long long r = i % total, k = r / len;
+        dst[i] = src[(long long)idx[k] * len + (r - k * len)];
+    }
+}
+// dst[idx[k]][e] = src[k][e]
+__global__ void __launch_bounds__(256) k_scatter_rows(const double* __restrict__ src, const int* __restrict__ idx, double* __restrict__ dst,
+                                                      long long nsel, long long len) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nsel * len; i += (long long)gridDim.x * blockDim.x) {
+        const long long k = i / len;
+        dst[(long long)idx[k] * len + (i - k * len)] = src[i];
+    }
+}
+// line-search trials of the selected rows: out[a][k][e] = x[idx[k]][e] + alpha_all[a] * u[idx[k]][e]  (k_axpy_rows's arithmetic)
+__global__ void __launch_bounds__(256) k_ls_trials(const double* __restrict__ x, const double* __restrict__ u, const int* __restrict__ idx,
+                                                   const double* __restrict__ alpha_all, double* __restrict__ out, long long nsel, long long len) {
+    const long long total = nsel * len;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total * NA; i += (long long)gridDim.x * blockDim.x) {
+        const long long a = i / total, r = i - a * total, k = r / len;
+        const long long s = (long long)idx[k] * len + (r - k * len);
+        out[i] = fma(alpha_all[a], u[s], x[s]);
+    }
+}
+
+// End of a solver call's step for the rows of the indirect engine's work set, each with its own iteration counter wit[j]
+// (-1: the call has just started and waits for its nominal pass).  phase 0: after the nominal pass (:274) of the rows with
+// wit < 0 (the others only count); phase 1: after a Newton iteration of every row.  Same rules as k_iter_end:
+// er = norm(defect[:], Inf); abort above 1e3 (:333-336); maxIter (:282-286); loop condition er > 1e-10; NaN -> flag 2.
+// count[0]: rows still iterating; count[1]: of these, the ones whose next iteration runs the line search (iterCount > 3).
+__global__ void k_call_end(const double* __restrict__ er, int* __restrict__ active, const int* __restrict__ orig, int* __restrict__ wit,
+                           int* __restrict__ iters, int* __restrict__ flag, double* __restrict__ er_full, unsigned long long* __restrict__ count,
+                           long long n, int phase, int max_iter) {
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    int c = wit[j];
+    bool go = true;
+    if (phase == 1 || c < 0) {
+        c = phase == 0 ? 0 : c + 1;
+        wit[j] = c;
+        const int o = orig[j];
+        const double e = er[j];
+        er_full[o] = e;
+        if (c > 0) iters[o] = c;
+        go = e > 1e-10;                                   // NaN -> false: the reference's while-condition ends the loop as well
+        if (!(e == e)) flag[o] = 2;
+        if (go && !(e <= 1e3)) { go = false; flag[o] = 1; }
+        if (go && c >= max_iter) { go = false; flag[o] = 1; }
+        active[j] = go ? 1 : 0;
+    }
+    if (go) { atomicAdd(&count[0], 1ull); if (c >= 3) atomicAdd(&count[1], 1ull); }
+}
+
+// The continuation ladder's hook (lto_ladder.h), one warp per work-set row whose solver call just ended (active[j] == 0).  The
+// call's status is that of lto_indirect_solve_batch (k_call_end's flag, 2 when a node is non-finite, as k_retire_rows reports it).
+// A ladder that goes on accepts XC_new as its start or resets the row to the accepted start (acc), sets the call's rho and
+// re-enters the work set at its nominal pass (count[0], count[2]); a ladder that ends writes its row to the caller-ordered outputs.
+__global__ void __launch_bounds__(256) k_ladder_hook(double* __restrict__ XC, const double* __restrict__ Def, double* __restrict__ RH,
+                                                     int* __restrict__ active, const int* __restrict__ orig, int* __restrict__ wit,
+                                                     int* __restrict__ iters, int* __restrict__ flag, LadderState* __restrict__ ladder,
+                                                     const double* __restrict__ draws, double* __restrict__ acc, double* __restrict__ XCout,
+                                                     double* __restrict__ DefOut, int* __restrict__ status, int* __restrict__ calls,
+                                                     int* __restrict__ newton_iters, double* __restrict__ rho_last, unsigned long long* __restrict__ count, long long n,
+                                                     long long LX, long long LD) {
+    const long long j = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (j >= n || active[j]) return;
+    const long long o = orig[j];
+    double* x = XC + j * LX;
+    bool bad = false;
+    for (long long i = lane; i < LX; i += 32) bad |= !(fabs(x[i]) <= 1.7976931348623157e308);
+    bad = __any_sync(0xffffffffu, bad);
+    int go = 0, take = 0;
+    if (lane == 0) {
+        const int st = bad ? 2 : flag[o];
+        newton_iters[o] += iters[o];
+        LadderState s = ladder[o];
+        int fin = 0;
+        go = ladder_step(&s, st, draws + o * LADDER_DRAWS, &take, &fin);
+        ladder[o] = s;
+        if (go) {
+            RH[j] = s.rho; wit[j] = -1; active[j] = 1; flag[o] = 0; iters[o] = 0; calls[o] += 1;
+            atomicAdd(&count[0], 1ull); atomicAdd(&count[2], 1ull);
+        } else {
+            status[o] = fin; rho_last[o] = s.rho;
+        }
+    }
+    go = __shfl_sync(0xffffffffu, go, 0);
+    take = __shfl_sync(0xffffffffu, take, 0);
+    double* a = acc + o * LX;
+    if (go) {
+        if (take) { for (long long i = lane; i < LX; i += 32) a[i] = x[i]; }
+        else      { for (long long i = lane; i < LX; i += 32) x[i] = a[i]; }
+    } else {
+        for (long long i = lane; i < LX; i += 32) XCout[o * LX + i] = x[i];
+        for (long long i = lane; i < LD; i += 32) DefOut[o * LD + i] = Def[j * LD + i];
+    }
+}
+
+// RH: rho_current on entry, the rho of the first call on return
+__global__ void k_ladder_init(double* __restrict__ RH, const double* __restrict__ rho_target, LadderState* __restrict__ ladder,
+                              int* __restrict__ calls, int* __restrict__ newton_iters, long long n) {
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    LadderState s;
+    RH[j] = ladder_init(&s, RH[j], rho_target[j]);
+    ladder[j] = s; calls[j] = 1; newton_iters[j] = 0;
 }
 
 // tile the per-trajectory parameter arrays for the NA trial copies
@@ -200,6 +333,192 @@ static int split_trajectories(lto_handle* h, long long n_traj, F&& call) {
     for (int i = 0; i < nc; ++i)
         if (rcs[i]) return fail(h, rcs[i], "device %d: %s", h->child[i]->device, h->child[i]->err);
     return LTO_SUCCESS;
+}
+
+// ---- the iteration engine of the batched indirect solver (multiShoot_CRTBP_indirect :254-345, p as given) ----
+// The work set holds the trajectories whose solver call is running, compacted to the front after every step; every row has
+// its own iteration counter wit[j] (-1: the call has just started and waits for its nominal pass).  When a row's call ends,
+// `hook` decides what becomes of it: lto_indirect_solve_batch_nd retires it into the caller-ordered outputs; the continuation
+// ladder either retires it or starts its next call in place (it then re-enters at its nominal pass, in the same step).
+// Per step the host reads back one set of counts.
+struct EngineArrays {
+    double *XC, *Def, *RH, *XCout, *DefOut, *ErOut;
+    int *active, *orig, *wit, *iters, *flag;
+    unsigned long long* count;         // [0] rows iterating, [1] of them due a line search, [2] rows the hook restarted
+};
+
+template <class Setup, class Hook>
+static int indirect_engine(lto_handle* h, const lto_indirect_params* p, int ND, long long T, int N, int max_iter, int flag_adjointsOnly,
+                           const double* XC_all, const double* t_TU, const double* thrustLimit_traj, const double* rho_traj,
+                           size_t extra_bytes, EngineArrays* w, Setup&& setup, Hook&& hook) {
+    const int NA = slv::NA;
+    const long long ns = T * (N - 1), nn = T * N;
+    const long long LX = (long long)N * ND, LD = (long long)(N - 1) * ND;      // row lengths: states / defects of one trajectory
+    cudaStream_t st = h->s_compute;
+    // ---- device arrays.  "work" arrays hold the trajectories still iterating (compacted to the front after every step);
+    // "out" arrays are in the caller's order and receive a trajectory's rows when it stops.
+    const size_t bXC = al(nn * ND * 8), bT = al(nn * 8), bPar = al(T * 8), bDef = al(ns * ND * 8), bPhi = al(ns * ND * ND * 8);
+    const size_t bTrX = al((size_t)NA * nn * ND * 8), bTrD = al((size_t)NA * ns * ND * 8), bTrT = al((size_t)NA * nn * 8), bTrP = al((size_t)NA * T * 8);
+    const size_t bVec = al((size_t)NA * T * 8), bInt = al(T * 4);
+    size_t need = bXC * 4 + bT + bPar * 2 + bDef * 3 + bPhi + bTrX + bTrD + bTrT + bTrP * 2 + bVec * 8 + bInt * 9 + al(NA * 8) + 256 + al(extra_bytes);
+    int rc = ensure(h, &h->d_slv, &h->d_slv_cap, need); if (rc) return rc;
+    char* q = (char*)h->d_slv;
+    auto take = [&](size_t b) { char* r = q; q += b; return r; };
+    double* dXC = (double*)take(bXC); double* dXS = (double*)take(bXC); double* dUp = (double*)take(bXC); double* dUp2 = dXS;   // the SOC state buffer is free again when the SOC update is computed
+    double* dXCout = (double*)take(bXC);
+    double* dT = (double*)take(bT);
+    double* dTL = thrustLimit_traj ? (double*)take(bPar) : nullptr; double* dRH = rho_traj ? (double*)take(bPar) : nullptr;
+    double* dDef = (double*)take(bDef); double* dDs = (double*)take(bDef); double* dDefOut = (double*)take(bDef); double* dPhi = (double*)take(bPhi);
+    double* dTrX = (double*)take(bTrX); double* dTrD = (double*)take(bTrD); double* dTrT = (double*)take(bTrT);
+    double* dTrTL = thrustLimit_traj ? (double*)take(bTrP) : nullptr; double* dTrRH = rho_traj ? (double*)take(bTrP) : nullptr;
+    double* dEr = (double*)take(bVec); double* dUmax = (double*)take(bVec); double* dMask = (double*)take(bVec);
+    double* dErs = (double*)take(bVec); double* dAlpha = (double*)take(bVec); double* dScale = (double*)take(bVec);
+    double* dLsTable = (double*)take(bVec); double* dErOut = (double*)take(bVec);
+    int* dActive = (int*)take(bInt); int* dIters = (int*)take(bInt); int* dFlag = (int*)take(bInt);
+    int* dOrig = (int*)take(bInt); int* dOrig2 = (int*)take(bInt); int* dPos = (int*)take(bInt);
+    int* dWit = (int*)take(bInt); int* dSel = (int*)take(bInt); int* dIdx = (int*)take(bInt);
+    double* dAlphaAll = (double*)take(al(NA * 8));
+    unsigned long long* dCount = (unsigned long long*)take(256);
+    char* dExtra = take(al(extra_bytes));
+    *w = EngineArrays{dXC, dDef, dRH, dXCout, dDefOut, dErOut, dActive, dOrig, dWit, dIters, dFlag, dCount};
+    // ---- inputs
+    CK(h, cudaMemcpyAsync(dXC, XC_all, nn * ND * 8, cudaMemcpyHostToDevice, st));
+    CK(h, cudaMemcpyAsync(dT, t_TU, nn * 8, cudaMemcpyHostToDevice, st));
+    if (dTL) CK(h, cudaMemcpyAsync(dTL, thrustLimit_traj, T * 8, cudaMemcpyHostToDevice, st));
+    if (dRH) CK(h, cudaMemcpyAsync(dRH, rho_traj, T * 8, cudaMemcpyHostToDevice, st));
+    double alpha_all[slv::NA];
+    for (int a = 0; a < NA; ++a) alpha_all[a] = 0.1 + (double)a * ((1.0 - 0.1) / (double)(NA - 1));      // LinRange(0.1, 1, 20)
+    alpha_all[NA - 1] = 1.0;
+    CK(h, cudaMemcpyAsync(dAlphaAll, alpha_all, NA * 8, cudaMemcpyHostToDevice, st));
+    rc = setup(dExtra); if (rc) return rc;
+    CK(h, cudaStreamSynchronize(st));                                     // alpha_all is a stack array
+    CK(h, cudaMemsetAsync(dIters, 0, T * 4, st));
+    CK(h, cudaMemsetAsync(dFlag, 0, T * 4, st));
+    slv::k_iota<<<slv::nblk(T, 256), 256, 0, st>>>(dOrig, dActive, T);
+    slv::k_set_int<<<slv::nblk(T, 256), 256, 0, st>>>(dWit, -1, T);                           // every call starts at its nominal pass
+    h->launches += 2;
+    CK(h, cudaEventRecord(h->ev_t0, st));
+
+    long long nc = T;                                                     // size of the work set
+    auto defect_pass = [&](const double* X, const double* T_, const double* tl, const double* rh, long long ntr, double* D) -> int {
+        return lto_indirect_dev(h, p, ntr * (N - 1), N, ND, X, T_, nullptr, nullptr, tl, rh, D, nullptr, nullptr, nullptr);
+    };
+    auto rowmax = [&](const double* v, long long rows, long long len, double* out) {
+        slv::k_rowmaxabs<<<slv::nblk(rows * 32, 256), 256, 0, st>>>(v, rows, len, out); h->launches += 1;
+    };
+    auto axpy = [&](const double* x, const double* u, const double* scale, double* out, long long rows, long long len, int reps) {
+        dim3 g(std::min<unsigned>(slv::nblk(rows * len, 256), 148u * 16u), (unsigned)reps);
+        slv::k_axpy_rows<<<g, 256, 0, st>>>(x, u, scale, out, rows, len); h->launches += 1;
+    };
+    auto grid_for = [&](long long n) { return std::min<unsigned>(slv::nblk(n, 256), 148u * 16u); };
+    // idx[0..nsel) = the work-set rows at their nominal pass (line_search = 0) or due a line search (1)
+    auto select = [&](int line_search) {
+        slv::k_select<<<slv::nblk(nc, 256), 256, 0, st>>>(dWit, dSel, nc, line_search);
+        slv::k_scan_active<<<1, 1024, 0, st>>>(dSel, dPos, nc);
+        slv::k_index_of<<<slv::nblk(nc, 256), 256, 0, st>>>(dSel, dPos, dIdx, nc);
+        h->launches += 3;
+    };
+    auto gather = [&](const double* src, double* dst, long long nsel, long long len, int reps) {
+        slv::k_gather_rows<<<grid_for(nsel * len * reps), 256, 0, st>>>(src, dIdx, dst, nsel, len, reps); h->launches += 1;
+    };
+    auto scatter = [&](const double* src, double* dst, long long nsel, long long len) {
+        slv::k_scatter_rows<<<grid_for(nsel * len), 256, 0, st>>>(src, dIdx, dst, nsel, len); h->launches += 1;
+    };
+    // end of a step: bookkeeping, the hook on the rows whose call ended, compaction of the rest.  Reads back the counts.
+    unsigned long long cnt[3] = {0, 0, 0};
+    auto step_end = [&](int phase) -> int {
+        CK(h, cudaMemsetAsync(dCount, 0, 3 * 8, st));
+        slv::k_call_end<<<slv::nblk(nc, 256), 256, 0, st>>>(dEr, dActive, dOrig, dWit, dIters, dFlag, dErOut, dCount, nc, phase, max_iter);
+        h->launches += 1;
+        int rc2 = hook(nc); if (rc2) return rc2;
+        CK(h, cudaMemcpyAsync(cnt, dCount, 3 * 8, cudaMemcpyDeviceToHost, st));
+        CK(h, cudaStreamSynchronize(st));
+        const long long na = (long long)cnt[0];
+        if (na > 0 && na < nc) {
+            slv::k_scan_active<<<1, 1024, 0, st>>>(dActive, dPos, nc);
+            // XC, defects (through free buffers), times, parameters, original indices, iteration counters
+            slv::k_compact_rows<double><<<grid_for(nc * LX), 256, 0, st>>>(dXC, dXS, dPos, dActive, nc, LX);
+            CK(h, cudaMemcpyAsync(dXC, dXS, (size_t)na * LX * 8, cudaMemcpyDeviceToDevice, st));
+            slv::k_compact_rows<double><<<grid_for(nc * LD), 256, 0, st>>>(dDef, dDs, dPos, dActive, nc, LD);
+            CK(h, cudaMemcpyAsync(dDef, dDs, (size_t)na * LD * 8, cudaMemcpyDeviceToDevice, st));
+            slv::k_compact_rows<double><<<grid_for(nc * N), 256, 0, st>>>(dT, dUp, dPos, dActive, nc, N);
+            CK(h, cudaMemcpyAsync(dT, dUp, (size_t)na * N * 8, cudaMemcpyDeviceToDevice, st));
+            if (dTL) { slv::k_compact_rows<double><<<grid_for(nc), 256, 0, st>>>(dTL, dUmax, dPos, dActive, nc, 1); CK(h, cudaMemcpyAsync(dTL, dUmax, (size_t)na * 8, cudaMemcpyDeviceToDevice, st)); }
+            if (dRH) { slv::k_compact_rows<double><<<grid_for(nc), 256, 0, st>>>(dRH, dUmax, dPos, dActive, nc, 1); CK(h, cudaMemcpyAsync(dRH, dUmax, (size_t)na * 8, cudaMemcpyDeviceToDevice, st)); }
+            slv::k_compact_rows<int><<<grid_for(nc), 256, 0, st>>>(dOrig, dOrig2, dPos, dActive, nc, 1);
+            CK(h, cudaMemcpyAsync(dOrig, dOrig2, (size_t)na * 4, cudaMemcpyDeviceToDevice, st));
+            slv::k_compact_rows<int><<<grid_for(nc), 256, 0, st>>>(dWit, dOrig2, dPos, dActive, nc, 1);
+            CK(h, cudaMemcpyAsync(dWit, dOrig2, (size_t)na * 4, cudaMemcpyDeviceToDevice, st));
+            slv::k_set_int<<<slv::nblk(na, 256), 256, 0, st>>>(dActive, 1, na);      // the compacted work set: all iterating
+            h->launches += 7 + (dTL ? 1 : 0) + (dRH ? 1 : 0);
+        }
+        nc = na;
+        return 0;
+    };
+
+    long long n_fresh = nc;                                               // rows at the nominal pass of a new call
+    for (;;) {
+        // ---- nominal runs (:274) of the calls that start; a call that converges there ends after 0 iterations
+        while (n_fresh > 0) {
+            if (n_fresh == nc) {
+                rc = defect_pass(dXC, dT, dTL, dRH, nc, dDef); if (rc) return rc;
+                rowmax(dDef, nc, LD, dEr);
+            } else {
+                select(0);
+                gather(dXC, dTrX, n_fresh, LX, 1); gather(dT, dTrT, n_fresh, N, 1);
+                if (dTL) gather(dTL, dTrTL, n_fresh, 1, 1);
+                if (dRH) gather(dRH, dTrRH, n_fresh, 1, 1);
+                rc = defect_pass(dTrX, dTrT, dTrTL, dTrRH, n_fresh, dTrD); if (rc) return rc;
+                rowmax(dTrD, n_fresh, LD, dErs);
+                scatter(dTrD, dDef, n_fresh, LD); scatter(dErs, dEr, n_fresh, 1);
+            }
+            rc = step_end(0); if (rc) return rc;
+            n_fresh = (long long)cnt[2];
+        }
+        if (nc == 0) break;
+        const long long n_ls = (long long)cnt[1];
+        // ---- one Newton iteration of every row of the work set
+        // jacobianCalc (:290): one launch, Phi_i of every segment of every trajectory still iterating (and the defects, unchanged)
+        rc = lto_indirect_dev(h, p, nc * (N - 1), N, ND, dXC, dT, nullptr, nullptr, dTL, dRH, dDef, nullptr, nullptr, dPhi); if (rc) return rc;
+        // optimizeTraj_OLS (:149-183)
+        rc = lto_indirect_newton_nd_dev(h, ND, nc, N, flag_adjointsOnly, dPhi, dDef, dUp, nullptr); if (rc) return rc;
+        // second-order correction (:187-214), only where norm(xc_update, Inf) < 1e-1
+        rowmax(dUp, nc, LX, dUmax);
+        slv::k_soc_mask<<<slv::nblk(nc, 256), 256, 0, st>>>(dUmax, dActive, dMask, nc); h->launches += 1;
+        axpy(dXC, dUp, dMask, dXS, nc, LX, 1);                                                 // XC_all_soc (:194)
+        rc = defect_pass(dXS, dT, dTL, dRH, nc, dDs); if (rc) return rc;                       // :197
+        rc = lto_indirect_newton_resolve_nd_dev(h, ND, nc, N, flag_adjointsOnly, dDs, dUp2, nullptr); if (rc) return rc;   // :207 (same Jacobian: stored reflections replayed)
+        axpy(dUp, dUp2, dMask, dUp, nc, LX, 1);                                                // xc_update += xc_update_soc (:213)
+        // line search (:298-302) for the rows whose iterCount > 3: all 20 x n trial trajectories in one launch
+        if (n_ls == nc) {
+            slv::k_fill_ls<<<slv::nblk(nc * NA, 256), 256, 0, st>>>(dAlphaAll, dLsTable, nc);
+            slv::k_tile<<<slv::nblk((long long)NA * nc * N, 256), 256, 0, st>>>(dT, dTrT, nc * N, NA);
+            if (dTL) slv::k_tile<<<slv::nblk((long long)NA * nc, 256), 256, 0, st>>>(dTL, dTrTL, nc, NA);
+            if (dRH) slv::k_tile<<<slv::nblk((long long)NA * nc, 256), 256, 0, st>>>(dRH, dTrRH, nc, NA);
+            h->launches += 2 + (dTL ? 1 : 0) + (dRH ? 1 : 0);
+            axpy(dXC, dUp, dLsTable, dTrX, nc, LX, NA);                                        // XC_all + xc_update*alpha (:235)
+        } else if (n_ls > 0) {                                                                 // only the rows due one, gathered
+            select(1);
+            slv::k_ls_trials<<<grid_for((long long)NA * n_ls * LX), 256, 0, st>>>(dXC, dUp, dIdx, dAlphaAll, dTrX, n_ls, LX); h->launches += 1;
+            gather(dT, dTrT, n_ls, N, NA);
+            if (dTL) gather(dTL, dTrTL, n_ls, 1, NA);
+            if (dRH) gather(dRH, dTrRH, n_ls, 1, NA);
+        }
+        if (n_ls > 0) {
+            rc = defect_pass(dTrX, dTrT, dTrTL, dTrRH, (long long)NA * n_ls, dTrD); if (rc) return rc;   // :238
+            rc = lto_sumsq_dev(h, dTrD, (long long)NA * n_ls, LD, dErs); if (rc) return rc;    // er[ind] = sum(defect[:].^2) (:241)
+        }
+        slv::k_pick_alpha<<<slv::nblk(nc, 256), 256, 0, st>>>(dErs, dAlphaAll, dActive, dAlpha, dScale, nc, n_ls == nc); h->launches += 1;
+        if (n_ls > 0 && n_ls < nc) { slv::k_pick_alpha_sel<<<slv::nblk(n_ls, 256), 256, 0, st>>>(dErs, dAlphaAll, dIdx, dScale, n_ls); h->launches += 1; }
+        axpy(dXC, dUp, dScale, dXC, nc, LX, 1);                                                // XC_all = XC_all + xc_update*alpha (:304)
+        // the end states cannot have moved (:324-325): their update entries are exact zeros (lto_newton.cu; 14-dim: the 7-element pins)
+        rc = defect_pass(dXC, dT, dTL, dRH, nc, dDef); if (rc) return rc;                      // :328
+        rowmax(dDef, nc, LD, dEr);                                                             // :332
+        rc = step_end(1); if (rc) return rc;
+        n_fresh = (long long)cnt[2];
+    }
+    CK(h, cudaEventRecord(h->ev_t1, st));
+    return 0;
 }
 
 extern "C" {
@@ -533,148 +852,101 @@ int lto_indirect_solve_batch_nd(lto_handle* h, const lto_indirect_params* p, int
         });
     }
     CK(h, cudaSetDevice(h->device));
-    const int ND = ndim, N = n_nodes, NA = slv::NA;
-    const long long T = n_traj, ns = T * (N - 1), nn = T * N;
+    const long long T = n_traj, N = n_nodes, ns = T * (N - 1), nn = T * N;
     if (T > 0x7fffffffll) return fail(h, LTO_ERR_ARG, "too many trajectories");
-    const long long LX = (long long)N * ND, LD = (long long)(N - 1) * ND;      // row lengths: states / defects of one trajectory
+    const long long LX = N * ndim, LD = (N - 1) * ndim;
     cudaStream_t st = h->s_compute;
-    // ---- device arrays.  "work" arrays hold the trajectories still iterating (compacted to the front after every iteration);
-    // "out" arrays are in the caller's order and receive a trajectory's rows when it stops.
-    const size_t bXC = al(nn * ND * 8), bT = al(nn * 8), bPar = al(T * 8), bDef = al(ns * ND * 8), bPhi = al(ns * ND * ND * 8);
-    const size_t bTrX = al((size_t)NA * nn * ND * 8), bTrD = al((size_t)NA * ns * ND * 8), bTrT = al((size_t)NA * nn * 8), bTrP = al((size_t)NA * T * 8);
-    const size_t bVec = al((size_t)NA * T * 8), bInt = al(T * 4);
-    size_t need = bXC * 4 + bT + bPar * 2 + bDef * 3 + bPhi + bTrX + bTrD + bTrT + bTrP * 2 + bVec * 8 + bInt * 6 + al(NA * 8) + 256;
-    int rc = ensure(h, &h->d_slv, &h->d_slv_cap, need); if (rc) return rc;
-    char* q = (char*)h->d_slv;
-    auto take = [&](size_t b) { char* r = q; q += b; return r; };
-    double* dXC = (double*)take(bXC); double* dXS = (double*)take(bXC); double* dUp = (double*)take(bXC); double* dUp2 = dXS;   // the SOC state buffer is free again when the SOC update is computed
-    double* dXCout = (double*)take(bXC);
-    double* dT = (double*)take(bT);
-    double* dTL = thrustLimit_traj ? (double*)take(bPar) : nullptr; double* dRH = rho_traj ? (double*)take(bPar) : nullptr;
-    double* dDef = (double*)take(bDef); double* dDs = (double*)take(bDef); double* dDefOut = (double*)take(bDef); double* dPhi = (double*)take(bPhi);
-    double* dTrX = (double*)take(bTrX); double* dTrD = (double*)take(bTrD); double* dTrT = (double*)take(bTrT);
-    double* dTrTL = thrustLimit_traj ? (double*)take(bTrP) : nullptr; double* dTrRH = rho_traj ? (double*)take(bTrP) : nullptr;
-    double* dEr = (double*)take(bVec); double* dUmax = (double*)take(bVec); double* dMask = (double*)take(bVec);
-    double* dErs = (double*)take(bVec); double* dAlpha = (double*)take(bVec); double* dScale = (double*)take(bVec);
-    double* dLsTable = (double*)take(bVec); double* dErOut = (double*)take(bVec);
-    int* dActive = (int*)take(bInt); int* dIters = (int*)take(bInt); int* dFlag = (int*)take(bInt);
-    int* dOrig = (int*)take(bInt); int* dOrig2 = (int*)take(bInt); int* dPos = (int*)take(bInt);
-    double* dAlphaAll = (double*)take(al(NA * 8));
-    unsigned long long* dCount = (unsigned long long*)take(256);
-    // ---- inputs
-    CK(h, cudaMemcpyAsync(dXC, XC_all, nn * ND * 8, cudaMemcpyHostToDevice, st));
-    CK(h, cudaMemcpyAsync(dT, t_TU, nn * 8, cudaMemcpyHostToDevice, st));
-    if (dTL) CK(h, cudaMemcpyAsync(dTL, thrustLimit_traj, T * 8, cudaMemcpyHostToDevice, st));
-    if (dRH) CK(h, cudaMemcpyAsync(dRH, rho_traj, T * 8, cudaMemcpyHostToDevice, st));
-    double alpha_all[slv::NA];
-    for (int a = 0; a < NA; ++a) alpha_all[a] = 0.1 + (double)a * ((1.0 - 0.1) / (double)(NA - 1));      // LinRange(0.1, 1, 20)
-    alpha_all[NA - 1] = 1.0;
-    CK(h, cudaMemcpyAsync(dAlphaAll, alpha_all, NA * 8, cudaMemcpyHostToDevice, st));
-    CK(h, cudaStreamSynchronize(st));                                     // alpha_all is a stack array
-    CK(h, cudaMemsetAsync(dIters, 0, T * 4, st));
-    CK(h, cudaMemsetAsync(dFlag, 0, T * 4, st));
-    slv::k_iota<<<slv::nblk(T, 256), 256, 0, st>>>(dOrig, dActive, T);
-    h->launches += 1;
-    CK(h, cudaEventRecord(h->ev_t0, st));
-
-    long long nc = T;                                                     // size of the work set
-    auto defect_pass = [&](const double* X, const double* T_, const double* tl, const double* rh, long long ntr, double* D) -> int {
-        return lto_indirect_dev(h, p, ntr * (N - 1), N, ND, X, T_, nullptr, nullptr, tl, rh, D, nullptr, nullptr, nullptr);
-    };
-    auto rowmax = [&](const double* v, long long rows, long long len, double* out) {
-        slv::k_rowmaxabs<<<slv::nblk(rows * 32, 256), 256, 0, st>>>(v, rows, len, out); h->launches += 1;
-    };
-    auto axpy = [&](const double* x, const double* u, const double* scale, double* out, long long rows, long long len, int reps) {
-        dim3 g(std::min<unsigned>(slv::nblk(rows * len, 256), 148u * 16u), (unsigned)reps);
-        slv::k_axpy_rows<<<g, 256, 0, st>>>(x, u, scale, out, rows, len); h->launches += 1;
-    };
-    auto grid_for = [&](long long n) { return std::min<unsigned>(slv::nblk(n, 256), 148u * 16u); };
-    // per-work-set tables for the batched line search: alpha table and the NA-fold tiled time / parameter arrays
-    auto prepare_trials = [&]() {
-        slv::k_fill_ls<<<slv::nblk(nc * NA, 256), 256, 0, st>>>(dAlphaAll, dLsTable, nc);
-        slv::k_tile<<<slv::nblk((long long)NA * nc * N, 256), 256, 0, st>>>(dT, dTrT, nc * N, NA);
-        if (dTL) slv::k_tile<<<slv::nblk((long long)NA * nc, 256), 256, 0, st>>>(dTL, dTrTL, nc, NA);
-        if (dRH) slv::k_tile<<<slv::nblk((long long)NA * nc, 256), 256, 0, st>>>(dRH, dTrRH, nc, NA);
-        h->launches += 2 + (dTL ? 1 : 0) + (dRH ? 1 : 0);
-    };
-    // end of an iteration: bookkeeping, retire the rows that stopped, compact the rest.  Returns the new work-set size.
-    auto iter_end = [&](int it, long long* n_next) -> int {
-        CK(h, cudaMemsetAsync(dCount, 0, 8, st));
-        slv::k_iter_end<<<slv::nblk(nc, 256), 256, 0, st>>>(dEr, dActive, dOrig, dIters, dFlag, dErOut, dCount, nc, it, max_iter);
-        slv::k_retire_rows<<<grid_for(nc * LX), 256, 0, st>>>(dXC, dXCout, dOrig, dActive, nc, LX, dFlag);
-        slv::k_retire_rows<<<grid_for(nc * LD), 256, 0, st>>>(dDef, dDefOut, dOrig, dActive, nc, LD);
-        h->launches += 3;
-        unsigned long long na = 0;
-        CK(h, cudaMemcpyAsync(&na, dCount, 8, cudaMemcpyDeviceToHost, st));
-        CK(h, cudaStreamSynchronize(st));
-        if (na > 0 && (long long)na < nc) {
-            slv::k_scan_active<<<1, 1024, 0, st>>>(dActive, dPos, nc);
-            // XC, defects (through free buffers), times, parameters, original indices
-            slv::k_compact_rows<double><<<grid_for(nc * LX), 256, 0, st>>>(dXC, dXS, dPos, dActive, nc, LX);
-            CK(h, cudaMemcpyAsync(dXC, dXS, (size_t)na * LX * 8, cudaMemcpyDeviceToDevice, st));
-            slv::k_compact_rows<double><<<grid_for(nc * LD), 256, 0, st>>>(dDef, dDs, dPos, dActive, nc, LD);
-            CK(h, cudaMemcpyAsync(dDef, dDs, (size_t)na * LD * 8, cudaMemcpyDeviceToDevice, st));
-            slv::k_compact_rows<double><<<grid_for(nc * N), 256, 0, st>>>(dT, dUp, dPos, dActive, nc, N);
-            CK(h, cudaMemcpyAsync(dT, dUp, (size_t)na * N * 8, cudaMemcpyDeviceToDevice, st));
-            if (dTL) { slv::k_compact_rows<double><<<grid_for(nc), 256, 0, st>>>(dTL, dUmax, dPos, dActive, nc, 1); CK(h, cudaMemcpyAsync(dTL, dUmax, (size_t)na * 8, cudaMemcpyDeviceToDevice, st)); }
-            if (dRH) { slv::k_compact_rows<double><<<grid_for(nc), 256, 0, st>>>(dRH, dUmax, dPos, dActive, nc, 1); CK(h, cudaMemcpyAsync(dRH, dUmax, (size_t)na * 8, cudaMemcpyDeviceToDevice, st)); }
-            slv::k_compact_rows<int><<<grid_for(nc), 256, 0, st>>>(dOrig, dOrig2, dPos, dActive, nc, 1);
-            CK(h, cudaMemcpyAsync(dOrig, dOrig2, (size_t)na * 4, cudaMemcpyDeviceToDevice, st));
-            slv::k_set_int<<<slv::nblk((long long)na, 256), 256, 0, st>>>(dActive, 1, (long long)na);      // the compacted work set: all iterating
-            h->launches += 6 + (dTL ? 1 : 0) + (dRH ? 1 : 0);
-        }
-        *n_next = (long long)na;
-        return 0;
-    };
-
-    // ---- first nominal run (:274)
-    rc = defect_pass(dXC, dT, dTL, dRH, nc, dDef); if (rc) return rc;
-    rowmax(dDef, nc, LD, dEr);
-    long long n_next = 0;
-    rc = iter_end(0, &n_next); if (rc) return rc;
-    int it = 0;
-    while (n_next > 0 && it < max_iter) {
-        nc = n_next;                                                      // every row of the work set is iterating
-        ++it;
-        // jacobianCalc (:290): one launch, Phi_i of every segment of every trajectory still iterating (and the defects, unchanged)
-        rc = lto_indirect_dev(h, p, nc * (N - 1), N, ND, dXC, dT, nullptr, nullptr, dTL, dRH, dDef, nullptr, nullptr, dPhi); if (rc) return rc;
-        // optimizeTraj_OLS (:149-183)
-        rc = lto_indirect_newton_nd_dev(h, ND, nc, N, flag_adjointsOnly, dPhi, dDef, dUp, nullptr); if (rc) return rc;
-        // second-order correction (:187-214), only where norm(xc_update, Inf) < 1e-1
-        rowmax(dUp, nc, LX, dUmax);
-        slv::k_soc_mask<<<slv::nblk(nc, 256), 256, 0, st>>>(dUmax, dActive, dMask, nc); h->launches += 1;
-        axpy(dXC, dUp, dMask, dXS, nc, LX, 1);                                                 // XC_all_soc (:194)
-        rc = defect_pass(dXS, dT, dTL, dRH, nc, dDs); if (rc) return rc;                       // :197
-        rc = lto_indirect_newton_resolve_nd_dev(h, ND, nc, N, flag_adjointsOnly, dDs, dUp2, nullptr); if (rc) return rc;   // :207 (same Jacobian: stored reflections replayed)
-        axpy(dUp, dUp2, dMask, dUp, nc, LX, 1);                                                // xc_update += xc_update_soc (:213)
-        // line search (:298-302)
-        const int use_ls = it > 3;
-        if (use_ls) {
-            prepare_trials();
-            axpy(dXC, dUp, dLsTable, dTrX, nc, LX, NA);                                        // XC_all + xc_update*alpha (:235)
-            rc = defect_pass(dTrX, dTrT, dTrTL, dTrRH, (long long)NA * nc, dTrD); if (rc) return rc;   // :238, all 20 x n trial trajectories in one launch
-            rc = lto_sumsq_dev(h, dTrD, (long long)NA * nc, LD, dErs); if (rc) return rc;      // er[ind] = sum(defect[:].^2) (:241)
-        }
-        slv::k_pick_alpha<<<slv::nblk(nc, 256), 256, 0, st>>>(dErs, dAlphaAll, dActive, dAlpha, dScale, nc, use_ls); h->launches += 1;
-        axpy(dXC, dUp, dScale, dXC, nc, LX, 1);                                                // XC_all = XC_all + xc_update*alpha (:304)
-        // the end states cannot have moved (:324-325): their update entries are exact zeros (lto_newton.cu; 14-dim: the 7-element pins)
-        rc = defect_pass(dXC, dT, dTL, dRH, nc, dDef); if (rc) return rc;                      // :328
-        rowmax(dDef, nc, LD, dEr);                                                             // :332
-        rc = iter_end(it, &n_next); if (rc) return rc;
-    }
-    CK(h, cudaEventRecord(h->ev_t1, st));
+    EngineArrays w{};
+    // the hook retires every row whose call ended (every row starts together: one call per trajectory)
+    int rc = indirect_engine(h, p, ndim, T, n_nodes, max_iter, flag_adjointsOnly, XC_all, t_TU, thrustLimit_traj, rho_traj, 0, &w,
+                             [](char*) { return 0; },
+                             [&](long long nc) -> int {
+                                 slv::k_retire_rows<<<std::min<unsigned>(slv::nblk(nc * LX, 256), 148u * 16u), 256, 0, st>>>(w.XC, w.XCout, w.orig, w.active, nc, LX, w.flag);
+                                 slv::k_retire_rows<<<std::min<unsigned>(slv::nblk(nc * LD, 256), 148u * 16u), 256, 0, st>>>(w.Def, w.DefOut, w.orig, w.active, nc, LD);
+                                 h->launches += 2;
+                                 return 0;
+                             });
+    if (rc) return rc;
     // ---- outputs (every trajectory has been retired into the caller-ordered arrays by now)
-    CK(h, cudaMemcpyAsync(XC_all, dXCout, nn * ND * 8, cudaMemcpyDeviceToHost, st));
-    if (defect) CK(h, cudaMemcpyAsync(defect, dDefOut, ns * ND * 8, cudaMemcpyDeviceToHost, st));
-    if (iters) CK(h, cudaMemcpyAsync(iters, dIters, T * 4, cudaMemcpyDeviceToHost, st));
-    if (er_out) CK(h, cudaMemcpyAsync(er_out, dErOut, T * 8, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(XC_all, w.XCout, nn * ndim * 8, cudaMemcpyDeviceToHost, st));
+    if (defect) CK(h, cudaMemcpyAsync(defect, w.DefOut, ns * ndim * 8, cudaMemcpyDeviceToHost, st));
+    if (iters) CK(h, cudaMemcpyAsync(iters, w.iters, T * 4, cudaMemcpyDeviceToHost, st));
+    if (er_out) CK(h, cudaMemcpyAsync(er_out, w.ErOut, T * 8, cudaMemcpyDeviceToHost, st));
     std::vector<int32_t> flag((size_t)T);
-    CK(h, cudaMemcpyAsync(flag.data(), dFlag, T * 4, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(flag.data(), w.flag, T * 4, cudaMemcpyDeviceToHost, st));
     CK(h, cudaStreamSynchronize(st));
     float ms = 0.f; CK(h, cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1)); h->last_ms = ms;
     if (status_flag) {
         for (long long j = 0; j < T; ++j) status_flag[j] = flag[(size_t)j];                    // (non-finite nodes were flagged when the row was retired)
     }
+    return LTO_SUCCESS;
+}
+
+// reduceFuel_indirect (HelperFunctions.jl:105-193) for n_traj independent ladders (lto_ladder.h), every solver call on the device:
+// maxIter = max_iter, p = 1, flag_adjointsOnly = false.  A ladder's next call enters the work set as soon as its last one ends.
+int lto_indirect_reduce_fuel_batch(lto_handle* h, const lto_indirect_params* p, int ndim, int64_t n_traj, int n_nodes, int max_iter,
+                                   double* XC_all, const double* t_TU, const double* thrustLimit_traj, const double* rho_current,
+                                   const double* rho_target, const double* backoff_uniform, double* defect, int32_t* status,
+                                   int32_t* calls, int32_t* newton_iters, double* rho_last) {
+    LTO_NVTX();
+    if (!h) return fail(nullptr, LTO_ERR_ARG, "null handle");
+    if (!p) return fail(h, LTO_ERR_ARG, "null params");
+    if (p->p != 1.0) return fail(h, LTO_ERR_ARG, "the rho continuation needs p = 1 (got p = %g)", p->p);
+    if (!valid_ndim(ndim)) return fail(h, LTO_ERR_ARG, "ndim must be 12 or 14 (got %d)", ndim);
+    if (n_traj < 0) return fail(h, LTO_ERR_ARG, "negative trajectory count");
+    if (n_nodes < 2) return fail(h, LTO_ERR_ARG, "n_nodes must be >= 2");
+    if (max_iter < 0) return fail(h, LTO_ERR_ARG, "negative max_iter");
+    if (n_traj == 0) return LTO_SUCCESS;
+    if (!XC_all || !t_TU || !rho_current || !rho_target || !backoff_uniform || !defect || !status) return fail(h, LTO_ERR_ARG, "null array argument");
+    if (h->n_child > 0) {
+        const long long N = n_nodes;
+        return split_trajectories(h, n_traj, [&](lto_handle* c, long long u0, long long nu) {
+            return lto_indirect_reduce_fuel_batch(c, p, ndim, nu, n_nodes, max_iter, XC_all + u0 * N * ndim, t_TU + u0 * N,
+                                                  thrustLimit_traj ? thrustLimit_traj + u0 : nullptr, rho_current + u0, rho_target + u0,
+                                                  backoff_uniform + u0 * LADDER_DRAWS, defect + u0 * (N - 1) * ndim, status + u0,
+                                                  calls ? calls + u0 : nullptr, newton_iters ? newton_iters + u0 : nullptr,
+                                                  rho_last ? rho_last + u0 : nullptr);
+        });
+    }
+    CK(h, cudaSetDevice(h->device));
+    const long long T = n_traj, N = n_nodes, ns = T * (N - 1), nn = T * N;
+    if (T > 0x7fffffffll) return fail(h, LTO_ERR_ARG, "too many trajectories");
+    const long long LX = N * ndim, LD = (N - 1) * ndim;
+    cudaStream_t st = h->s_compute;
+    // caller-ordered ladder arrays after the engine's: accepted starts, ladder states, draws, rho targets, the outputs
+    const size_t bAcc = al(nn * ndim * 8), bLad = al(T * sizeof(LadderState)), bDraw = al(T * LADDER_DRAWS * 8), bVec = al(T * 8), bInt = al(T * 4);
+    double* dAcc = nullptr; LadderState* dLad = nullptr; double* dDraw = nullptr; double* dTgt = nullptr; double* dRhoLast = nullptr;
+    int* dStatus = nullptr; int* dCalls = nullptr; int* dNit = nullptr;
+    EngineArrays w{};
+    int rc = indirect_engine(h, p, ndim, T, n_nodes, max_iter, 0, XC_all, t_TU, thrustLimit_traj, rho_current,
+                             bAcc + bLad + bDraw + bVec * 2 + bInt * 3, &w,
+                             [&](char* q) -> int {
+                                 dAcc = (double*)q; q += bAcc; dLad = (LadderState*)q; q += bLad; dDraw = (double*)q; q += bDraw;
+                                 dTgt = (double*)q; q += bVec; dRhoLast = (double*)q; q += bVec;
+                                 dStatus = (int*)q; q += bInt; dCalls = (int*)q; q += bInt; dNit = (int*)q;
+                                 CK(h, cudaMemcpyAsync(dAcc, w.XC, nn * ndim * 8, cudaMemcpyDeviceToDevice, st));      // the first start
+                                 CK(h, cudaMemcpyAsync(dDraw, backoff_uniform, T * LADDER_DRAWS * 8, cudaMemcpyHostToDevice, st));
+                                 CK(h, cudaMemcpyAsync(dTgt, rho_target, T * 8, cudaMemcpyHostToDevice, st));
+                                 slv::k_ladder_init<<<slv::nblk(T, 256), 256, 0, st>>>(w.RH, dTgt, dLad, dCalls, dNit, T);
+                                 h->launches += 1;
+                                 return 0;
+                             },
+                             [&](long long nc) -> int {
+                                 slv::k_ladder_hook<<<slv::nblk(nc * 32, 256), 256, 0, st>>>(w.XC, w.Def, w.RH, w.active, w.orig, w.wit, w.iters, w.flag,
+                                                                                        dLad, dDraw, dAcc, w.XCout, w.DefOut, dStatus, dCalls, dNit,
+                                                                                        dRhoLast, w.count, nc, LX, LD);
+                                 h->launches += 1;
+                                 return 0;
+                             });
+    if (rc) return rc;
+    CK(h, cudaMemcpyAsync(XC_all, w.XCout, nn * ndim * 8, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(defect, w.DefOut, ns * ndim * 8, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(status, dStatus, T * 4, cudaMemcpyDeviceToHost, st));
+    if (calls) CK(h, cudaMemcpyAsync(calls, dCalls, T * 4, cudaMemcpyDeviceToHost, st));
+    if (newton_iters) CK(h, cudaMemcpyAsync(newton_iters, dNit, T * 4, cudaMemcpyDeviceToHost, st));
+    if (rho_last) CK(h, cudaMemcpyAsync(rho_last, dRhoLast, T * 8, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaStreamSynchronize(st));
+    float ms = 0.f; CK(h, cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1)); h->last_ms = ms;
     return LTO_SUCCESS;
 }
 

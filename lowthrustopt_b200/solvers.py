@@ -91,6 +91,11 @@ class GpuBackend:
         return self.h.indirect_solve_batch(XC, t, params=self._ip(params), thrustLimit=thrustLimit, rho=rho, max_iter=max_iter,
                                            flag_adjointsOnly=flag_adjointsOnly)
 
+    def indirect_reduce_fuel_batch(self, XC, t, params, rho_current, rho_target, backoff_uniform, thrustLimit=None, max_iter=10):
+        self.calls += 1
+        return self.h.indirect_reduce_fuel_batch(XC, t, rho_current, rho_target, backoff_uniform, params=self._ip(params),
+                                                 thrustLimit=thrustLimit, max_iter=max_iter)
+
 
 _default_backend = None
 
@@ -555,19 +560,35 @@ def reduceFuel_indirect(XC_all, t_TU, MU, DU, TU, n_nodes, mass, thrustLimit, rh
 
 
 def reduceFuel_indirect_batch(XC_all, t_TU, MU, DU, TU, n_nodes, mass, thrustLimit, rho_current, rho_target, backend=None, rngs=None,
-                              log=None, Isp=2000.0):
+                              log=None, Isp=2000.0, device_ladder=False):
     """reduceFuel_indirect for a BATCH of independent trajectories (SURVEY 8(f) row 3): every trajectory walks its own rho ladder
     (halving on success, x 3(1 + rand) back-off on failure, :155-187); each round, the solver calls all unfinished trajectories
     ask for are issued as ONE lto_indirect_solve_batch call with per-trajectory rho / thrustLimit.
     XC_all: (n_traj, m, n_nodes), m = 12 or 14 (`Isp` enters the mass flow of the 14-dim system); t_TU: (n_traj, n_nodes);
     thrustLimit, rho_current, rho_target: scalars or (n_traj,).
-    Returns (XC_new (n_traj, m, n_nodes), defect (n_traj, m, n_nodes-1), status (n_traj,), rounds)."""
+    Returns (XC_new (n_traj, m, n_nodes), defect (n_traj, m, n_nodes-1), status (n_traj,), rounds).
+    device_ladder: run the whole ladder in ONE device call (lto_indirect_reduce_fuel_batch): a trajectory's next solver call starts
+    as soon as its last one ends.  Same results; each trajectory's 100 back-off draws are taken up front with rng.random(100), the
+    same values as its successive rng.random() calls.  `rounds` is then the most solver calls any trajectory made, the round count
+    of the default driver; `log` is not supported."""
     be = backend or default_backend()
     XC_all = np.asarray(XC_all, dtype=np.float64); t_TU = np.asarray(t_TU, dtype=np.float64)
     T = XC_all.shape[0]
     tl = np.broadcast_to(np.asarray(thrustLimit, dtype=np.float64), (T,)).copy()
     r0 = np.broadcast_to(np.asarray(rho_current, dtype=np.float64), (T,)); r1 = np.broadcast_to(np.asarray(rho_target, dtype=np.float64), (T,))
     rngs = rngs or [np.random.default_rng(j) for j in range(T)]
+    if device_ladder:
+        if log is not None:
+            raise ValueError("log is not available with device_ladder=True: the ladder has no rounds on the device")
+        m = XC_all.shape[1]
+        if m not in (12, 14):
+            raise ValueError("XC_all must be (n_traj, 12 or 14, n_nodes) (got %s)" % (XC_all.shape,))
+        draws = np.array([rngs[j].random(100) for j in range(T)], dtype=np.float64).reshape(T, 100)
+        params = (MU, DU, TU, float(tl[0]) if T else 0.0, mass, 1.0, 1.0, 1.0) + ((Isp,) if m == 14 else ())
+        r = be.indirect_reduce_fuel_batch(np.ascontiguousarray(XC_all.transpose(0, 2, 1)), t_TU, params, r0, r1, draws, thrustLimit=tl,
+                                          max_iter=10)
+        rounds = int(r["calls"].max()) if T else 0
+        return r["XC_all"].transpose(0, 2, 1).copy(), r["defect"].transpose(0, 2, 1).copy(), r["status"], rounds
     gens = [_reduceFuel_steps(XC_all[j].copy(), float(r0[j]), float(r1[j]), rngs[j]) for j in range(T)]
     req = {j: next(gens[j]) for j in range(T)}
     res = [None] * T
