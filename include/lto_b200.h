@@ -303,6 +303,25 @@ int lto_direct_solve_batch(lto_handle* h, const lto_direct_params* p, int64_t n_
                            double* X_all, double* u_all, const double* t_TU, const double* state_0, const double* state_f, double mass,
                            double* defect, int32_t* iters, double* er_out);
 
+/* lto_stack_guess_batch: the demos' trajectory-stacking initial guess (CRTBP_Multishoot_direct_demo.jl:117-157, with interpInitialStates /
+ * find_τ of src/HelperFunctions.jl:18-48) for n_traj transfers in one call, every stage on the device.  Per trajectory j:
+ *   state_0 = spline(X0)(tau1[j]);  arc 1 = [state_0; 0] propagated from t_TU[0] to every node with t_TU < t_split (strict) and to t_split;
+ *   tau2_0 = find_τ(Xf, arc-1 end);  arc 2 = [spline(Xf)(tau2_0); 0] from t_split to every remaining node and to t_TU[end];
+ *   tau2 = find_τ(Xf, arc-2 end);  state_f = spline(Xf)(tau2);  XC_all = the arcs at the nodes, node 0 [state_0; 0], the last [state_f; 0].
+ * spline(X): a natural cubic spline per row of the 6 x n table on LinRange(0, 1, n) (n >= 3), tau wrapped by +-1 steps into [0, 1];
+ * find_τ: the first of tau = 0, 0.001, ..., 1 whose spline state is nearest (Euclidean) to the given state.  The arcs integrate the
+ * 12-dim system with p as given and no STM (zero costates: the control is zero, the arcs are ballistic for any thrustLimit).
+ *   X0_states, Xf_states  6 x n0, 6 x nf column-major orbit tables (finite)
+ *   tau1, t_split         n_traj each: |tau1| <= 1e3, t_TU[0] < t_split <= t_TU[end]
+ *   t_TU                  n_nodes per trajectory, finite and strictly increasing (n_nodes >= 2)
+ *   XC_all                out, 12 x n_nodes per trajectory;  tau2: out, n_traj;  state_0, state_f: out, 6 per trajectory
+ *   status                out, n_traj (may be NULL): the worst LTO_ST_* (largest code) of the trajectory's arc segments
+ * A bad argument is LTO_ERR_ARG naming the first offending trajectory.  Multi-device handles split whole trajectories. */
+int lto_stack_guess_batch(lto_handle* h, const lto_indirect_params* p, int64_t n_traj, int n_nodes,
+                          const double* X0_states, int n0, const double* Xf_states, int nf,
+                          const double* tau1, const double* t_TU, const double* t_split,
+                          double* XC_all, double* tau2, double* state_0, double* state_f, int32_t* status);
+
 /* ---- peer memory: one process per GPU, results delivered to the solver rank without a collective --------
  * The rank that runs the Newton step allocates its full output arrays with lto_dev_alloc and exports them
  * (lto_ipc_export: a 64-byte cudaIpcMemHandle_t to send to the other processes by any means); every other rank

@@ -186,4 +186,20 @@ function multiShoot_CRTBP_direct_batch(X_batch::Array{Float64,3}, u_batch::Array
         handle[], p, n_traj, n_nodes, nstate, nsteps, maxIter, X, u, t_batch, state_0, state_f, mass, defect, iters, er))
     (X, u, defect, iters)
 end
+# ---- trajectory stacking (CRTBP_Multishoot_direct_demo.jl:117-157) for a BATCH of transfers in ONE call: splines, both ballistic arcs and
+# both find_τ scans on the device.  X0_states / Xf_states: the 6 x n orbit tables; tau1, t_split: per transfer; t_batch: n_nodes x n_traj.
+# Returns (XC 12 x n_nodes x n_traj, tau2, state_0 6 x n_traj, state_f 6 x n_traj, status); XC[1:6, :, :], state_0 and state_f feed
+# multiShoot_CRTBP_direct_batch below.  Like the rest of this shim, not run under Julia here (the same ABI is exercised from Python).
+function trajectory_stack_guess_batch(X0_states::Matrix{Float64}, Xf_states::Matrix{Float64}, tau1::Vector{Float64}, t_batch::Matrix{Float64},
+                                      t_split::Vector{Float64}, MU, DU, TU)
+    n_nodes = size(t_batch, 1); n_traj = size(t_batch, 2)
+    XC = zeros(12, n_nodes, n_traj); tau2 = zeros(n_traj); state_0 = zeros(6, n_traj); state_f = zeros(6, n_traj); status = zeros(Int32, n_traj)
+    prm = iparams((MU, DU, TU, 0.0, 1e3, 1.0, 1.0, 1.0))
+    GC.@preserve X0_states Xf_states tau1 t_batch t_split XC tau2 state_0 state_f status check(ccall((:lto_stack_guess_batch, lib), Cint,
+        (Ptr{Cvoid}, Ref{IndirectParams}, Int64, Cint, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+        handle[], prm, n_traj, n_nodes, X0_states, size(X0_states, 2), Xf_states, size(Xf_states, 2), tau1, t_batch, t_split,
+        XC, tau2, state_0, state_f, status))
+    (XC, tau2, state_0, state_f, status)
+end
 end # module

@@ -32,7 +32,7 @@ EXPORTS = [
     "lto_push_async", "lto_sync_copies", "lto_signal_dev", "lto_wait_dev", "lto_fp64_peak_probe", "lto_debug_profile",
     "lto_indirect_newton", "lto_indirect_newton_dev", "lto_indirect_newton_resolve_dev", "lto_indirect_solve_batch", "lto_direct_qp", "lto_direct_qp_dev", "lto_direct_solve_batch",
     "lto_indirect_newton_nd", "lto_indirect_newton_nd_dev", "lto_indirect_newton_resolve_nd_dev", "lto_indirect_solve_batch_nd",
-    "lto_indirect_reduce_fuel_batch",
+    "lto_indirect_reduce_fuel_batch", "lto_stack_guess_batch",
 ]
 
 
@@ -117,6 +117,7 @@ def lib():
         L.lto_direct_qp.argtypes = [vp, i64, ci, ci] + [vp] * 9
         L.lto_direct_qp_dev.argtypes = [vp, i64, ci, ci] + [vp] * 9
         L.lto_direct_solve_batch.argtypes = [vp, vp, i64, ci, ci, ci, ci] + [vp] * 5 + [C.c_double] + [vp] * 3
+        L.lto_stack_guess_batch.argtypes = [vp, vp, i64, ci, vp, ci, vp, ci] + [vp] * 3 + [vp] * 5
         _lib = L
     return _lib
 
@@ -606,3 +607,26 @@ class Handle:
         self._ck(lib().lto_direct_solve_batch(self._h, C.addressof(p), n_traj, n_nodes, ns, int(nsteps), int(max_iter), _ptr(X), _ptr(U), _ptr(t_TU),
                                               _ptr(state_0), _ptr(state_f), float(mass), _ptr(defect), _ptr(iters), _ptr(er)))
         return dict(X_all=X, u_all=U, defect=defect, iters=iters, er=er)
+
+    # ---- the trajectory-stacking initial guess on the device ----
+    def stack_guess_batch(self, X0_states, Xf_states, tau1, t_TU, t_split, params=None):
+        """The demos' trajectory-stacking guess (CRTBP_Multishoot_direct_demo.jl:117-157, solvers.trajectory_stack_guess) for n_traj
+        transfers in one device call (lto_stack_guess_batch).  X0_states, Xf_states: the reference's (6, n) orbit tables; tau1, t_split:
+        (n_traj,); t_TU: (n_traj, n_nodes).  params: the arcs' indirect parameters, by default the host mirror's
+        (thrustLimit 0, mass 1e3, p = rho = 1).
+        Returns dict(XC_all (n_traj, n_nodes, 12), tau2 (n_traj,), state_0 (n_traj, 6), state_f (n_traj, 6), status (n_traj,))."""
+        p = params or indirect_params(thrustLimit=0.0, mass=1e3, time_direction=1.0, p=1.0, rho=1.0)
+        X0, Xf = _f64(X0_states), _f64(Xf_states)
+        if X0.ndim != 2 or X0.shape[0] != 6 or Xf.ndim != 2 or Xf.shape[0] != 6:
+            raise ValueError("X0_states and Xf_states must be (6, n) orbit tables (got %s, %s)" % (X0.shape, Xf.shape))
+        t_TU = _f64(t_TU)
+        if t_TU.ndim != 2:
+            raise ValueError("t_TU must be (n_traj, n_nodes) (got %s)" % (t_TU.shape,))
+        n_traj, n_nodes = t_TU.shape
+        tau1 = _shaped("tau1", tau1, (n_traj,)); t_split = _shaped("t_split", t_split, (n_traj,))
+        X0c, Xfc = np.ascontiguousarray(X0.T), np.ascontiguousarray(Xf.T)                # column-major 6 x n
+        XC = np.empty((n_traj, n_nodes, 12)); tau2 = np.empty(n_traj); s0 = np.empty((n_traj, 6)); sf = np.empty((n_traj, 6))
+        status = np.empty(n_traj, dtype=np.int32)
+        self._ck(lib().lto_stack_guess_batch(self._h, C.addressof(p), n_traj, n_nodes, _ptr(X0c), X0.shape[1], _ptr(Xfc), Xf.shape[1], _ptr(tau1),
+                                             _ptr(t_TU), _ptr(t_split), _ptr(XC), _ptr(tau2), _ptr(s0), _ptr(sf), _ptr(status)))
+        return dict(XC_all=XC, tau2=tau2, state_0=s0, state_f=sf, status=status)

@@ -1,11 +1,14 @@
 // lto_handle.h -- the library handle and the error helpers shared by the C ABI translation units
-// (lto_capi.cu: propagation entry points; lto_solve.cu: Newton update / batched solver entry points).
+// (lto_capi.cu: propagation entry points; lto_solve.cu: Newton update / batched solver entry points; lto_guess.cu: the batched
+// trajectory-stacking guess).
 #pragma once
 #include "../../include/lto_b200.h"
 #include <cuda_runtime.h>
 #include <nvtx3/nvToolsExt.h>
 #include <stddef.h>
 #include <stdint.h>
+#include <thread>
+#include <vector>
 
 static const size_t LTO_PROF_WORDS = 16384;
 #define LTO_MAX_DEVICES 16
@@ -53,3 +56,21 @@ int lto_ensure(lto_handle* h, void** p, size_t* cap, size_t need);      // grow-
     } while (0)
 
 static inline size_t al(size_t x) { return (x + 255) & ~(size_t)255; }
+
+// Multi-device handles (lto_init_devices): whole trajectories in equal contiguous ranges, one host worker thread per device;
+// every device copies its slab of the results straight into the caller's arrays.
+template <class F>
+static inline int split_trajectories(lto_handle* h, long long n_traj, F&& call) {
+    const int nc = h->n_child;
+    std::vector<int> rcs(nc, 0);
+    std::vector<std::thread> th;
+    for (int i = 0; i < nc; ++i) {
+        const long long u0 = n_traj * i / nc, u1 = n_traj * (i + 1) / nc;
+        if (u1 <= u0) continue;
+        th.emplace_back([&, i, u0, u1] { rcs[i] = call(h->child[i], u0, u1 - u0); });
+    }
+    for (auto& t : th) t.join();
+    for (int i = 0; i < nc; ++i)
+        if (rcs[i]) return fail(h, rcs[i], "device %d: %s", h->child[i]->device, h->child[i]->err);
+    return LTO_SUCCESS;
+}

@@ -317,24 +317,6 @@ static inline unsigned nblk(long long n, int t) { return (unsigned)((n + t - 1) 
 
 using namespace lto;
 
-// Multi-device handles (lto_init_devices): whole trajectories in equal contiguous ranges, one host worker thread per device;
-// every device copies its slab of the results straight into the caller's arrays.
-template <class F>
-static int split_trajectories(lto_handle* h, long long n_traj, F&& call) {
-    const int nc = h->n_child;
-    std::vector<int> rcs(nc, 0);
-    std::vector<std::thread> th;
-    for (int i = 0; i < nc; ++i) {
-        const long long u0 = n_traj * i / nc, u1 = n_traj * (i + 1) / nc;
-        if (u1 <= u0) continue;
-        th.emplace_back([&, i, u0, u1] { rcs[i] = call(h->child[i], u0, u1 - u0); });
-    }
-    for (auto& t : th) t.join();
-    for (int i = 0; i < nc; ++i)
-        if (rcs[i]) return fail(h, rcs[i], "device %d: %s", h->child[i]->device, h->child[i]->err);
-    return LTO_SUCCESS;
-}
-
 // ---- the iteration engine of the batched indirect solver (multiShoot_CRTBP_indirect :254-345, p as given) ----
 // The work set holds the trajectories whose solver call is running, compacted to the front after every step; every row has
 // its own iteration counter wit[j] (-1: the call has just started and waits for its nominal pass).  When a row's call ends,

@@ -4,7 +4,8 @@
     multiShoot_CRTBP_direct      src/multiShoot_CRTBP_direct.jl:58-594   (+ multiShoot_CRTBP_direct_batch: many trajectories, QP on the device)
     multiShoot_CRTBP_indirect    src/multiShoot_CRTBP_indirect.jl:58-345
     reduceFuel_indirect          src/HelperFunctions.jl:105-193   (+ reduceFuel_indirect_batch: many trajectories, one device call per round)
-    trajectory_stack_guess       CRTBP_Multishoot_direct_demo.jl:117-157
+    trajectory_stack_guess       CRTBP_Multishoot_direct_demo.jl:117-157   (+ trajectory_stack_guess_batch: many transfers in one device call,
+                                                                        direct_transfer_sweep: those guesses solved by the batched direct solver)
     densify, jacobiConstant, interpInitialStates, find_tau   src/HelperFunctions.jl:10-101
 
 Same names, argument order and return values.  Arrays use the reference's shapes
@@ -95,6 +96,16 @@ class GpuBackend:
         self.calls += 1
         return self.h.indirect_reduce_fuel_batch(XC, t, rho_current, rho_target, backoff_uniform, params=self._ip(params),
                                                  thrustLimit=thrustLimit, max_iter=max_iter)
+
+    def stack_guess_batch(self, X0_states, Xf_states, tau1, t_TU, t_split, params):
+        """trajectory_stack_guess for many transfers in one device call (lto_stack_guess_batch); params = the reference's tuple."""
+        self.calls += 1
+        return self.h.stack_guess_batch(X0_states, Xf_states, tau1, t_TU, t_split, params=self._ip(params))
+
+    def direct_solve_batch(self, X, U, t, state_0, state_f, mass, nsteps, max_iter, Isp, MU, DU, TU):
+        self.calls += 1
+        return self.h.direct_solve_batch(X, U, t, state_0, state_f, mass=mass, nsteps=nsteps, max_iter=max_iter,
+                                         params=capi.direct_params(Isp=Isp, MU_=MU, DU_=DU, TU_=TU))
 
 
 _default_backend = None
@@ -212,6 +223,65 @@ def trajectory_stack_guess(X0_states, Xf_states, MU=capi.MU, DU=capi.DU, TU=capi
     XC[:, 0] = state_0
     XC[:, -1] = state_f
     return XC, t_TU, tau1, tau2, state_0, state_f
+
+
+def trajectory_stack_guess_batch(X0_states, Xf_states, MU=capi.MU, DU=capi.DU, TU=capi.TU, n_nodes=30, tof1_days=10.0, tof2_days=10.0,
+                                 tau1=0.75, backend=None):
+    """trajectory_stack_guess for a BATCH of transfers in one device call (lto_stack_guess_batch): the spline lookups, both ballistic
+    arcs and both find_tau scans of every transfer run on the device.  tau1, tof1_days, tof2_days: scalars or (T,) arrays; per row the
+    same arithmetic as trajectory_stack_guess (t_TU = linspace(0, tof1 + tof2, n_nodes), the arcs split at tof1).
+    Returns (XC (T, 12, n_nodes), t_TU (T, n_nodes), tau1 (T,), tau2 (T,), state_0 (T, 12), state_f (T, 12))."""
+    be = backend or default_backend()
+    tau1, tof1_days, tof2_days = np.broadcast_arrays(*[np.atleast_1d(np.asarray(a, dtype=np.float64)) for a in (tau1, tof1_days, tof2_days)])
+    if tau1.ndim != 1:
+        raise ValueError("tau1, tof1_days and tof2_days must be scalars or (T,) arrays")
+    T = tau1.shape[0]
+    t_TU = np.empty((T, n_nodes)); t_split = np.empty(T)
+    for j in range(T):
+        tof1 = float(tof1_days[j]) * DAY / TU; tof2 = float(tof2_days[j]) * DAY / TU
+        t_TU[j] = np.linspace(0.0, tof1 + tof2, n_nodes)
+        t_split[j] = tof1
+    tau1 = np.ascontiguousarray(tau1)
+    r = be.stack_guess_batch(X0_states, Xf_states, tau1, t_TU, t_split, (MU, DU, TU, 0.0, 1e3, 1.0, 1.0, 1.0))
+    z = np.zeros((T, 6))
+    return (r["XC_all"].transpose(0, 2, 1).copy(), t_TU, tau1.copy(), r["tau2"], np.concatenate([r["state_0"], z], axis=1),
+            np.concatenate([r["state_f"], z], axis=1))
+
+
+def _quad_cost(u_all, t_TU):
+    """quadCost of optimizeTraj (multiShoot_CRTBP_direct.jl:367-368, dV = 0) at the controls u_all (T, 3, N): the node weights dt_temp
+    of _qp_direct (:323-325) on the solver's fixed time grid."""
+    t0 = t_TU[:, :1]; tf = t_TU[:, -1:]
+    tau = (t_TU - t0) / (tf - t0) * 2 - 1
+    t_fixed = t0 + (tau + 1) / 2 * (tf - t0)
+    dt = np.diff(t_fixed, axis=1)
+    z = np.zeros((t_TU.shape[0], 1))
+    w = np.concatenate([dt / 2, dt[:, -1:] / 2], axis=1) + np.concatenate([z, dt[:, :-1] / 2, z], axis=1)
+    return np.sum(u_all ** 2 * w[:, None, :], axis=(1, 2))
+
+
+def direct_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, n_nodes=30, nsteps=10, nstate=6, mass=1e3, Isp=2000.0,
+                          maxIter=100, backend=None):
+    """A trade study over departure phase and flight times: the trajectory-stacking guesses of every (tau1, tof1_days, tof2_days) row
+    (trajectory_stack_guess_batch), then multiShoot_CRTBP_direct on all of them at once on the device (lto_direct_solve_batch; the demo's
+    setting: flagEnd = false, allowImpulsive = false, u_all = 0 to start, nstate 7 adds a mass row of `mass`).  Two library calls.
+    Returns dict(X_all (T, nstate, N), u_all (T, 3, N), t_TU (T, N), tau2 (T,), iters (T,), er (T,), converged (T,) = er <= 1e-6,
+    cost (T,) = quadCost at the returned controls)."""
+    be = backend or default_backend()
+    MU, DU, TU = capi.MU, capi.DU, capi.TU
+    if nstate not in (6, 7):
+        raise ValueError("nstate must be 6 or 7 (got %r)" % (nstate,))
+    XC, t_TU, tau1, tau2, s0, sf = trajectory_stack_guess_batch(X0_states, Xf_states, MU, DU, TU, n_nodes, tof1_days, tof2_days, tau1,
+                                                                backend=be)
+    T = XC.shape[0]
+    X = XC[:, :6].transpose(0, 2, 1)
+    if nstate == 7:
+        X = np.concatenate([X, np.full((T, n_nodes, 1), float(mass))], axis=2)
+    r = be.direct_solve_batch(np.ascontiguousarray(X), np.zeros((T, n_nodes, 3)), t_TU, np.ascontiguousarray(s0[:, :6]),
+                              np.ascontiguousarray(sf[:, :6]), mass, nsteps, maxIter, Isp, MU, DU, TU)
+    u_all = r["u_all"].transpose(0, 2, 1).copy()
+    return dict(X_all=r["X_all"].transpose(0, 2, 1).copy(), u_all=u_all, t_TU=t_TU, tau2=tau2, iters=r["iters"], er=r["er"],
+                converged=r["er"] <= 1e-6, cost=_quad_cost(u_all, t_TU))
 
 
 # --------------------------------------------------------------------------- direct method
