@@ -322,6 +322,26 @@ int lto_stack_guess_batch(lto_handle* h, const lto_indirect_params* p, int64_t n
                           const double* tau1, const double* t_TU, const double* t_split,
                           double* XC_all, double* tau2, double* state_0, double* state_f, int32_t* status);
 
+/* lto_indirect_cost_batch: the control cost of n_traj 12-dim indirect trajectories (trajectory form, as lto_indirect_defect_traj) in one
+ * call.  Every segment is integrated by the defect-only kernel K4 with two quadratures riding on its accepted steps, with the weights b
+ * of the 8th-order update: int |a_u| dt and int |a_u|^2 dt, |a_u| = the control law's thrust-acceleration magnitude
+ * (CRTBP_stateCostate_deriv.jl:36-53; 0 where |lv| = 0).  They are not in the error norm, so the steps and states are bitwise those of
+ * lto_indirect_defect_traj; a trajectory's segments are summed in segment order, so its result does not depend on the batch around it.
+ *   XC_all, t_TU, thrustLimit_traj, rho_traj: as lto_indirect_defect_traj with ndim = 12 (t_TU finite and non-decreasing)
+ *   dv        out, n_traj: int |a_u| dt * DU 1e3 / TU, in m/s
+ *   energy    out, n_traj: int (|a_u| mass DU 1e3 / TU^2)^2 dt, in N^2 TU (the units of the direct method's quadCost)
+ *   defect    out, 12 x (n_nodes-1) per trajectory, the same output lto_indirect_defect_traj produces; may be NULL
+ *   status    out, n_traj: the worst LTO_ST_* (largest code) of the trajectory's segments; may be NULL.  A trajectory with a segment
+ *             whose status is not LTO_ST_OK has dv = energy = NaN (that segment never reached its end time)
+ * The reference has no cost arithmetic to compare against: the quadrature is pinned by the constant-thrust closed form (p = 0) and an
+ * independent DOP853 integration of the augmented 14-component system (tests/test_gpu_transfer_cost.py).
+ * p->controller must be LTO_CTRL_RMS and p->kernel not LTO_KERNEL_GENERIC (the quadrature lives in K4): otherwise LTO_ERR_ARG, as for a
+ * reversed or non-finite span (naming the first offending trajectory).  Multi-device handles split whole trajectories. */
+int lto_indirect_cost_batch(lto_handle* h, const lto_indirect_params* p, int64_t n_traj, int n_nodes,
+                            const double* XC_all, const double* t_TU,
+                            const double* thrustLimit_traj, const double* rho_traj,
+                            double* dv, double* energy, double* defect, int32_t* status);
+
 /* ---- peer memory: one process per GPU, results delivered to the solver rank without a collective --------
  * The rank that runs the Newton step allocates its full output arrays with lto_dev_alloc and exports them
  * (lto_ipc_export: a 64-byte cudaIpcMemHandle_t to send to the other processes by any means); every other rank

@@ -202,4 +202,19 @@ function trajectory_stack_guess_batch(X0_states::Matrix{Float64}, Xf_states::Mat
         XC, tau2, state_0, state_f, status))
     (XC, tau2, state_0, state_f, status)
 end
+# ---- control cost of 12-dim indirect trajectories in ONE call (lto_indirect_cost_batch): the defect-only kernel's steps with the quadratures
+# of |a_u| and |a_u|^2 on them.  XC_batch: 12 x n_nodes x n_traj; t_batch: n_nodes x n_traj; thrustLimit, rho: per trajectory.
+# Returns (dv in m/s, energy in N^2 TU, status).  Like the rest of this shim, not run under Julia here (the same ABI is exercised from Python).
+function indirect_cost_batch(XC_batch::Array{Float64,3}, t_batch::Matrix{Float64}, MU, DU, TU, mass, thrustLimit::Vector{Float64}, p,
+                             rho::Vector{Float64})
+    n_nodes = size(XC_batch, 2); n_traj = size(XC_batch, 3)
+    size(XC_batch, 1) == 12 || error("indirect_cost_batch: XC_batch must have 12 rows (the 14-dim cost is exact from the node masses)")
+    dv = zeros(n_traj); energy = zeros(n_traj); status = zeros(Int32, n_traj)
+    prm = iparams((MU, DU, TU, thrustLimit[1], mass, 1.0, p, rho[1]))
+    GC.@preserve XC_batch t_batch thrustLimit rho dv energy status check(ccall((:lto_indirect_cost_batch, lib), Cint,
+        (Ptr{Cvoid}, Ref{IndirectParams}, Int64, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Int32}),
+        handle[], prm, n_traj, n_nodes, XC_batch, t_batch, thrustLimit, rho, dv, energy, C_NULL, status))
+    (dv, energy, status)
+end
 end # module

@@ -32,7 +32,7 @@ EXPORTS = [
     "lto_push_async", "lto_sync_copies", "lto_signal_dev", "lto_wait_dev", "lto_fp64_peak_probe", "lto_debug_profile",
     "lto_indirect_newton", "lto_indirect_newton_dev", "lto_indirect_newton_resolve_dev", "lto_indirect_solve_batch", "lto_direct_qp", "lto_direct_qp_dev", "lto_direct_solve_batch",
     "lto_indirect_newton_nd", "lto_indirect_newton_nd_dev", "lto_indirect_newton_resolve_nd_dev", "lto_indirect_solve_batch_nd",
-    "lto_indirect_reduce_fuel_batch", "lto_stack_guess_batch",
+    "lto_indirect_reduce_fuel_batch", "lto_stack_guess_batch", "lto_indirect_cost_batch",
 ]
 
 
@@ -118,6 +118,7 @@ def lib():
         L.lto_direct_qp_dev.argtypes = [vp, i64, ci, ci] + [vp] * 9
         L.lto_direct_solve_batch.argtypes = [vp, vp, i64, ci, ci, ci, ci] + [vp] * 5 + [C.c_double] + [vp] * 3
         L.lto_stack_guess_batch.argtypes = [vp, vp, i64, ci, vp, ci, vp, ci] + [vp] * 3 + [vp] * 5
+        L.lto_indirect_cost_batch.argtypes = [vp, vp, i64, ci] + [vp] * 4 + [vp] * 4
         _lib = L
     return _lib
 
@@ -442,6 +443,35 @@ class Handle:
         self._ck(lib().lto_indirect_defect_traj(self._h, C.addressof(p), n_traj, n_nodes, nd, _ptr(XC_all), _ptr(t_TU), _ptr(tl),
                                                 _ptr(rh), _ptr(defect), _ptr(status), _ptr(nst)))
         return dict(defect=defect, status=status, nsteps=nst)
+
+    def indirect_cost_batch(self, XC_all, t_TU, params=None, thrustLimit=None, rho=None, defect=False):
+        """Control cost of 12-dim indirect trajectories in one device call (lto_indirect_cost_batch): the defect-only kernel's steps with
+        the quadratures of |a_u| and |a_u|^2 on them.  XC_all: (n_traj, n_nodes, 12); t_TU: (n_traj, n_nodes), finite and non-decreasing;
+        thrustLimit / rho: scalars or (n_traj,); params.controller must be LTO_CTRL_RMS.  defect: also return the defects (bitwise those of
+        indirect_traj(jac=False)).  Returns dict(dv (m/s), energy (N^2 TU), status (worst segment status)[, defect (n_traj, n_nodes-1, 12)])."""
+        p = params or indirect_params()
+        XC = _f64(XC_all)
+        if XC.ndim != 3 or XC.shape[2] != 12:
+            raise ValueError("XC_all must be (n_traj, n_nodes, 12): the cost quadrature is in the 12-dim kernel (got %s)" % (XC.shape,))
+        n_traj, n_nodes, _ = XC.shape
+        if n_nodes < 2:
+            raise ValueError("n_nodes must be >= 2 (got %d)" % n_nodes)
+        if p.controller != LTO_CTRL_RMS:
+            raise ValueError("the cost quadrature needs controller = LTO_CTRL_RMS (got %d)" % p.controller)
+        t_TU = _shaped("t_TU", t_TU, (n_traj, n_nodes))
+        bad = ~np.isfinite(t_TU).all(axis=1) | (np.diff(t_TU, axis=1) < 0).any(axis=1)
+        if bad.any():
+            raise ValueError("trajectory %d: t_TU must be finite and non-decreasing (reversed spans are not supported)" % int(np.argmax(bad)))
+        tl = _per_unit("thrustLimit", thrustLimit, n_traj)
+        rh = _per_unit("rho", rho, n_traj)
+        dv = np.empty(n_traj); energy = np.empty(n_traj); status = np.empty(n_traj, dtype=np.int32)
+        d = np.empty((n_traj, n_nodes - 1, 12)) if defect else None
+        self._ck(lib().lto_indirect_cost_batch(self._h, C.addressof(p), n_traj, n_nodes, _ptr(XC), _ptr(t_TU), _ptr(tl), _ptr(rh), _ptr(dv),
+                                               _ptr(energy), _ptr(d), _ptr(status)))
+        out = dict(dv=dv, energy=energy, status=status)
+        if defect:
+            out["defect"] = d
+        return out
 
     # ---- device-resident (raw device addresses, e.g. torch .data_ptr()) --
     def direct_dev(self, params, n_seg, n_nodes, nstate, nsteps, Xa, Xb, ua, ub, ta, tb, defect, errors, status, jac):

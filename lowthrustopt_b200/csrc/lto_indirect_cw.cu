@@ -358,7 +358,7 @@ struct LawConst { double aL, rho_inv, rho_inv_quarter_aL; };   // per slot: aL =
 template <bool LIN>
 __device__ __forceinline__ void sc_eval(const double (&R)[3], const double (&V)[3], const double (&L)[3], const double (&M)[3],
                                         const SCConst& c, const LawConst& lw, double (&kv)[3], double (&kl)[3], double (&km)[3],
-                                        double2* __restrict__ w) {
+                                        double2* __restrict__ w, double* umag_out = nullptr) {
     const double w2 = 2.0 * c.omega;
     // ---- gravity (:69-70, :78-81) and its gradient
     const double dx1 = R[0] + c.mu, dx2 = dx1 - 1.0;
@@ -396,6 +396,7 @@ __device__ __forceinline__ void sc_eval(const double (&R)[3], const double (&V)[
     }
     if (dead) { umag = 0.0; dn = 0.0; }
     if (!(n2 == n2)) umag = n2;                                        // a NaN costate stays NaN (reported through status[])
+    if (umag_out) *umag_out = umag;
     const double uon = umag * in;
     // ---- derivatives (:78-88)
     kv[0] = fma(-uon, M[0], fma(-a31, dx1, fma(-a32, dx2, fma(w2, V[1], R[0]))));
@@ -749,9 +750,52 @@ __device__ __forceinline__ void state_only_stage(KStore& K, const double (&x)[ND
 #endif
 }
 
+// The cost pass's stage: sc_eval_state_call's derivatives plus the stage's thrust-acceleration magnitude |a_u| = umag of the control
+// law (CRTBP_stateCostate_deriv.jl:36-53: zero when |lv| = 0, the clamped branch for p > 1) in v[9].
+struct Out10 { double v[10]; };
+__device__ __noinline__ Out10 sc_eval_quad_call(double r0, double r1, double r2, double v0, double v1, double v2, double l0, double l1, double l2,
+                                                double m0, double m1, double m2, double mu, double mu1, double omega, double pexp, double aL,
+                                                double rho_inv, double rq) {
+    const double R[3] = {r0, r1, r2}, V[3] = {v0, v1, v2}, L[3] = {l0, l1, l2}, M[3] = {m0, m1, m2};
+    SCConst c; c.mu = mu; c.m1 = mu1; c.omega = omega; c.p = pexp;
+    LawConst lw; lw.aL = aL; lw.rho_inv = rho_inv; lw.rho_inv_quarter_aL = rq;
+    double kv[3], kl[3], km[3];
+    Out10 o;
+    sc_eval<false>(R, V, L, M, c, lw, kv, kl, km, nullptr, &o.v[9]);
+#pragma unroll
+    for (int q = 0; q < 3; ++q) { o.v[q] = kv[q]; o.v[3 + q] = kl[q]; o.v[6 + q] = km[q]; }
+    return o;
+}
+
+// Stage J of K4.  QUAD: also s_dv += b_J umag_J and s_e += b_J umag_J^2 with the weights b of the 8th-order update (step_finish), so
+// that h s_dv and h s_e are the update's quadratures of |a_u| and |a_u|^2 over the step.
+template <int J, bool QUAD>
+__device__ __forceinline__ void k4_stage(KStore& K, const double (&x)[ND], double h, double h2, const SCConst& c, const LawConst& lw,
+                                         double& s_dv, double& s_e) {
+    if (!QUAD) { state_only_stage<J>(K, x, h, h2, c, lw); return; }
+    double R[3], V[3], L[3], M[3];
+    stage_input<J>(K, x, h, h2, R, V, L, M);
+    const Out10 o = sc_eval_quad_call(R[0], R[1], R[2], V[0], V[1], V[2], L[0], L[1], L[2], M[0], M[1], M[2], c.mu, c.m1, c.omega, c.p, lw.aL,
+                                      lw.rho_inv, lw.rho_inv_quarter_aL);
+#pragma unroll
+    for (int q = 0; q < 3; ++q) { K.kv[J][q] = o.v[q]; K.kl[J][q] = o.v[3 + q]; K.km[J][q] = o.v[6 + q]; }
+    if (J == 0) { s_dv = 0.0; s_e = 0.0; }
+    if (lto_tab::CHIf(J) != 0.0) {
+        const double u = o.v[9];
+        s_dv = fma(lto_tab::CHIf(J), u, s_dv);
+        s_e = fma(lto_tab::CHIf(J), u * u, s_e);
+    }
+}
+
 constexpr int K4I_THREADS = 128;
 
-__global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state(IndirectArgs a) {
+// QUAD = false: the defect-only kernel k_indirect_state.  QUAD = true (k_indirect_state_cost): the same steps (the quadratures are not in
+// the error norm, so the step sequence and every state are bitwise those of QUAD = false) and, per segment, a.quad[2 seg] =
+// int |a_u| dt and a.quad[2 seg + 1] = int |a_u|^2 dt, accumulated over the accepted steps only (NaN for a segment whose status is not
+// LTO_ST_OK: it never reached t1).  `a` is taken by value: so
+// k_indirect_state compiles to the same SASS as when this body was its own (through a reference, the register allocation changed).
+template <bool QUAD>
+__device__ __forceinline__ void k4_body(IndirectArgs a) {
     const unsigned fullmask = 0xffffffffu;
     double atol = a.cfg.atol, rtol = a.cfg.rtol;                          // per slot: state_tol_scale(p, rho) of the slot's segment
     double x[ND], xn[ND];
@@ -762,6 +806,7 @@ __global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state(IndirectArgs 
     long long seg = -1, ia = 0;
     int na = 0, nt = 0, status = 0;
     bool active = false, lastrej = false, last = false, have = false, exhausted = false;
+    double q_dv = 0.0, q_e = 0.0, s_dv = 0.0, s_e = 0.0;                  // QUAD: the segment's quadratures and the attempted step's sums
     while (true) {
         bool finished = false;
         if (have && active) {
@@ -774,6 +819,7 @@ __global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state(IndirectArgs 
                     ++na;
 #pragma unroll
                     for (int i = 0; i < ND; ++i) x[i] = xn[i];
+                    if (QUAD) { q_dv = fma(h, s_dv, q_dv); q_e = fma(h, s_e, q_e); }
                     if (last) { tcur = tf; finished = true; }
                     else { tcur += h; if (lastrej) q = fmin(q, 1.0); lastrej = false; }
                 } else {
@@ -795,6 +841,10 @@ __global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state(IndirectArgs 
             for (int i = 0; i < ND; ++i) a.defect[seg * ND + i] = a.x_target ? x[i] - a.x_target[ia * ND + i] : x[i];   // :82
             if (a.status) a.status[seg] = status;
             if (a.nsteps_out) { a.nsteps_out[2 * seg] = na; a.nsteps_out[2 * seg + 1] = nt; }
+            if (QUAD) {                                                   // a segment that did not reach t1 has no cost: NaN
+                const double nanv = __longlong_as_double(0x7ff8000000000000ll);
+                a.quad[2 * seg] = status ? nanv : q_dv; a.quad[2 * seg + 1] = status ? nanv : q_e;
+            }
             active = false;
         }
         bool fresh = false;
@@ -815,6 +865,7 @@ __global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state(IndirectArgs 
                 lw.rho_inv_quarter_aL = lw.aL / (4.0 * rho);
                 { const double ts = state_tol_scale(a.c.p, rho); atol = a.cfg.atol * ts; rtol = a.cfg.rtol * ts; }
                 na = 0; nt = 0; status = 0; lastrej = false;
+                if (QUAD) { q_dv = 0.0; q_e = 0.0; }
                 active = true; fresh = true;
             } else {
                 exhausted = true;
@@ -822,7 +873,7 @@ __global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state(IndirectArgs 
         }
         if (!__any_sync(fullmask, active)) break;
         KStore K;
-        state_only_stage<0>(K, x, 0.0, 0.0, a.c, lw);
+        k4_stage<0, QUAD>(K, x, 0.0, 0.0, a.c, lw, s_dv, s_e);
         if (__any_sync(fullmask, fresh)) {
             // Hairer-Norsett-Wanner initial step (drive_rk8 in lto_prop_generic.cuh)
             double f0[ND], y1[ND];
@@ -849,14 +900,17 @@ __global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state(IndirectArgs 
         if (tcur + h >= tf) { h = tf - tcur; last = true; }
         if (active) ++nt;
         const double h2 = h * h;
-        state_only_stage<1>(K, x, h, h2, a.c, lw);  state_only_stage<2>(K, x, h, h2, a.c, lw);  state_only_stage<3>(K, x, h, h2, a.c, lw);
-        state_only_stage<4>(K, x, h, h2, a.c, lw);  state_only_stage<5>(K, x, h, h2, a.c, lw);  state_only_stage<6>(K, x, h, h2, a.c, lw);
-        state_only_stage<7>(K, x, h, h2, a.c, lw);  state_only_stage<8>(K, x, h, h2, a.c, lw);  state_only_stage<9>(K, x, h, h2, a.c, lw);
-        state_only_stage<10>(K, x, h, h2, a.c, lw); state_only_stage<11>(K, x, h, h2, a.c, lw); state_only_stage<12>(K, x, h, h2, a.c, lw);
+        k4_stage<1, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e);  k4_stage<2, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e);  k4_stage<3, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e);
+        k4_stage<4, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e);  k4_stage<5, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e);  k4_stage<6, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e);
+        k4_stage<7, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e);  k4_stage<8, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e);  k4_stage<9, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e);
+        k4_stage<10, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e); k4_stage<11, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e); k4_stage<12, QUAD>(K, x, h, h2, a.c, lw, s_dv, s_e);
         esum = step_finish<true, true>(K, x, h, h2, atol, rtol, xn);
         have = true;
     }
 }
+
+__global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state(IndirectArgs a) { k4_body<false>(a); }
+__global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state_cost(IndirectArgs a) { k4_body<true>(a); }
 
 }  // namespace icw
 
@@ -896,6 +950,46 @@ static cudaError_t launch_k4i(const IndirectArgs& a, cudaStream_t st) {
     const int grid = (int)std::min<long long>(blocks, (long long)n_sm * 2);
     icw::k_indirect_state<<<grid, icw::K4I_THREADS, 0, st>>>(a);
     return cudaGetLastError();
+}
+
+namespace icw {
+// Per trajectory, its segments' quadratures summed in segment order (no atomics: the sum does not depend on the batch around it).
+__global__ void k_cost_sum(const double* __restrict__ quad, const int32_t* __restrict__ seg_status, long long n_traj, int seg_per_traj,
+                           double dv_scale, double e_scale, double* __restrict__ dv, double* __restrict__ energy, int32_t* __restrict__ status) {
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n_traj) return;
+    double sd = 0.0, se = 0.0;
+    int w = 0;
+    for (int i = 0; i < seg_per_traj; ++i) {
+        const long long s = j * seg_per_traj + i;
+        sd += quad[2 * s]; se += quad[2 * s + 1];
+        w = max(w, (int)seg_status[s]);
+    }
+    dv[j] = sd * dv_scale; energy[j] = se * e_scale;
+    if (status) status[j] = w;
+}
+}  // namespace icw
+
+cudaError_t launch_indirect_cost(const IndirectArgs& a, long long n_traj, double dv_scale, double e_scale, double* dv, double* energy,
+                                 int32_t* status_traj, cudaStream_t st, int* n_launch) {
+    *n_launch = 0;
+    if (a.phi != nullptr || a.counter == nullptr || a.quad == nullptr || a.status == nullptr || a.cfg.controller != 0 || a.npt < 2 ||
+        a.n_seg <= 0 || a.n_seg > 0x7fffffffll || a.n_seg != n_traj * (a.npt - 1))
+        return cudaErrorNotSupported;
+    int dev = 0, n_sm = 0;
+    cudaError_t e = cudaGetDevice(&dev); if (e != cudaSuccess) return e;
+    e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev); if (e != cudaSuccess) return e;
+    e = cudaMemsetAsync(a.counter, 0, sizeof(unsigned long long), st); if (e != cudaSuccess) return e;
+    const long long blocks = (a.n_seg + icw::K4I_THREADS - 1) / icw::K4I_THREADS;
+    const int grid = (int)std::min<long long>(blocks, (long long)n_sm * 2);
+    icw::k_indirect_state_cost<<<grid, icw::K4I_THREADS, 0, st>>>(a);
+    e = cudaGetLastError(); if (e != cudaSuccess) return e;
+    *n_launch = 1;
+    icw::k_cost_sum<<<(unsigned)((n_traj + 127) / 128), 128, 0, st>>>(a.quad, a.status, n_traj, a.npt - 1, dv_scale, e_scale, dv, energy,
+                                                                      status_traj);
+    e = cudaGetLastError(); if (e != cudaSuccess) return e;
+    *n_launch = 2;
+    return cudaSuccess;
 }
 
 cudaError_t launch_indirect_cw(const IndirectArgs& a, int ndim, cudaStream_t st, int* n_launch) {

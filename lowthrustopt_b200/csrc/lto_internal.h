@@ -32,6 +32,7 @@ struct IndirectArgs {
     int npt;
     IndirectCfg cfg;
     SCConst c;
+    double* quad;                              // K4 cost pass only (launch_indirect_cost): per segment (int |a_u| dt, int |a_u|^2 dt)
 };
 
 __host__ __device__ inline long long lto_node_a(long long s, int npt) { return npt > 0 ? s + s / (npt - 1) : s; }
@@ -44,6 +45,10 @@ cudaError_t launch_indirect_generic(const IndirectArgs& a, int ndim, cudaStream_
 cudaError_t launch_direct_fast(const DirectArgs& a, int nstate, cudaStream_t st, int* n_launch);
 cudaError_t launch_indirect_fast(const IndirectArgs& a, int ndim, cudaStream_t st, int* n_launch);
 size_t indirect_cw_scratch_bytes(int n_sm);
+// K4 with the control-cost quadrature (a.quad) and the per-trajectory sums of lto_indirect_cost_batch: dv[j] = dv_scale * sum of the
+// trajectory's int |a_u| dt, energy[j] = e_scale * sum of its int |a_u|^2 dt, status_traj[j] = the worst segment status (a.status)
+cudaError_t launch_indirect_cost(const IndirectArgs& a, long long n_traj, double dv_scale, double e_scale, double* dv, double* energy,
+                                 int32_t* status_traj, cudaStream_t st, int* n_launch);
 cudaError_t launch_sumsq_rows(const double* v, long long n_rows, long long len, double* out, cudaStream_t st);
 cudaError_t launch_fp64_probe(int iters, double* d_sink, int n_sm, cudaStream_t st, long long* n_threads, int* chains);
 

@@ -6,6 +6,8 @@
     reduceFuel_indirect          src/HelperFunctions.jl:105-193   (+ reduceFuel_indirect_batch: many trajectories, one device call per round)
     trajectory_stack_guess       CRTBP_Multishoot_direct_demo.jl:117-157   (+ trajectory_stack_guess_batch: many transfers in one device call,
                                                                         direct_transfer_sweep: those guesses solved by the batched direct solver)
+    indirect_transfer_sweep      CRTBP_Multishoot_indirect_demo.jl:166-281 over a direct_transfer_sweep, batched, with each result's
+                                 transfer_cost_indirect (delta-v and control energy; no reference counterpart)
     densify, jacobiConstant, interpInitialStates, find_tau   src/HelperFunctions.jl:10-101
 
 Same names, argument order and return values.  Arrays use the reference's shapes
@@ -101,6 +103,11 @@ class GpuBackend:
         """trajectory_stack_guess for many transfers in one device call (lto_stack_guess_batch); params = the reference's tuple."""
         self.calls += 1
         return self.h.stack_guess_batch(X0_states, Xf_states, tau1, t_TU, t_split, params=self._ip(params))
+
+    def indirect_cost(self, XC, t, params, thrustLimit=None, rho=None, defect=False):
+        """delta-v and control energy of 12-dim trajectories XC (B, N, 12) in one device call (lto_indirect_cost_batch)."""
+        self.calls += 1
+        return self.h.indirect_cost_batch(XC, t, params=self._ip(params), thrustLimit=thrustLimit, rho=rho, defect=defect)
 
     def direct_solve_batch(self, X, U, t, state_0, state_f, mass, nsteps, max_iter, Isp, MU, DU, TU):
         self.calls += 1
@@ -266,7 +273,7 @@ def direct_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, n_no
     (trajectory_stack_guess_batch), then multiShoot_CRTBP_direct on all of them at once on the device (lto_direct_solve_batch; the demo's
     setting: flagEnd = false, allowImpulsive = false, u_all = 0 to start, nstate 7 adds a mass row of `mass`).  Two library calls.
     Returns dict(X_all (T, nstate, N), u_all (T, 3, N), t_TU (T, N), tau2 (T,), iters (T,), er (T,), converged (T,) = er <= 1e-6,
-    cost (T,) = quadCost at the returned controls)."""
+    cost (T,) = quadCost at the returned controls, state_0 / state_f (T, 6): the end states the solutions are pinned to)."""
     be = backend or default_backend()
     MU, DU, TU = capi.MU, capi.DU, capi.TU
     if nstate not in (6, 7):
@@ -281,7 +288,122 @@ def direct_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, n_no
                               np.ascontiguousarray(sf[:, :6]), mass, nsteps, maxIter, Isp, MU, DU, TU)
     u_all = r["u_all"].transpose(0, 2, 1).copy()
     return dict(X_all=r["X_all"].transpose(0, 2, 1).copy(), u_all=u_all, t_TU=t_TU, tau2=tau2, iters=r["iters"], er=r["er"],
-                converged=r["er"] <= 1e-6, cost=_quad_cost(u_all, t_TU))
+                converged=r["er"] <= 1e-6, cost=_quad_cost(u_all, t_TU), state_0=s0[:, :6].copy(), state_f=sf[:, :6].copy())
+
+
+G0 = 9.81                                          # the mass flow's g0 (CRTBP_prop_EP_deriv.jl:41; lto_indirect_params.g0)
+
+
+def transfer_cost_indirect(XC_all, t_TU, MU, DU, TU, mass, thrustLimit, p, rho, Isp=2000.0, backend=None):
+    """The cost of indirect trajectories XC_all (T, 12 or 14, N) on the time grids t_TU (T, N); thrustLimit and rho: scalars or (T,).
+      12 rows (constant mass): ONE device call (lto_indirect_cost_batch) integrates every segment with the quadratures of |a_u| and
+          |a_u|^2 along its adaptive steps: dv = int |a_u| dt in m/s and energy = int (|a_u| mass)^2 dt in N^2 TU, the units of the direct
+          method's quadCost (direct_transfer_sweep's cost).  propellant: the rocket equation's mass for that dv at `Isp`.
+      14 rows: no device call.  The mass is a state, so propellant = m0 - m_f from the node values and dv = Isp g0 ln(m0 / m_f), which
+          is exact for the 14-dim dynamics (mdot = -|T| / (Isp g0), |a_u| = |T| / m); energy is not available (NaN).
+    Returns dict(dv (T,), energy (T,), propellant (T,), status (T,): the worst LTO_ST_* of a trajectory's segments (14 rows: LTO_ST_NAN
+    where a node mass is not finite))."""
+    XC = np.asarray(XC_all, dtype=np.float64)
+    if XC.ndim != 3 or XC.shape[1] not in (12, 14) or XC.shape[2] < 2:
+        raise ValueError("XC_all must be (T, 12 or 14, n_nodes >= 2) (got %s)" % (XC.shape,))
+    T, m, N = XC.shape
+    t_TU = np.asarray(t_TU, dtype=np.float64)
+    if t_TU.shape != (T, N):
+        raise ValueError("t_TU must be (T, n_nodes) = %s (got %s)" % ((T, N), t_TU.shape))
+    if m == 14:
+        m0, mf = XC[:, 6, 0], XC[:, 6, -1]
+        with np.errstate(divide="ignore", invalid="ignore"):
+            dv = Isp * G0 * np.log(m0 / mf)
+        ok = np.isfinite(m0) & np.isfinite(mf)
+        return dict(dv=dv, energy=np.full(T, np.nan), propellant=m0 - mf, status=np.where(ok, 0, 1).astype(np.int32))   # LTO_ST_NAN
+    be = backend or default_backend()
+    tl = np.broadcast_to(np.asarray(thrustLimit, dtype=np.float64), (T,)).copy()
+    rh = np.broadcast_to(np.asarray(rho, dtype=np.float64), (T,)).copy()
+    params = (MU, DU, TU, float(tl[0]) if T else 0.0, mass, 1.0, p, float(rh[0]) if T else 1.0)
+    r = be.indirect_cost(np.ascontiguousarray(XC.transpose(0, 2, 1)), t_TU, params, thrustLimit=tl, rho=rh)
+    return dict(dv=r["dv"], energy=r["energy"], propellant=mass * -np.expm1(-r["dv"] / (Isp * G0)), status=r["status"])
+
+
+def indirect_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, thrustLimit=0.05, rho_target=1e-4, seeds=None, n_nodes=30,
+                            nsteps=10, mass=1e3, Isp=2000.0, maxIter_direct=100, backend=None):
+    """Fuel-optimal transfers for a grid of departure phases and flight times: the indirect demo's chain
+    (CRTBP_Multishoot_indirect_demo.jl:166-281) run on every row of direct_transfer_sweep (nstate 6), each stage as one batched device call:
+      start   per row j, as the demo: costates 0.1 * N(0, 1) from np.random.default_rng(seeds[j]), end states pinned to state_0 / state_f,
+              1e-10 jitter on the interior nodes (seeds default to 0 .. T-1);
+      stage 1 adjoints-only solve, p = 2, 10 N, maxIter 10 (status 1 is expected there; only NaN fails the stage);
+      stage 2 full solve, p = 2, 10 N, maxIter 50;
+      stage 3 p = 1 at thrustLimit, rho = 1, maxIter 30;
+      stage 4 reduceFuel_indirect_batch(device_ladder=True) to rho_target, back-off draws from a fresh np.random.default_rng(seeds[j]);
+      then transfer_cost_indirect of every surviving row (p = 1, its last rho).
+    A row that fails a stage (status != 0) enters no later stage: stage_failed (T,) is that stage (1-4), 0 for a row that came through; its
+    dv and energy are NaN.  Each row's result does not depend on the other rows.
+    Returns dict(XC_all (T, 12, N): each row's last solution, t_TU, tau2, state_0, state_f, stage_failed, status and rho_last of the ladder
+    (-1 / NaN for rows that did not reach it), dv (m/s), energy (N^2 TU), energy_p2: the stage-2 solution's energy at 10 N (NaN if it
+    failed), and the direct sweep's cost / converged / iters alongside)."""
+    MU, DU, TU = capi.MU, capi.DU, capi.TU
+    shape = np.broadcast(*[np.atleast_1d(np.asarray(a, dtype=np.float64)) for a in (tau1, tof1_days, tof2_days)]).shape
+    if len(shape) != 1:
+        raise ValueError("tau1, tof1_days and tof2_days must be scalars or (T,) arrays")
+    T = shape[0]
+    seeds = list(range(T)) if seeds is None else [int(s) for s in np.atleast_1d(seeds)]
+    if len(seeds) != T:
+        raise ValueError("seeds must have one entry per row (%d, got %d)" % (T, len(seeds)))
+    if not (np.isfinite(thrustLimit) and thrustLimit > 0):
+        raise ValueError("thrustLimit must be a positive number of newtons (got %r)" % (thrustLimit,))
+    if not (np.isfinite(rho_target) and 0 < rho_target <= 1):
+        raise ValueError("rho_target must be in (0, 1] (got %r)" % (rho_target,))
+    if n_nodes < 3:
+        raise ValueError("n_nodes must be >= 3 (got %r)" % (n_nodes,))
+    be = backend or default_backend()
+    d = direct_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, n_nodes=n_nodes, nsteps=nsteps, nstate=6, mass=mass, Isp=Isp,
+                              maxIter=maxIter_direct, backend=be)
+    t_TU = d["t_TU"]
+    N = t_TU.shape[1]
+    XC = np.empty((T, 12, N))
+    for j in range(T):
+        rng = np.random.default_rng(seeds[j])
+        XC[j] = np.vstack([d["X_all"][j], 0.1 * rng.standard_normal((6, N))])
+        XC[j, :6, 0] = d["state_0"][j]; XC[j, :6, -1] = d["state_f"][j]
+        XC[j, :, 1:-1] += 1e-10 * rng.standard_normal((12, N - 2))
+    stage_failed = np.zeros(T, dtype=np.int32)
+
+    def solve(stage, thrust, p, rho, max_iter, adjoints_only, fail_on):
+        idx = np.flatnonzero(stage_failed == 0)
+        if idx.size == 0:
+            return
+        Xn, _, st, _ = multiShoot_CRTBP_indirect_batch(XC[idx], t_TU[idx], MU, DU, TU, N, mass, thrust, adjoints_only, max_iter, p, rho,
+                                                       backend=be)
+        XC[idx] = Xn
+        stage_failed[idx[np.isin(st, fail_on)]] = stage
+
+    solve(1, 10.0, 2.0, 1.0, 10, True, (2,))
+    solve(2, 10.0, 2.0, 1.0, 50, False, (1, 2))
+    alive = np.flatnonzero(stage_failed == 0)
+    energy_p2 = np.full(T, np.nan)
+    if alive.size:
+        energy_p2[alive] = transfer_cost_indirect(XC[alive], t_TU[alive], MU, DU, TU, mass, 10.0, 2.0, 1.0, Isp, backend=be)["energy"]
+    solve(3, thrustLimit, 1.0, 1.0, 30, False, (1, 2))
+    status = np.full(T, -1, dtype=np.int32); rho_last = np.full(T, np.nan)
+    dv = np.full(T, np.nan); energy = np.full(T, np.nan)
+    idx = np.flatnonzero(stage_failed == 0)
+    if idx.size:
+        # reduceFuel_indirect_batch(device_ladder=True) with its back-off draws taken the same way; called directly for rho_last
+        draws = np.array([np.random.default_rng(seeds[j]).random(100) for j in idx], dtype=np.float64).reshape(idx.size, 100)
+        r = be.indirect_reduce_fuel_batch(np.ascontiguousarray(XC[idx].transpose(0, 2, 1)), t_TU[idx], (MU, DU, TU, float(thrustLimit), mass,
+                                          1.0, 1.0, 1.0), np.ones(idx.size), np.full(idx.size, float(rho_target)), draws,
+                                          thrustLimit=np.full(idx.size, float(thrustLimit)), max_iter=10)
+        st = r["status"]
+        XC[idx] = r["XC_all"].transpose(0, 2, 1)
+        status[idx] = st
+        rho_last[idx] = r["rho_last"]
+        stage_failed[idx[st != 0]] = 4
+        ok = idx[st == 0]
+        if ok.size:
+            c = transfer_cost_indirect(XC[ok], t_TU[ok], MU, DU, TU, mass, thrustLimit, 1.0, rho_last[ok], Isp, backend=be)
+            dv[ok] = c["dv"]; energy[ok] = c["energy"]
+    return dict(XC_all=XC, t_TU=t_TU, tau2=d["tau2"], state_0=d["state_0"], state_f=d["state_f"], stage_failed=stage_failed, status=status,
+                rho_last=rho_last, dv=dv, energy=energy, energy_p2=energy_p2, cost=d["cost"], direct_converged=d["converged"],
+                direct_iters=d["iters"])
 
 
 # --------------------------------------------------------------------------- direct method
