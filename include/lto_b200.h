@@ -303,6 +303,29 @@ int lto_direct_solve_batch(lto_handle* h, const lto_direct_params* p, int64_t n_
                            double* X_all, double* u_all, const double* t_TU, const double* state_0, const double* state_f, double mass,
                            double* defect, int32_t* iters, double* er_out);
 
+/* lto_direct_costates_batch: the costates of n_traj nstate-6 direct solutions (the layout of lto_direct_solve_batch), from the dual
+ * solution of optimizeTraj's QP at the given point.  One K1 launch for the Jacobian blocks at (X_all, u_all), one launch of K7's dual
+ * instantiation: the multipliers lambda_i of segment i's defect rows, mapped to node costates with Jx(i, k) = the 6 x 6 block of segment i's
+ * Jacobian in node k's columns,
+ *     p_i = Jx(i, i)^T lambda_i (i < n_nodes-1),  p_{n_nodes-1} = -Jx(n_nodes-2, n_nodes-1)^T lambda_{n_nodes-2},
+ *     [lr; lv](t_i) = -p_i / kappa^2,  kappa = default_mass / kthr = default_mass DU 1e3 / TU^2 (u in N = kappa x nondimensional acceleration).
+ * At a KKT point of the energy-optimal direct problem these are the discrete costates of the 12-dim p = 2 system (whose law a = -lv / 2
+ * then gives lv(t_i) ~ -2 u_i / kappa), a start for lto_indirect_solve_batch at a thrust limit that does not bind.  The X_i rows of the KKT
+ * system carry no objective term, so both one-sided values of an interior node agree up to the band solve's rounding.  nstate 7 is not
+ * accepted (the X layout is 6 x n_nodes): the direct nstate-7 objective is not the 14-dim law's cost, so lm has no such map.
+ *   X_all 6 x n_nodes, u_all 3 x n_nodes, t_TU n_nodes (finite, strictly increasing), state_0 / state_f 6: per trajectory
+ *   XC_all       out, 12 x n_nodes per trajectory: rows 0-5 X_all bitwise, rows 6-11 the costates (NaN where status != LTO_ST_OK)
+ *   multipliers  out, 6 x (n_nodes-1) per trajectory, lambda_i as solved; may be NULL
+ *   du_max       out, n_traj: max |du| in N of the QP's control step at the given point (0 at an exact KKT point); may be NULL
+ *   status       out, n_traj: the worst of the K1 segment statuses and K7's singular flag (LTO_ST_*); may be NULL
+ * p->mode must be LTO_FIXED.  Null arrays, n_nodes < 2, non-finite t_TU / state_0 / state_f and a t_TU that is not strictly increasing are
+ * LTO_ERR_ARG, naming the first offending trajectory; non-finite X_all / u_all show up in that trajectory's status.  n_traj = 0 does
+ * nothing.  Inputs go up in one copy and the call synchronises once.  Multi-device handles split whole trajectories. */
+int lto_direct_costates_batch(lto_handle* h, const lto_direct_params* p, int64_t n_traj, int n_nodes, int nsteps,
+                              const double* X_all, const double* u_all, const double* t_TU,
+                              const double* state_0, const double* state_f,
+                              double* XC_all, double* multipliers, double* du_max, int32_t* status);
+
 /* lto_stack_guess_batch: the demos' trajectory-stacking initial guess (CRTBP_Multishoot_direct_demo.jl:117-157, with interpInitialStates /
  * find_τ of src/HelperFunctions.jl:18-48) for n_traj transfers in one call, every stage on the device.  Per trajectory j:
  *   state_0 = spline(X0)(tau1[j]);  arc 1 = [state_0; 0] propagated from t_TU[0] to every node with t_TU < t_split (strict) and to t_split;

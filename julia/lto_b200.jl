@@ -217,4 +217,21 @@ function indirect_cost_batch(XC_batch::Array{Float64,3}, t_batch::Matrix{Float64
         handle[], prm, n_traj, n_nodes, XC_batch, t_batch, thrustLimit, rho, dv, energy, C_NULL, status))
     (dv, energy, status)
 end
+# ---- costates of nstate-6 direct solutions in ONE call (lto_direct_costates_batch): the direct QP's multipliers at (X, u), mapped to the
+# node costates of the 12-dim p = 2 system.  X_batch 6 x n_nodes x n_traj, u_batch 3 x n_nodes x n_traj, t_batch n_nodes x n_traj,
+# state_0 / state_f 6 x n_traj.  Returns (XC 12 x n_nodes x n_traj: X bitwise and the costates, multipliers 6 x (n_nodes-1) x n_traj,
+# du_max in N, status); XC with the end states pinned is a start for multiShoot_CRTBP_indirect at p = 2.  Like the rest of this shim, not run
+# under Julia here (the same ABI is exercised from Python).
+function direct_costates_batch(X_batch::Array{Float64,3}, u_batch::Array{Float64,3}, t_batch::Matrix{Float64}, state_0::Matrix{Float64},
+                               state_f::Matrix{Float64}, MU, DU, TU; nsteps=10)
+    size(X_batch, 1) == 6 || error("direct_costates_batch: X_batch must have 6 rows (nstate 7 has no costate map)")
+    n_nodes = size(X_batch, 2); n_traj = size(X_batch, 3)
+    p = DirectParams(); p.MU, p.DU, p.TU = MU, DU, TU
+    XC = zeros(12, n_nodes, n_traj); mult = zeros(6, n_nodes - 1, n_traj); du = zeros(n_traj); status = zeros(Int32, n_traj)
+    GC.@preserve X_batch u_batch t_batch state_0 state_f XC mult du status check(ccall((:lto_direct_costates_batch, lib), Cint,
+        (Ptr{Cvoid}, Ref{DirectParams}, Int64, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+        handle[], p, n_traj, n_nodes, nsteps, X_batch, u_batch, t_batch, state_0, state_f, XC, mult, du, status))
+    (XC, mult, du, status)
+end
 end # module

@@ -32,7 +32,7 @@ EXPORTS = [
     "lto_push_async", "lto_sync_copies", "lto_signal_dev", "lto_wait_dev", "lto_fp64_peak_probe", "lto_debug_profile",
     "lto_indirect_newton", "lto_indirect_newton_dev", "lto_indirect_newton_resolve_dev", "lto_indirect_solve_batch", "lto_direct_qp", "lto_direct_qp_dev", "lto_direct_solve_batch",
     "lto_indirect_newton_nd", "lto_indirect_newton_nd_dev", "lto_indirect_newton_resolve_nd_dev", "lto_indirect_solve_batch_nd",
-    "lto_indirect_reduce_fuel_batch", "lto_stack_guess_batch", "lto_indirect_cost_batch",
+    "lto_indirect_reduce_fuel_batch", "lto_stack_guess_batch", "lto_indirect_cost_batch", "lto_direct_costates_batch",
 ]
 
 
@@ -119,6 +119,7 @@ def lib():
         L.lto_direct_solve_batch.argtypes = [vp, vp, i64, ci, ci, ci, ci] + [vp] * 5 + [C.c_double] + [vp] * 3
         L.lto_stack_guess_batch.argtypes = [vp, vp, i64, ci, vp, ci, vp, ci] + [vp] * 3 + [vp] * 5
         L.lto_indirect_cost_batch.argtypes = [vp, vp, i64, ci] + [vp] * 4 + [vp] * 4
+        L.lto_direct_costates_batch.argtypes = [vp, vp, i64, ci, ci] + [vp] * 5 + [vp] * 4
         _lib = L
     return _lib
 
@@ -637,6 +638,32 @@ class Handle:
         self._ck(lib().lto_direct_solve_batch(self._h, C.addressof(p), n_traj, n_nodes, ns, int(nsteps), int(max_iter), _ptr(X), _ptr(U), _ptr(t_TU),
                                               _ptr(state_0), _ptr(state_f), float(mass), _ptr(defect), _ptr(iters), _ptr(er)))
         return dict(X_all=X, u_all=U, defect=defect, iters=iters, er=er)
+
+    def direct_costates_batch(self, X, U, t, state_0, state_f, nsteps=10, params=None):
+        """Costates of nstate-6 direct solutions from the dual solution of optimizeTraj's QP (lto_direct_costates_batch): K1's Jacobian
+        blocks at (X, U), then K7's multipliers of the defect rows mapped to the node costates of the 12-dim p = 2 system.
+        X: (n_traj, n_nodes, 6); U: (n_traj, n_nodes, 3); t: (n_traj, n_nodes), finite and strictly increasing; state_0, state_f: (n_traj, 6);
+        params.mode must be LTO_FIXED.  Returns dict(XC_all (n_traj, n_nodes, 12): X bitwise and the costates (NaN where status != 0),
+        multipliers (n_traj, n_nodes-1, 6), du_max (n_traj,): max |du| in N of the QP step at (X, U), status (n_traj,))."""
+        p = params or direct_params()
+        X = _f64(X)
+        if X.ndim != 3 or X.shape[2] != 6:
+            raise ValueError("X must be (n_traj, n_nodes, 6): the costate map is for nstate 6 (got %s)" % (X.shape,))
+        n_traj, n_nodes, _ = X.shape
+        if n_nodes < 2:
+            raise ValueError("n_nodes must be >= 2 (got %d)" % n_nodes)
+        if p.mode != LTO_FIXED:
+            raise ValueError("the direct costates run the fixed-grid path: params.mode must be LTO_FIXED (got %d)" % p.mode)
+        U = _shaped("U", U, (n_traj, n_nodes, 3)); t = _shaped("t", t, (n_traj, n_nodes))
+        state_0 = _shaped("state_0", state_0, (n_traj, 6)); state_f = _shaped("state_f", state_f, (n_traj, 6))
+        bad = ~np.isfinite(t).all(axis=1) | ~(np.diff(t, axis=1) > 0).all(axis=1)
+        if bad.any():
+            raise ValueError("trajectory %d: t must be finite and strictly increasing" % int(np.argmax(bad)))
+        XC = np.empty((n_traj, n_nodes, 12)); mult = np.empty((n_traj, n_nodes - 1, 6)); du = np.empty(n_traj)
+        status = np.empty(n_traj, dtype=np.int32)
+        self._ck(lib().lto_direct_costates_batch(self._h, C.addressof(p), n_traj, n_nodes, int(nsteps), _ptr(X), _ptr(U), _ptr(t), _ptr(state_0),
+                                                 _ptr(state_f), _ptr(XC), _ptr(mult), _ptr(du), _ptr(status)))
+        return dict(XC_all=XC, multipliers=mult, du_max=du, status=status)
 
     # ---- the trajectory-stacking initial guess on the device ----
     def stack_guess_batch(self, X0_states, Xf_states, tau1, t_TU, t_split, params=None):

@@ -100,13 +100,24 @@ __device__ __forceinline__ double kkt_rhs(int a, int N, const QpArgs& A, long lo
     return 0.0;
 }
 
-template <int NS>
-__global__ void __launch_bounds__(32 * WARPS) k_direct_qp(QpArgs A) {
+// Outputs of the dual instantiation (nstate 6): the multipliers of the defect rows and the node costates they map to.
+struct DualArgs {
+    const int32_t* seg_status;                // K1's status per segment, n_traj x (n_nodes-1)
+    double *mult, *XC, *du_max;               // 6 x (n_nodes-1), 12 x n_nodes, 1 per trajectory
+    double kappa;                             // default_mass / kthr: u in N = kappa x the nondimensional acceleration
+};
+
+// K7's body.  DUAL = false: the primal step (x_update, u_update) of lto_direct_qp.  DUAL = true (NS = 6): the back substitution keeps
+// the K_L unknowns -- the multipliers lambda_i of segment i's defect -- instead, and an epilogue maps them to node costates.
+template <int NS, bool DUAL>
+__device__ __forceinline__ void qp_body(QpArgs A, DualArgs D) {
     typedef Geo<NS> G;
     constexpr int BW = G::BW;
     extern __shared__ __align__(16) double smem_d[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const long long traj = (long long)blockIdx.x * WARPS + wid;
+    // wid < WARPS, so | is +.  Written as | because that is what the compiler made of + when this was the kernel's own body (it knew
+    // the launch bound there): k_direct_qp<NS> keeps the instructions it had.
+    const long long traj = ((long long)blockIdx.x * WARPS) | wid;
     if (traj >= A.n_traj) return;
     const int N = A.n_nodes, TOT = G::total(N);
     double* W = smem_d + (size_t)wid * SM_PER_WARP;          // W[(row & 31) * 64 + (col & 63)]
@@ -185,6 +196,7 @@ __global__ void __launch_bounds__(32 * WARPS) k_direct_qp(QpArgs A) {
     __syncwarp();
     double un = U[(long long)(TOT - 1) * UROW + 1 + lane], pn = U[(long long)(TOT - 1) * UROW], rn = U[(long long)(TOT - 1) * UROW + 33];
     bool bad = singular;
+    double du = 0.0;                                         // DUAL: max |du| (N)
 #pragma unroll 1
     for (int j = TOT - 1; j >= 0; --j) {
         const double u = un, piv = pn, rhs = rn;
@@ -198,12 +210,51 @@ __global__ void __launch_bounds__(32 * WARPS) k_direct_qp(QpArgs A) {
         if (lane == 0) {
             xs[j & (WC - 1)] = x;
             const Idx d = G::decode(j, N);
-            if (d.kind == K_X) A.x_update[(traj * N + d.node) * NS + d.comp] = x;              // X_jump (:391)
-            else if (d.kind == K_U) A.u_update[(traj * N + d.node) * 3 + d.comp] = x;          // u_jump (:392)
+            if (!DUAL) {
+                if (d.kind == K_X) A.x_update[(traj * N + d.node) * NS + d.comp] = x;          // X_jump (:391)
+                else if (d.kind == K_U) A.u_update[(traj * N + d.node) * 3 + d.comp] = x;      // u_jump (:392)
+            } else {
+                if (d.kind == K_L) D.mult[(traj * (N - 1) + d.node) * NS + d.comp] = x;
+                else if (d.kind == K_U) { const double a = fabs(x); if (!(a <= du)) du = a; }   // NaN sticks
+            }
         }
         __syncwarp();
     }
-    if (A.status && lane == 0) A.status[traj] = bad ? LTO_ST_NAN : 0;
+    if (!DUAL) {
+        if (A.status && lane == 0) A.status[traj] = bad ? LTO_ST_NAN : 0;
+        return;
+    }
+    // ---------------- dual epilogue: status, then the costates of every node from the multipliers lane 0 stored
+    int worst = bad ? LTO_ST_NAN : LTO_OK;
+    for (int k = lane; k < N - 1; k += 32) worst = max(worst, (int)D.seg_status[traj * (N - 1) + k]);
+    worst = __reduce_max_sync(full, worst);
+    if (lane == 0) { A.status[traj] = worst; D.du_max[traj] = du; }
+    __threadfence_block();
+    __syncwarp();
+    const double* lam = D.mult + traj * (long long)(N - 1) * NS;
+    for (int k = lane; k < N * NS; k += 32) {
+        const int i = k / NS, c = k - i * NS;
+        // p_i = Jx(i, i)^T lambda_i (forward leg); the last node: p = -Jx(N-2, N-1)^T lambda_{N-2} (backward leg)
+        const int seg = i < N - 1 ? i : N - 2, col = i < N - 1 ? c : NS + c;
+        const double* Jc = jac + ((long long)seg * (2 * (NS + 3)) + col) * NS;
+        const double* l = lam + (long long)seg * NS;
+        double p = 0.0;
+#pragma unroll
+        for (int r = 0; r < NS; ++r) p = fma(Jc[r], l[r], p);
+        if (i == N - 1) p = -p;
+        double* xc = D.XC + (traj * N + i) * 12;
+        xc[c] = A.X_all[(traj * N + i) * NS + c];
+        xc[NS + c] = worst == LTO_OK ? -p / (D.kappa * D.kappa) : nan("");              // [lr; lv] = -p / kappa^2
+    }
+}
+
+template <int NS>
+__global__ void __launch_bounds__(32 * WARPS) k_direct_qp(QpArgs A) {
+    qp_body<NS, false>(A, DualArgs());
+}
+
+__global__ void __launch_bounds__(32 * WARPS) k_direct_qp_dual(QpArgs A, DualArgs D) {
+    qp_body<6, true>(A, D);
 }
 
 }  // namespace dqp
@@ -231,6 +282,24 @@ cudaError_t launch_direct_qp(const double* jac, const double* defect, const doub
         e = cudaFuncSetAttribute(dqp::k_direct_qp<7>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); if (e != cudaSuccess) return e;
         dqp::k_direct_qp<7><<<(int)blocks, 32 * dqp::WARPS, smem, st>>>(A);
     }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_direct_qp_dual(const double* jac, const double* defect, const double* X_all, const double* u_all, const double* t,
+                                  const double* b0, const double* bf, const int32_t* seg_status, double kappa, double* work, double* mult,
+                                  double* XC, double* du_max, int32_t* status, long long n_traj, int n_nodes, cudaStream_t st) {
+    if (n_traj <= 0 || n_nodes < 2) return cudaErrorInvalidValue;
+    dqp::QpArgs A;
+    A.jac = jac; A.defect = defect; A.X_all = X_all; A.u_all = u_all; A.t = t; A.b0 = b0; A.bf = bf;
+    A.work = work; A.x_update = nullptr; A.u_update = nullptr; A.status = status; A.n_traj = n_traj; A.n_nodes = n_nodes;
+    dqp::DualArgs D;
+    D.seg_status = seg_status; D.mult = mult; D.XC = XC; D.du_max = du_max; D.kappa = kappa;
+    const long long blocks = (n_traj + dqp::WARPS - 1) / dqp::WARPS;
+    if (blocks > 0x7fffffffll) return cudaErrorInvalidValue;
+    const size_t smem = (size_t)dqp::WARPS * dqp::SM_PER_WARP * sizeof(double);
+    cudaError_t e = cudaFuncSetAttribute(dqp::k_direct_qp_dual, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    dqp::k_direct_qp_dual<<<(int)blocks, 32 * dqp::WARPS, smem, st>>>(A, D);
     return cudaGetLastError();
 }
 

@@ -32,6 +32,9 @@ size_t direct_qp_workspace_bytes(long long n_traj, int n_nodes, int nstate);
 cudaError_t launch_direct_qp(const double* jac, const double* defect, const double* X_all, const double* u_all, const double* t,
                              const double* b0, const double* bf, double* work, double* x_update, double* u_update, int32_t* status,
                              long long n_traj, int n_nodes, int nstate, cudaStream_t st);
+cudaError_t launch_direct_qp_dual(const double* jac, const double* defect, const double* X_all, const double* u_all, const double* t,
+                                  const double* b0, const double* bf, const int32_t* seg_status, double kappa, double* work, double* mult,
+                                  double* XC, double* du_max, int32_t* status, long long n_traj, int n_nodes, cudaStream_t st);
 
 namespace slv {
 
@@ -808,6 +811,91 @@ int lto_direct_solve_batch(lto_handle* h, const lto_direct_params* p, int64_t n_
     if (iters) CK(h, cudaMemcpyAsync(iters, dIters, T * 4, cudaMemcpyDeviceToHost, st));
     if (er_out) CK(h, cudaMemcpyAsync(er_out, dErOut, T * 8, cudaMemcpyDeviceToHost, st));
     CK(h, cudaStreamSynchronize(st));
+    float ms = 0.f; CK(h, cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1)); h->last_ms = ms;
+    return LTO_SUCCESS;
+}
+
+// The dual solution of optimizeTraj's QP at a given nstate-6 point, mapped to the costates of the 12-dim p = 2 system: one K1 launch for
+// the Jacobian blocks, one k_direct_qp_dual launch.
+int lto_direct_costates_batch(lto_handle* h, const lto_direct_params* p, int64_t n_traj, int n_nodes, int nsteps, const double* X_all,
+                              const double* u_all, const double* t_TU, const double* state_0, const double* state_f, double* XC_all,
+                              double* multipliers, double* du_max, int32_t* status) {
+    LTO_NVTX();
+    if (!h) return fail(nullptr, LTO_ERR_ARG, "null handle");
+    if (!p) return fail(h, LTO_ERR_ARG, "null params");
+    if (n_traj < 0) return fail(h, LTO_ERR_ARG, "negative trajectory count");
+    if (n_nodes < 2) return fail(h, LTO_ERR_ARG, "n_nodes must be >= 2 (got %d)", n_nodes);
+    if (p->mode != LTO_FIXED) return fail(h, LTO_ERR_ARG, "lto_direct_costates_batch runs the direct solver's fixed-grid path (LTO_FIXED)");
+    if (n_traj == 0) return LTO_SUCCESS;
+    if (!X_all || !u_all || !t_TU || !state_0 || !state_f || !XC_all) return fail(h, LTO_ERR_ARG, "null array argument");
+    const long long T = n_traj, N = n_nodes, ns = T * (N - 1), nn = T * N;
+    for (long long j = 0; j < T; ++j) {
+        const double* t = t_TU + j * N;
+        for (int i = 0; i < N; ++i) {
+            if (!std::isfinite(t[i])) return fail(h, LTO_ERR_ARG, "trajectory %lld: t_TU[%d] is not finite", j, i);
+            if (i > 0 && !(t[i] > t[i - 1]))
+                return fail(h, LTO_ERR_ARG, "trajectory %lld: t_TU is not strictly increasing at node %d (%.17g after %.17g)", j, i, t[i], t[i - 1]);
+        }
+        for (int k = 0; k < 6; ++k)
+            if (!std::isfinite(state_0[j * 6 + k]) || !std::isfinite(state_f[j * 6 + k]))
+                return fail(h, LTO_ERR_ARG, "trajectory %lld: state_0 / state_f is not finite", j);
+    }
+    if (h->n_child > 0) {
+        return split_trajectories(h, T, [&](lto_handle* c, long long u0, long long nu) {
+            return lto_direct_costates_batch(c, p, nu, n_nodes, nsteps, X_all + u0 * N * 6, u_all + u0 * N * 3, t_TU + u0 * N, state_0 + u0 * 6,
+                                             state_f + u0 * 6, XC_all + u0 * N * 12, multipliers ? multipliers + u0 * (N - 1) * 6 : nullptr,
+                                             du_max ? du_max + u0 : nullptr, status ? status + u0 : nullptr);
+        });
+    }
+    if (T > 0x7fffffffll) return fail(h, LTO_ERR_ARG, "too many trajectories");
+    CK(h, cudaSetDevice(h->device));
+    cudaStream_t st = h->s_compute;
+    // inputs: one staged copy; b0 / bf as lto_direct_solve_batch builds them (dV = 0, multiShoot_CRTBP_direct.jl:374-375)
+    const size_t bX = al(nn * 6 * 8), bU = al(nn * 3 * 8), bT = al(nn * 8), bB = al(T * 6 * 8);
+    const size_t in_bytes = bX + bU + bT + 2 * bB;
+    std::vector<char> stage(in_bytes);
+    {
+        char* q = stage.data();
+        memcpy(q, X_all, nn * 6 * 8); q += bX;
+        memcpy(q, u_all, nn * 3 * 8); q += bU;
+        memcpy(q, t_TU, nn * 8); q += bT;
+        double* b0 = (double*)q; q += bB;
+        double* bf = (double*)q;
+        for (long long j = 0; j < T; ++j)
+            for (int k = 0; k < 6; ++k) {
+                b0[j * 6 + k] = state_0[j * 6 + k] - X_all[(j * N) * 6 + k];
+                bf[j * 6 + k] = state_f[j * 6 + k] - X_all[(j * N + N - 1) * 6 + k];
+            }
+    }
+    int rc = ensure(h, &h->d_in, &h->d_in_cap, in_bytes); if (rc) return rc;
+    const size_t bD = al(ns * 6 * 8), bE = al(ns * 8), bSS = al(ns * 4), bJ = al(ns * 6 * 18 * 8), bXC = al(nn * 12 * 8), bV = al(T * 8),
+                 bS = al(T * 4);
+    rc = ensure(h, &h->d_out, &h->d_out_cap, bD * 2 + bE + bSS + bJ + bXC + bV + bS); if (rc) return rc;
+    h->nwt_traj = 0;                                                      // the workspace is shared with the indirect Newton update
+    rc = ensure(h, &h->d_nwt, &h->d_nwt_cap, direct_qp_workspace_bytes(T, n_nodes, 6)); if (rc) return rc;
+    char* di = (char*)h->d_in;
+    const double* dX = (const double*)di; di += bX;
+    const double* dU = (const double*)di; di += bU;
+    const double* dT = (const double*)di; di += bT;
+    const double* dB0 = (const double*)di; di += bB;
+    const double* dBf = (const double*)di;
+    char* dq = (char*)h->d_out;
+    auto take = [&](size_t b) { char* r = dq; dq += b; return r; };
+    double* dD = (double*)take(bD); double* dE = (double*)take(bE); int32_t* dSS = (int32_t*)take(bSS); double* dJ = (double*)take(bJ);
+    double* dM = (double*)take(bD); double* dXC = (double*)take(bXC); double* dV = (double*)take(bV); int32_t* dS = (int32_t*)take(bS);
+    CK(h, cudaMemcpyAsync(h->d_in, stage.data(), in_bytes, cudaMemcpyHostToDevice, st));
+    CK(h, cudaEventRecord(h->ev_t0, st));
+    rc = lto_direct_dev(h, p, ns, n_nodes, 6, nsteps, dX, nullptr, dU, nullptr, dT, nullptr, dD, dE, dSS, dJ); if (rc) return rc;
+    const double kappa = (p->default_mass > 0 ? p->default_mass : 1000.0) / (p->TU * p->TU / p->DU / 1e3);   // make_direct's mass and kthr
+    cudaError_t e = launch_direct_qp_dual(dJ, dD, dX, dU, dT, dB0, dBf, dSS, kappa, (double*)h->d_nwt, dM, dXC, dV, dS, T, n_nodes, st);
+    if (e != cudaSuccess) return fail(h, LTO_ERR_CUDA, "direct QP dual kernel launch: %s", cudaGetErrorString(e));
+    h->launches += 1;
+    CK(h, cudaEventRecord(h->ev_t1, st));
+    CK(h, cudaMemcpyAsync(XC_all, dXC, nn * 12 * 8, cudaMemcpyDeviceToHost, st));
+    if (multipliers) CK(h, cudaMemcpyAsync(multipliers, dM, ns * 6 * 8, cudaMemcpyDeviceToHost, st));
+    if (du_max) CK(h, cudaMemcpyAsync(du_max, dV, T * 8, cudaMemcpyDeviceToHost, st));
+    if (status) CK(h, cudaMemcpyAsync(status, dS, T * 4, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaStreamSynchronize(st));                                     // (also keeps `stage` alive until its copy is done)
     float ms = 0.f; CK(h, cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1)); h->last_ms = ms;
     return LTO_SUCCESS;
 }

@@ -114,6 +114,11 @@ class GpuBackend:
         return self.h.direct_solve_batch(X, U, t, state_0, state_f, mass=mass, nsteps=nsteps, max_iter=max_iter,
                                          params=capi.direct_params(Isp=Isp, MU_=MU, DU_=DU, TU_=TU))
 
+    def direct_costates(self, X, U, t, state_0, state_f, nsteps, Isp, MU, DU, TU):
+        """Costates of nstate-6 direct solutions X (B, N, 6), U (B, N, 3) in one device call (lto_direct_costates_batch)."""
+        self.calls += 1
+        return self.h.direct_costates_batch(X, U, t, state_0, state_f, nsteps=nsteps, params=capi.direct_params(Isp=Isp, MU_=MU, DU_=DU, TU_=TU))
+
 
 _default_backend = None
 
@@ -291,6 +296,23 @@ def direct_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, n_no
                 converged=r["er"] <= 1e-6, cost=_quad_cost(u_all, t_TU), state_0=s0[:, :6].copy(), state_f=sf[:, :6].copy())
 
 
+def direct_costates(X_all, u_all, t_TU, state_0, state_f, nsteps=10, backend=None):
+    """Costates of nstate-6 direct solutions in one device call (lto_direct_costates_batch): the multipliers of the direct QP's defect rows
+    at (X_all, u_all), mapped to the node costates of the 12-dim p = 2 system (_direct_costate_map is the host mirror).  At a converged
+    direct solution they are that energy-optimal problem's discrete costates, a start for multiShoot_CRTBP_indirect at a thrust limit that
+    does not bind.  X_all (T, 6, N), u_all (T, 3, N), t_TU (T, N), state_0 / state_f (T, 6): direct_transfer_sweep's results.
+    Returns dict(XC_all (T, 12, N): X_all bitwise and the costates (NaN where status != 0), multipliers (T, 6, N-1), du_max (T,): max |du|
+    in N of the QP step at the given point, status (T,): the worst LTO_ST_* of K1's segments and the QP)."""
+    be = backend or default_backend()
+    X = np.asarray(X_all, dtype=np.float64)
+    if X.ndim != 3 or X.shape[1] != 6:
+        raise ValueError("X_all must be (T, 6, n_nodes) (got %s)" % (X.shape,))
+    r = be.direct_costates(np.ascontiguousarray(X.transpose(0, 2, 1)), np.ascontiguousarray(np.asarray(u_all, dtype=np.float64).transpose(0, 2, 1)),
+                           t_TU, state_0, state_f, nsteps, 2000.0, capi.MU, capi.DU, capi.TU)
+    return dict(XC_all=r["XC_all"].transpose(0, 2, 1).copy(), multipliers=r["multipliers"].transpose(0, 2, 1).copy(), du_max=r["du_max"],
+                status=r["status"])
+
+
 G0 = 9.81                                          # the mass flow's g0 (CRTBP_prop_EP_deriv.jl:41; lto_indirect_params.g0)
 
 
@@ -325,12 +347,16 @@ def transfer_cost_indirect(XC_all, t_TU, MU, DU, TU, mass, thrustLimit, p, rho, 
 
 
 def indirect_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, thrustLimit=0.05, rho_target=1e-4, seeds=None, n_nodes=30,
-                            nsteps=10, mass=1e3, Isp=2000.0, maxIter_direct=100, backend=None):
+                            nsteps=10, mass=1e3, Isp=2000.0, maxIter_direct=100, backend=None, start="seeded"):
     """Fuel-optimal transfers for a grid of departure phases and flight times: the indirect demo's chain
     (CRTBP_Multishoot_indirect_demo.jl:166-281) run on every row of direct_transfer_sweep (nstate 6), each stage as one batched device call:
-      start   per row j, as the demo: costates 0.1 * N(0, 1) from np.random.default_rng(seeds[j]), end states pinned to state_0 / state_f,
-              1e-10 jitter on the interior nodes (seeds default to 0 .. T-1);
-      stage 1 adjoints-only solve, p = 2, 10 N, maxIter 10 (status 1 is expected there; only NaN fails the stage);
+      start = "seeded" (the default), as the demo:
+        start   per row j: costates 0.1 * N(0, 1) from np.random.default_rng(seeds[j]), end states pinned to state_0 / state_f,
+                1e-10 jitter on the interior nodes (seeds default to 0 .. T-1);
+        stage 1 adjoints-only solve, p = 2, 10 N, maxIter 10 (status 1 is expected there; only NaN fails the stage);
+      start = "direct":
+        stage 1 direct_costates of the direct solutions (the direct QP's multipliers: the discrete costates of the energy-optimal problem
+                stage 2 solves), end states pinned to state_0 / state_f, no jitter; a row whose costate status is not 0 fails here;
       stage 2 full solve, p = 2, 10 N, maxIter 50;
       stage 3 p = 1 at thrustLimit, rho = 1, maxIter 30;
       stage 4 reduceFuel_indirect_batch(device_ladder=True) to rho_target, back-off draws from a fresh np.random.default_rng(seeds[j]);
@@ -354,18 +380,26 @@ def indirect_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, th
         raise ValueError("rho_target must be in (0, 1] (got %r)" % (rho_target,))
     if n_nodes < 3:
         raise ValueError("n_nodes must be >= 3 (got %r)" % (n_nodes,))
+    if start not in ("seeded", "direct"):
+        raise ValueError("start must be 'seeded' or 'direct' (got %r)" % (start,))
     be = backend or default_backend()
     d = direct_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, n_nodes=n_nodes, nsteps=nsteps, nstate=6, mass=mass, Isp=Isp,
                               maxIter=maxIter_direct, backend=be)
     t_TU = d["t_TU"]
     N = t_TU.shape[1]
-    XC = np.empty((T, 12, N))
-    for j in range(T):
-        rng = np.random.default_rng(seeds[j])
-        XC[j] = np.vstack([d["X_all"][j], 0.1 * rng.standard_normal((6, N))])
-        XC[j, :6, 0] = d["state_0"][j]; XC[j, :6, -1] = d["state_f"][j]
-        XC[j, :, 1:-1] += 1e-10 * rng.standard_normal((12, N - 2))
     stage_failed = np.zeros(T, dtype=np.int32)
+    if start == "direct":
+        c = direct_costates(d["X_all"], d["u_all"], t_TU, d["state_0"], d["state_f"], nsteps=nsteps, backend=be)
+        XC = c["XC_all"]
+        XC[:, :6, 0] = d["state_0"]; XC[:, :6, -1] = d["state_f"]
+        stage_failed[c["status"] != 0] = 1
+    else:
+        XC = np.empty((T, 12, N))
+        for j in range(T):
+            rng = np.random.default_rng(seeds[j])
+            XC[j] = np.vstack([d["X_all"][j], 0.1 * rng.standard_normal((6, N))])
+            XC[j, :6, 0] = d["state_0"][j]; XC[j, :6, -1] = d["state_f"][j]
+            XC[j, :, 1:-1] += 1e-10 * rng.standard_normal((12, N - 2))
 
     def solve(stage, thrust, p, rho, max_iter, adjoints_only, fail_on):
         idx = np.flatnonzero(stage_failed == 0)
@@ -376,7 +410,8 @@ def indirect_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, th
         XC[idx] = Xn
         stage_failed[idx[np.isin(st, fail_on)]] = stage
 
-    solve(1, 10.0, 2.0, 1.0, 10, True, (2,))
+    if start == "seeded":
+        solve(1, 10.0, 2.0, 1.0, 10, True, (2,))
     solve(2, 10.0, 2.0, 1.0, 50, False, (1, 2))
     alive = np.flatnonzero(stage_failed == 0)
     energy_p2 = np.full(T, np.nan)
@@ -418,9 +453,11 @@ def _band_direct(blocks, n, N):
     return J
 
 
-def _qp_direct(X_all, u_all, dV1, dV2, defect, Jac_full, n, N, state_0, state_f, mass, tau, t0_TU, tf_TU, DU, TU, allowImpulsive):
+def _qp_direct(X_all, u_all, dV1, dV2, defect, Jac_full, n, N, state_0, state_f, mass, tau, t0_TU, tf_TU, DU, TU, allowImpulsive,
+               multipliers=False):
     """optimizeTraj (:248-403) for flagEnd = false: variables [X_jump | u_jump | dV1_jump | dV2_jump]
-    (tf_jump, p1_jump, p2_jump are pinned to 0 by their bounds, :288-293)."""
+    (tf_jump, p1_jump, p2_jump are pinned to 0 by their bounds, :288-293).
+    multipliers: also return the KKT multipliers of the linearised dynamics rows, (N-1, n) -- lambda of K7's K_L unknowns."""
     nX, nU = n * N, 3 * N
     nz = nX + nU + 6
     t_fixed = t0_TU + (tau + 1) / 2 * (tf_TU - t0_TU)
@@ -465,7 +502,24 @@ def _qp_direct(X_all, u_all, dV1, dV2, defect, Jac_full, n, N, state_0, state_f,
     u_update = z[nX:nX + nU].reshape(N, 3).T
     dV1_update = z[nX + nU:nX + nU + 3]; dV2_update = z[nX + nU + 3:]
     cost = float(np.sum((u_all.T.ravel() + z[nX:nX + nU]) ** 2 * w) + s * np.sum((dV1 + dV1_update) ** 2) + s * np.sum((dV2 + dV2_update) ** 2))
+    if multipliers:
+        return x_update, u_update, dV1_update, dV2_update, cost, sol[nz:nz + n * (N - 1)].reshape(N - 1, n)
     return x_update, u_update, dV1_update, dV2_update, cost
+
+
+def _direct_costate_map(blocks, lam, mass, DU, TU):
+    """Host mirror of k_direct_qp_dual's epilogue: the multipliers lam (N-1, 6) of the direct QP's defect rows -> node costates
+    [lr; lv] (6, N) of the 12-dim p = 2 system.  blocks (N-1, 6, 18) [.., row, col] = [X_i, X_{i+1}, u_i, u_{i+1}] columns.
+    p_i = Jx(i, i)^T lam_i (i < N-1), p_{N-1} = -Jx(N-2, N-1)^T lam_{N-2}; costate = -p / kappa^2, kappa = mass DU 1e3 / TU^2
+    (u in N = kappa x the nondimensional acceleration)."""
+    blocks = np.asarray(blocks, dtype=np.float64); lam = np.asarray(lam, dtype=np.float64)
+    Nm1 = lam.shape[0]
+    p = np.empty((6, Nm1 + 1))
+    for i in range(Nm1):
+        p[:, i] = blocks[i][:, :6].T @ lam[i]
+    p[:, Nm1] = -(blocks[Nm1 - 1][:, 6:12].T @ lam[Nm1 - 1])
+    kappa = mass / (TU * TU / DU / 1e3)
+    return -p / (kappa * kappa)
 
 
 def multiShoot_CRTBP_direct(X_all, u_all, tau1, tau2, t_TU, dV1, dV2, MU, DU, TU, n_nodes, nsteps, mass, Isp, X0_times, X0_states,
