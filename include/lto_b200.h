@@ -365,6 +365,32 @@ int lto_indirect_cost_batch(lto_handle* h, const lto_indirect_params* p, int64_t
                             const double* thrustLimit_traj, const double* rho_traj,
                             double* dv, double* energy, double* defect, int32_t* status);
 
+/* lto_indirect_switch_batch: the switch times of n_traj 12-dim p = 1 indirect trajectories (trajectory form, as lto_indirect_defect_traj)
+ * in one call.  Switching function S = |lv| - 1 (n = sqrt of the fma sum, as the kernels form it): thrust on where S > 0, off where
+ * S <= 0.  Every segment is integrated by the defect-only kernel K4; on each accepted step [t, t + h] S is sampled at theta = k/8 on the
+ * quintic Hermite interpolant of lv from both ends' (lv, h lv', h^2 lv'') (lv'' = U(r) lv - C^T lv', no extra right-hand sides) and each
+ * sign change is refined by safeguarded Newton on that polynomial.  At an interior node, S on opposite sides at segment i's propagated end
+ * and at node i + 1 is one switch at t_{i+1}, in the direction of node i + 1's side.  The scan is not in the error norm, so the steps and
+ * defects are bitwise those of lto_indirect_defect_traj; a trajectory's segments are assembled in order, so its result does not depend on
+ * the batch around it.
+ *   XC_all, t_TU, thrustLimit_traj, rho_traj: as lto_indirect_defect_traj with ndim = 12 (t_TU finite and non-decreasing)
+ *   max_switch  1 .. 64: switch slots per trajectory
+ *   t_switch    out, max_switch per trajectory: the first max_switch switch times in TU, in time order (NaN in unused slots)
+ *   direction   out, max_switch per trajectory: +1 a burn starts (off -> on), -1 a burn ends (0 in unused slots); they alternate, the
+ *               first opposite to on_start
+ *   n_switch    out, n_traj: the trajectory's true number of switches (it may exceed max_switch); -1 where status is not LTO_ST_OK
+ *   on_start    out, n_traj: 1 where S > 0 at node 0
+ *   defect      out, 12 x (n_nodes-1) per trajectory, the same output lto_indirect_defect_traj produces; may be NULL
+ *   status      out, n_traj: the worst LTO_ST_* (largest code) of the trajectory's segments; may be NULL
+ * p->p must be 1, p->controller LTO_CTRL_RMS and p->kernel not LTO_KERNEL_GENERIC (the scan lives in K4): otherwise LTO_ERR_ARG, as for
+ * max_switch out of range or a reversed or non-finite span (naming the first offending trajectory).  Multi-device handles split whole
+ * trajectories. */
+int lto_indirect_switch_batch(lto_handle* h, const lto_indirect_params* p, int64_t n_traj, int n_nodes,
+                              const double* XC_all, const double* t_TU,
+                              const double* thrustLimit_traj, const double* rho_traj, int max_switch,
+                              double* t_switch, int32_t* direction, int32_t* n_switch, int32_t* on_start,
+                              double* defect, int32_t* status);
+
 /* ---- peer memory: one process per GPU, results delivered to the solver rank without a collective --------
  * The rank that runs the Newton step allocates its full output arrays with lto_dev_alloc and exports them
  * (lto_ipc_export: a 64-byte cudaIpcMemHandle_t to send to the other processes by any means); every other rank

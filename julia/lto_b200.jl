@@ -234,4 +234,22 @@ function direct_costates_batch(X_batch::Array{Float64,3}, u_batch::Array{Float64
         handle[], p, n_traj, n_nodes, nsteps, X_batch, u_batch, t_batch, state_0, state_f, XC, mult, du, status))
     (XC, mult, du, status)
 end
+# ---- switch times of 12-dim p = 1 indirect trajectories in ONE call (lto_indirect_switch_batch): the sign changes of |lv| - 1 (thrust on
+# where > 0) located on the defect-only kernel's steps, with the node rule between segments.  XC_batch: 12 x n_nodes x n_traj; t_batch:
+# n_nodes x n_traj; thrustLimit, rho: per trajectory.  Returns (t_switch max_switch x n_traj in TU (NaN unused), direction (+1 a burn starts,
+# -1 it ends, 0 unused), n_switch (the true count, -1 where status is not OK), on_start, status).  Like the rest of this shim, not run under
+# Julia here (the same ABI is exercised from Python).
+function indirect_switch_batch(XC_batch::Array{Float64,3}, t_batch::Matrix{Float64}, MU, DU, TU, mass, thrustLimit::Vector{Float64},
+                               rho::Vector{Float64}; max_switch=16)
+    n_nodes = size(XC_batch, 2); n_traj = size(XC_batch, 3)
+    size(XC_batch, 1) == 12 || error("indirect_switch_batch: XC_batch must have 12 rows")
+    t_sw = zeros(max_switch, n_traj); dir = zeros(Int32, max_switch, n_traj)
+    n_sw = zeros(Int32, n_traj); on = zeros(Int32, n_traj); status = zeros(Int32, n_traj)
+    prm = iparams((MU, DU, TU, thrustLimit[1], mass, 1.0, 1.0, rho[1]))
+    GC.@preserve XC_batch t_batch thrustLimit rho t_sw dir n_sw on status check(ccall((:lto_indirect_switch_batch, lib), Cint,
+        (Ptr{Cvoid}, Ref{IndirectParams}, Int64, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Cint, Ptr{Float64}, Ptr{Int32},
+         Ptr{Int32}, Ptr{Int32}, Ptr{Float64}, Ptr{Int32}),
+        handle[], prm, n_traj, n_nodes, XC_batch, t_batch, thrustLimit, rho, max_switch, t_sw, dir, n_sw, on, C_NULL, status))
+    (t_sw, dir, n_sw, on, status)
+end
 end # module

@@ -33,6 +33,7 @@ EXPORTS = [
     "lto_indirect_newton", "lto_indirect_newton_dev", "lto_indirect_newton_resolve_dev", "lto_indirect_solve_batch", "lto_direct_qp", "lto_direct_qp_dev", "lto_direct_solve_batch",
     "lto_indirect_newton_nd", "lto_indirect_newton_nd_dev", "lto_indirect_newton_resolve_nd_dev", "lto_indirect_solve_batch_nd",
     "lto_indirect_reduce_fuel_batch", "lto_stack_guess_batch", "lto_indirect_cost_batch", "lto_direct_costates_batch",
+    "lto_indirect_switch_batch",
 ]
 
 
@@ -120,6 +121,7 @@ def lib():
         L.lto_stack_guess_batch.argtypes = [vp, vp, i64, ci, vp, ci, vp, ci] + [vp] * 3 + [vp] * 5
         L.lto_indirect_cost_batch.argtypes = [vp, vp, i64, ci] + [vp] * 4 + [vp] * 4
         L.lto_direct_costates_batch.argtypes = [vp, vp, i64, ci, ci] + [vp] * 5 + [vp] * 4
+        L.lto_indirect_switch_batch.argtypes = [vp, vp, i64, ci] + [vp] * 4 + [ci] + [vp] * 6
         _lib = L
     return _lib
 
@@ -470,6 +472,45 @@ class Handle:
         self._ck(lib().lto_indirect_cost_batch(self._h, C.addressof(p), n_traj, n_nodes, _ptr(XC), _ptr(t_TU), _ptr(tl), _ptr(rh), _ptr(dv),
                                                _ptr(energy), _ptr(d), _ptr(status)))
         out = dict(dv=dv, energy=energy, status=status)
+        if defect:
+            out["defect"] = d
+        return out
+
+    def indirect_switch_batch(self, XC_all, t_TU, params=None, thrustLimit=None, rho=None, max_switch=16, defect=False):
+        """Switch times of 12-dim p = 1 indirect trajectories in one device call (lto_indirect_switch_batch): the sign changes of
+        S = |lv| - 1 (thrust on where S > 0), located on the defect-only kernel's steps, with one switch at a node where the propagated end of
+        the segment before it and the node lie on opposite sides.  XC_all: (n_traj, n_nodes, 12); t_TU: (n_traj, n_nodes), finite and
+        non-decreasing; thrustLimit / rho: scalars or (n_traj,); params.p must be 1 and params.controller LTO_CTRL_RMS; max_switch in
+        [1, 64].  defect: also return the defects (bitwise those of indirect_traj(jac=False)).
+        Returns dict(t_switch (n_traj, max_switch) in TU, NaN in unused slots; direction (n_traj, max_switch): +1 a burn starts, -1 it ends,
+        0 unused; n_switch (n_traj,): the true count (> max_switch: truncated; -1 where status is not LTO_ST_OK); on_start (n_traj,);
+        status (n_traj,)[, defect (n_traj, n_nodes-1, 12)])."""
+        p = params or indirect_params()
+        XC = _f64(XC_all)
+        if XC.ndim != 3 or XC.shape[2] != 12:
+            raise ValueError("XC_all must be (n_traj, n_nodes, 12): the switch scan is in the 12-dim kernel (got %s)" % (XC.shape,))
+        n_traj, n_nodes, _ = XC.shape
+        if n_nodes < 2:
+            raise ValueError("n_nodes must be >= 2 (got %d)" % n_nodes)
+        if p.controller != LTO_CTRL_RMS:
+            raise ValueError("the switch scan needs controller = LTO_CTRL_RMS (got %d)" % p.controller)
+        if p.p != 1.0:
+            raise ValueError("switch times are defined for the p = 1 law only (got p = %g)" % p.p)
+        if not (isinstance(max_switch, (int, np.integer)) and 1 <= max_switch <= 64):
+            raise ValueError("max_switch must be an integer in [1, 64] (got %r)" % (max_switch,))
+        t_TU = _shaped("t_TU", t_TU, (n_traj, n_nodes))
+        bad = ~np.isfinite(t_TU).all(axis=1) | (np.diff(t_TU, axis=1) < 0).any(axis=1)
+        if bad.any():
+            raise ValueError("trajectory %d: t_TU must be finite and non-decreasing (reversed spans are not supported)" % int(np.argmax(bad)))
+        tl = _per_unit("thrustLimit", thrustLimit, n_traj)
+        rh = _per_unit("rho", rho, n_traj)
+        K = int(max_switch)
+        ts = np.empty((n_traj, K)); dr = np.empty((n_traj, K), dtype=np.int32)
+        ns = np.empty(n_traj, dtype=np.int32); on = np.empty(n_traj, dtype=np.int32); status = np.empty(n_traj, dtype=np.int32)
+        d = np.empty((n_traj, n_nodes - 1, 12)) if defect else None
+        self._ck(lib().lto_indirect_switch_batch(self._h, C.addressof(p), n_traj, n_nodes, _ptr(XC), _ptr(t_TU), _ptr(tl), _ptr(rh), K,
+                                                 _ptr(ts), _ptr(dr), _ptr(ns), _ptr(on), _ptr(d), _ptr(status)))
+        out = dict(t_switch=ts, direction=dr, n_switch=ns, on_start=on, status=status)
         if defect:
             out["defect"] = d
         return out

@@ -782,6 +782,92 @@ int lto_indirect_cost_batch(lto_handle* h, const lto_indirect_params* p, int64_t
     return LTO_SUCCESS;
 }
 
+int lto_indirect_switch_batch(lto_handle* h, const lto_indirect_params* p, int64_t n_traj, int n_nodes, const double* XC_all,
+                              const double* t_TU, const double* thrustLimit_traj, const double* rho_traj, int max_switch, double* t_switch,
+                              int32_t* direction, int32_t* n_switch, int32_t* on_start, double* defect, int32_t* status) {
+    LTO_NVTX();
+    if (!h) return fail(nullptr, LTO_ERR_ARG, "null handle");
+    if (!p) return fail(h, LTO_ERR_ARG, "null params");
+    if (n_traj < 0) return fail(h, LTO_ERR_ARG, "negative trajectory count");
+    if (n_nodes < 2) return fail(h, LTO_ERR_ARG, "n_nodes must be >= 2 (got %d)", n_nodes);
+    if (p->controller != LTO_CTRL_RMS)
+        return fail(h, LTO_ERR_ARG, "the switch scan runs in the defect-only kernel K4: controller must be LTO_CTRL_RMS (got %d)", p->controller);
+    if (p->kernel == LTO_KERNEL_GENERIC) return fail(h, LTO_ERR_ARG, "the generic kernel has no switch scan (kernel must be AUTO or FAST)");
+    if (p->p != 1.0) return fail(h, LTO_ERR_ARG, "switch times are defined for the p = 1 law only (got p = %g)", p->p);
+    if (max_switch < 1 || max_switch > 64) return fail(h, LTO_ERR_ARG, "max_switch must be in [1, 64] (got %d)", max_switch);
+    IndirectArgs a; memset(&a, 0, sizeof a);
+    int rc = make_indirect(h, p, 12, false, &a); if (rc) return rc;
+    if (n_traj == 0) return LTO_SUCCESS;
+    if (!XC_all || !t_TU || !t_switch || !direction || !n_switch || !on_start) return fail(h, LTO_ERR_ARG, "null array argument");
+    const long long T = n_traj, N = n_nodes, n_seg = T * (N - 1), K = max_switch;
+    if (n_seg > 0x7fffffffll) return fail(h, LTO_ERR_ARG, "too many segments (%lld)", n_seg);
+    for (long long j = 0; j < T; ++j) {
+        const double* t = t_TU + j * N;
+        for (int i = 0; i < N; ++i) {
+            if (!std::isfinite(t[i])) return fail(h, LTO_ERR_ARG, "trajectory %lld: t_TU[%d] is not finite", j, i);
+            if (i > 0 && t[i] < t[i - 1])
+                return fail(h, LTO_ERR_ARG, "trajectory %lld: t_TU[%d] < t_TU[%d] (%.17g < %.17g): reversed spans are not supported", j, i, i - 1,
+                            t[i], t[i - 1]);
+        }
+    }
+    if (h->n_child > 0) {
+        return split_trajectories(h, T, [&](lto_handle* c, long long u0, long long nu) {
+            return lto_indirect_switch_batch(c, p, nu, n_nodes, XC_all + u0 * N * 12, t_TU + u0 * N,
+                                             thrustLimit_traj ? thrustLimit_traj + u0 : nullptr, rho_traj ? rho_traj + u0 : nullptr, max_switch,
+                                             t_switch + u0 * K, direction + u0 * K, n_switch + u0, on_start + u0,
+                                             defect ? defect + u0 * (N - 1) * 12 : nullptr, status ? status + u0 : nullptr);
+        });
+    }
+    CK(h, cudaSetDevice(h->device));
+    cudaStream_t st = h->s_compute;
+    // inputs: one staged copy
+    const size_t bX = al(T * N * 12 * 8), bT = al(T * N * 8), bP = al(T * 8);
+    const size_t in_bytes = bX + bT + (thrustLimit_traj ? bP : 0) + (rho_traj ? bP : 0);
+    std::vector<char> stage(in_bytes);
+    {
+        char* q = stage.data();
+        memcpy(q, XC_all, T * N * 12 * 8); q += bX;
+        memcpy(q, t_TU, T * N * 8); q += bT;
+        if (thrustLimit_traj) { memcpy(q, thrustLimit_traj, T * 8); q += bP; }
+        if (rho_traj) memcpy(q, rho_traj, T * 8);
+    }
+    rc = ensure(h, &h->d_in, &h->d_in_cap, in_bytes); if (rc) return rc;
+    // per segment: defect, status, switch times / directions, count, sides; per trajectory: times / directions, n_switch, on_start, status
+    const size_t bD = al(n_seg * 12 * 8), bS = al(n_seg * 4), bSW = al(n_seg * K * 8), bSD = al(n_seg * K * 4);
+    const size_t bTW = al(T * K * 8), bTD = al(T * K * 4), bI = al(T * 4);
+    rc = ensure(h, &h->d_out, &h->d_out_cap, bD + 3 * bS + bSW + bSD + bTW + bTD + 3 * bI); if (rc) return rc;
+    char* di = (char*)h->d_in;
+    double* dX = (double*)di; di += bX;
+    double* dT = (double*)di; di += bT;
+    double* dTL = nullptr; if (thrustLimit_traj) { dTL = (double*)di; di += bP; }
+    double* dRH = nullptr; if (rho_traj) dRH = (double*)di;
+    char* dq = (char*)h->d_out;
+    double* dD = (double*)dq; dq += bD; int32_t* dS = (int32_t*)dq; dq += bS;
+    int32_t* dCnt = (int32_t*)dq; dq += bS; int32_t* dSide = (int32_t*)dq; dq += bS;
+    double* dSwT = (double*)dq; dq += bSW; int32_t* dSwD = (int32_t*)dq; dq += bSD;
+    double* dTW = (double*)dq; dq += bTW; int32_t* dTD = (int32_t*)dq; dq += bTD;
+    int32_t* dN = (int32_t*)dq; dq += bI; int32_t* dOn = (int32_t*)dq; dq += bI; int32_t* dST = (int32_t*)dq;
+    CK(h, cudaMemcpyAsync(h->d_in, stage.data(), in_bytes, cudaMemcpyHostToDevice, st));
+    a.x0 = dX; a.t0 = dT; a.t1 = dT + 1; a.x_target = dX + 12; a.thrustLimit_arr = dTL; a.rho_arr = dRH;
+    a.defect = dD; a.status = dS; a.n_seg = n_seg; a.npt = n_nodes; a.counter = h->d_ctr;
+    a.sw_t = dSwT; a.sw_dir = dSwD; a.sw_count = dCnt; a.sw_side = dSide; a.max_switch = max_switch;
+    CK(h, cudaEventRecord(h->ev_t0, st));
+    int nl = 0;
+    const cudaError_t e = launch_indirect_switch(a, T, dT, dTW, dTD, dN, dOn, dST, st, &nl);
+    h->launches += nl;
+    if (e != cudaSuccess) return fail(h, LTO_ERR_CUDA, "indirect switch launch: %s", cudaGetErrorString(e));
+    CK(h, cudaEventRecord(h->ev_t1, st));
+    CK(h, cudaMemcpyAsync(t_switch, dTW, T * K * 8, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(direction, dTD, T * K * 4, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(n_switch, dN, T * 4, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(on_start, dOn, T * 4, cudaMemcpyDeviceToHost, st));
+    if (status) CK(h, cudaMemcpyAsync(status, dST, T * 4, cudaMemcpyDeviceToHost, st));
+    if (defect) CK(h, cudaMemcpyAsync(defect, dD, n_seg * 12 * 8, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaStreamSynchronize(st));                                     // (also keeps `stage` alive until its copy is done)
+    float ms = 0.f; CK(h, cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1)); h->last_ms = ms;
+    return LTO_SUCCESS;
+}
+
 int lto_sumsq_dev(lto_handle* h, const double* v, int64_t n_rows, int64_t row_len, double* out) {
     LTO_NVTX();
     if (!h) return fail(nullptr, LTO_ERR_ARG, "null handle");

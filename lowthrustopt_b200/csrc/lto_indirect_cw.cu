@@ -33,6 +33,7 @@
 // sequences and agree to the integration tolerance, not to rounding.
 #include "lto_internal.h"
 #include "lto_cw_common.cuh"
+#include "lto_switch.h"
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
@@ -787,14 +788,29 @@ __device__ __forceinline__ void k4_stage(KStore& K, const double (&x)[ND], doubl
     }
 }
 
+// The switch pass's scan of one accepted step [t, t + h] from x (start) to xn (end), out of line so that K4's main loop does not grow:
+// writes the step's switches after the segment's `count` (at most `cap` per segment) and returns the new count (lto_switch.h).
+__device__ __noinline__ int sw_step_call(double r0, double r1, double r2, double lr0, double lr1, double lr2, double lv0, double lv1, double lv2,
+                                         double s0, double s1, double s2, double sr0, double sr1, double sr2, double sv0, double sv1, double sv2,
+                                         double mu, double mu1, double omega, double t, double h, int count, int cap, double* t_out,
+                                         int32_t* dir_out) {
+    SwEnd e0, e1;
+    sw_end(r0, r1, r2, lr0, lr1, lr2, lv0, lv1, lv2, mu, mu1, omega, e0);
+    sw_end(s0, s1, s2, sr0, sr1, sr2, sv0, sv1, sv2, mu, mu1, omega, e1);
+    return sw_scan(e0, e1, t, h, count, cap, t_out, dir_out);
+}
+
 constexpr int K4I_THREADS = 128;
 
 // QUAD = false: the defect-only kernel k_indirect_state.  QUAD = true (k_indirect_state_cost): the same steps (the quadratures are not in
 // the error norm, so the step sequence and every state are bitwise those of QUAD = false) and, per segment, a.quad[2 seg] =
 // int |a_u| dt and a.quad[2 seg + 1] = int |a_u|^2 dt, accumulated over the accepted steps only (NaN for a segment whose status is not
-// LTO_ST_OK: it never reached t1).  `a` is taken by value: so
+// LTO_ST_OK: it never reached t1).  SW (k_indirect_state_switch): the same steps again (the scan is not in the error norm either) and,
+// per segment, the switches of |lv| - 1 located on every accepted step (sw_step_call) in a.sw_t / a.sw_dir (at most a.max_switch),
+// their count in a.sw_count (0 for a segment whose status is not LTO_ST_OK) and the sides of |lv| - 1 at the segment's start and
+// propagated end in a.sw_side.  `a` is taken by value: so
 // k_indirect_state compiles to the same SASS as when this body was its own (through a reference, the register allocation changed).
-template <bool QUAD>
+template <bool QUAD, bool SW>
 __device__ __forceinline__ void k4_body(IndirectArgs a) {
     const unsigned fullmask = 0xffffffffu;
     double atol = a.cfg.atol, rtol = a.cfg.rtol;                          // per slot: state_tol_scale(p, rho) of the slot's segment
@@ -807,6 +823,7 @@ __device__ __forceinline__ void k4_body(IndirectArgs a) {
     int na = 0, nt = 0, status = 0;
     bool active = false, lastrej = false, last = false, have = false, exhausted = false;
     double q_dv = 0.0, q_e = 0.0, s_dv = 0.0, s_e = 0.0;                  // QUAD: the segment's quadratures and the attempted step's sums
+    int n_sw = 0;                                                         // SW: the segment's switches so far
     while (true) {
         bool finished = false;
         if (have && active) {
@@ -817,6 +834,10 @@ __device__ __forceinline__ void k4_body(IndirectArgs a) {
                 q = fmin(5.0, fmax(0.2, q));
                 if (eest <= 1.0) {
                     ++na;
+                    if (SW)
+                        n_sw = sw_step_call(x[0], x[1], x[2], x[6], x[7], x[8], x[9], x[10], x[11], xn[0], xn[1], xn[2], xn[6], xn[7], xn[8],
+                                            xn[9], xn[10], xn[11], a.c.mu, a.c.m1, a.c.omega, tcur, h, n_sw, a.max_switch,
+                                            a.sw_t + seg * a.max_switch, a.sw_dir + seg * a.max_switch);
 #pragma unroll
                     for (int i = 0; i < ND; ++i) x[i] = xn[i];
                     if (QUAD) { q_dv = fma(h, s_dv, q_dv); q_e = fma(h, s_e, q_e); }
@@ -845,6 +866,10 @@ __device__ __forceinline__ void k4_body(IndirectArgs a) {
                 const double nanv = __longlong_as_double(0x7ff8000000000000ll);
                 a.quad[2 * seg] = status ? nanv : q_dv; a.quad[2 * seg + 1] = status ? nanv : q_e;
             }
+            if (SW) {                                                     // a segment that did not reach t1 has no switches
+                a.sw_count[seg] = status ? 0 : n_sw;
+                a.sw_side[seg] = sw_side(a.x0[ia * ND + 9], a.x0[ia * ND + 10], a.x0[ia * ND + 11]) | (sw_side(x[9], x[10], x[11]) << 1);
+            }
             active = false;
         }
         bool fresh = false;
@@ -866,6 +891,7 @@ __device__ __forceinline__ void k4_body(IndirectArgs a) {
                 { const double ts = state_tol_scale(a.c.p, rho); atol = a.cfg.atol * ts; rtol = a.cfg.rtol * ts; }
                 na = 0; nt = 0; status = 0; lastrej = false;
                 if (QUAD) { q_dv = 0.0; q_e = 0.0; }
+                if (SW) n_sw = 0;
                 active = true; fresh = true;
             } else {
                 exhausted = true;
@@ -909,8 +935,9 @@ __device__ __forceinline__ void k4_body(IndirectArgs a) {
     }
 }
 
-__global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state(IndirectArgs a) { k4_body<false>(a); }
-__global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state_cost(IndirectArgs a) { k4_body<true>(a); }
+__global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state(IndirectArgs a) { k4_body<false, false>(a); }
+__global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state_cost(IndirectArgs a) { k4_body<true, false>(a); }
+__global__ void __launch_bounds__(K4I_THREADS, 2) k_indirect_state_switch(IndirectArgs a) { k4_body<false, true>(a); }
 
 }  // namespace icw
 
@@ -987,6 +1014,71 @@ cudaError_t launch_indirect_cost(const IndirectArgs& a, long long n_traj, double
     *n_launch = 1;
     icw::k_cost_sum<<<(unsigned)((n_traj + 127) / 128), 128, 0, st>>>(a.quad, a.status, n_traj, a.npt - 1, dv_scale, e_scale, dv, energy,
                                                                       status_traj);
+    e = cudaGetLastError(); if (e != cudaSuccess) return e;
+    *n_launch = 2;
+    return cudaSuccess;
+}
+
+namespace icw {
+// Per trajectory, its segments' switches in time order with the node rule between them: where the side of |lv| - 1 at segment i's
+// propagated end and at node i + 1 (segment i + 1's start) differ, one switch at t_{i+1} in the direction of node i + 1's side.  The
+// first `cap` switches are written (NaN / 0 in the unused slots), n_switch is the true total (-1 where the worst segment status is not
+// LTO_ST_OK).  No atomics: a row's result does not depend on the batch around it.
+__global__ void k_switch_gather(const int32_t* __restrict__ seg_status, const int32_t* __restrict__ sw_count, const int32_t* __restrict__ sw_side,
+                                const double* __restrict__ sw_t, const int32_t* __restrict__ sw_dir, const double* __restrict__ t_node,
+                                long long n_traj, int npt, int cap, double* __restrict__ t_switch, int32_t* __restrict__ direction,
+                                int32_t* __restrict__ n_switch, int32_t* __restrict__ on_start, int32_t* __restrict__ status) {
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n_traj) return;
+    const int ns = npt - 1;
+    const long long s0 = j * ns;
+    int w = 0;
+    for (int i = 0; i < ns; ++i) w = max(w, (int)seg_status[s0 + i]);
+    double* to = t_switch + j * cap;
+    int32_t* dout = direction + j * cap;
+    int n = 0;
+    if (w == 0) {
+        int end_prev = 0;
+        for (int i = 0; i < ns; ++i) {
+            const long long s = s0 + i;
+            const int sd = sw_side[s];
+            if (i > 0 && (sd & 1) != end_prev) {                          // the node rule at t_i
+                if (n < cap) { to[n] = t_node[j * npt + i]; dout[n] = (sd & 1) ? 1 : -1; }
+                ++n;
+            }
+            const int c = sw_count[s];
+            for (int k = 0; k < c && k < cap && n + k < cap; ++k) { to[n + k] = sw_t[s * cap + k]; dout[n + k] = sw_dir[s * cap + k]; }
+            n += c;
+            end_prev = sd >> 1;
+        }
+    }
+    const double nanv = __longlong_as_double(0x7ff8000000000000ll);
+    for (int k = w == 0 ? min(n, cap) : 0; k < cap; ++k) { to[k] = nanv; dout[k] = 0; }
+    n_switch[j] = w ? -1 : n;
+    on_start[j] = sw_side[s0] & 1;
+    if (status) status[j] = w;
+}
+}  // namespace icw
+
+cudaError_t launch_indirect_switch(const IndirectArgs& a, long long n_traj, const double* t_node, double* t_switch, int32_t* direction,
+                                   int32_t* n_switch, int32_t* on_start, int32_t* status_traj, cudaStream_t st, int* n_launch) {
+    *n_launch = 0;
+    if (a.phi != nullptr || a.counter == nullptr || a.status == nullptr || a.sw_t == nullptr || a.sw_dir == nullptr || a.sw_count == nullptr ||
+        a.sw_side == nullptr || a.max_switch < 1 || a.cfg.controller != 0 || a.npt < 2 || a.n_seg <= 0 || a.n_seg > 0x7fffffffll ||
+        a.n_seg != n_traj * (a.npt - 1))
+        return cudaErrorNotSupported;
+    int dev = 0, n_sm = 0;
+    cudaError_t e = cudaGetDevice(&dev); if (e != cudaSuccess) return e;
+    e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev); if (e != cudaSuccess) return e;
+    e = cudaMemsetAsync(a.counter, 0, sizeof(unsigned long long), st); if (e != cudaSuccess) return e;
+    const long long blocks = (a.n_seg + icw::K4I_THREADS - 1) / icw::K4I_THREADS;
+    const int grid = (int)std::min<long long>(blocks, (long long)n_sm * 2);
+    icw::k_indirect_state_switch<<<grid, icw::K4I_THREADS, 0, st>>>(a);
+    e = cudaGetLastError(); if (e != cudaSuccess) return e;
+    *n_launch = 1;
+    icw::k_switch_gather<<<(unsigned)((n_traj + 127) / 128), 128, 0, st>>>(a.status, a.sw_count, a.sw_side, a.sw_t, a.sw_dir, t_node, n_traj,
+                                                                           a.npt, a.max_switch, t_switch, direction, n_switch, on_start,
+                                                                           status_traj);
     e = cudaGetLastError(); if (e != cudaSuccess) return e;
     *n_launch = 2;
     return cudaSuccess;

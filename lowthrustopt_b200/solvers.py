@@ -8,6 +8,8 @@
                                                                         direct_transfer_sweep: those guesses solved by the batched direct solver)
     indirect_transfer_sweep      CRTBP_Multishoot_indirect_demo.jl:166-281 over a direct_transfer_sweep, batched, with each result's
                                  transfer_cost_indirect (delta-v and control energy; no reference counterpart)
+    thrust_arcs_indirect         the burns of p = 1 indirect solutions (switch times of |lv| - 1; no reference counterpart on the
+                                 shooting path)
     densify, jacobiConstant, interpInitialStates, find_tau   src/HelperFunctions.jl:10-101
 
 Same names, argument order and return values.  Arrays use the reference's shapes
@@ -108,6 +110,12 @@ class GpuBackend:
         """delta-v and control energy of 12-dim trajectories XC (B, N, 12) in one device call (lto_indirect_cost_batch)."""
         self.calls += 1
         return self.h.indirect_cost_batch(XC, t, params=self._ip(params), thrustLimit=thrustLimit, rho=rho, defect=defect)
+
+    def indirect_switches(self, XC, t, params, thrustLimit=None, rho=None, max_switch=16, defect=False):
+        """Switch times of p = 1 12-dim trajectories XC (B, N, 12) in one device call (lto_indirect_switch_batch)."""
+        self.calls += 1
+        return self.h.indirect_switch_batch(XC, t, params=self._ip(params), thrustLimit=thrustLimit, rho=rho, max_switch=max_switch,
+                                            defect=defect)
 
     def direct_solve_batch(self, X, U, t, state_0, state_f, mass, nsteps, max_iter, Isp, MU, DU, TU):
         self.calls += 1
@@ -344,6 +352,50 @@ def transfer_cost_indirect(XC_all, t_TU, MU, DU, TU, mass, thrustLimit, p, rho, 
     params = (MU, DU, TU, float(tl[0]) if T else 0.0, mass, 1.0, p, float(rh[0]) if T else 1.0)
     r = be.indirect_cost(np.ascontiguousarray(XC.transpose(0, 2, 1)), t_TU, params, thrustLimit=tl, rho=rh)
     return dict(dv=r["dv"], energy=r["energy"], propellant=mass * -np.expm1(-r["dv"] / (Isp * G0)), status=r["status"])
+
+
+def thrust_arcs_indirect(XC_all, t_TU, MU, DU, TU, mass, thrustLimit, rho, max_switch=16, backend=None):
+    """The burns of p = 1 indirect trajectories XC_all (T, 12, N) on the time grids t_TU (T, N); thrustLimit and rho: scalars or (T,)
+    (for a sweep's rows: its XC_all, t_TU and rho_last).  ONE device call (lto_indirect_switch_batch) locates the switches of
+    S = |lv| - 1 (thrust on where S > 0) on every segment's adaptive steps, with the node rule between segments.
+    Returns dict(t_switch (T, max_switch) TU, direction (T, max_switch) (+1 a burn starts, -1 it ends), n_switch (T,) (the true count;
+    -1 where status is not OK), on_start (T,), status (T,), and per row: arcs, a (k, 2) array of [t_on, t_off] in TU clipped to
+    [t_TU[0], t_TU[-1]] (None where the status is not OK or n_switch > max_switch), n_burns (k; -1 where arcs is None) and on_time
+    (the total burn time in TU; NaN where arcs is None))."""
+    XC = np.asarray(XC_all, dtype=np.float64)
+    if XC.ndim != 3 or XC.shape[1] != 12 or XC.shape[2] < 2:
+        raise ValueError("XC_all must be (T, 12, n_nodes >= 2): switch times are located in the 12-dim system (got %s)" % (XC.shape,))
+    T, _, N = XC.shape
+    t_TU = np.asarray(t_TU, dtype=np.float64)
+    if t_TU.shape != (T, N):
+        raise ValueError("t_TU must be (T, n_nodes) = %s (got %s)" % ((T, N), t_TU.shape))
+    be = backend or default_backend()
+    tl = np.broadcast_to(np.asarray(thrustLimit, dtype=np.float64), (T,)).copy()
+    rh = np.broadcast_to(np.asarray(rho, dtype=np.float64), (T,)).copy()
+    params = (MU, DU, TU, float(tl[0]) if T else 0.0, mass, 1.0, 1.0, float(rh[0]) if T else 1.0)
+    r = be.indirect_switches(np.ascontiguousarray(XC.transpose(0, 2, 1)), t_TU, params, thrustLimit=tl, rho=rh, max_switch=max_switch)
+    arcs, n_burns, on_time = [], np.full(T, -1, dtype=np.int64), np.full(T, np.nan)
+    for j in range(T):
+        n = int(r["n_switch"][j])
+        if r["status"][j] != 0 or n < 0 or n > max_switch:
+            arcs.append(None)
+            continue
+        t0, tf = t_TU[j, 0], t_TU[j, -1]
+        on, begin, a = bool(r["on_start"][j]), t0, []
+        for ts, d in zip(r["t_switch"][j, :n], r["direction"][j, :n]):
+            if d > 0 and not on:
+                on, begin = True, ts
+            elif d < 0 and on:
+                on = False
+                a.append((begin, ts))
+        if on:
+            a.append((begin, tf))
+        a = np.clip(np.array(a, dtype=np.float64).reshape(-1, 2), t0, tf)
+        arcs.append(a)
+        n_burns[j] = len(a)
+        on_time[j] = float(np.sum(a[:, 1] - a[:, 0]))
+    return dict(t_switch=r["t_switch"], direction=r["direction"], n_switch=r["n_switch"], on_start=r["on_start"], status=r["status"],
+                arcs=arcs, n_burns=n_burns, on_time=on_time)
 
 
 def indirect_transfer_sweep(X0_states, Xf_states, tau1, tof1_days, tof2_days, thrustLimit=0.05, rho_target=1e-4, seeds=None, n_nodes=30,
