@@ -45,7 +45,13 @@ extern "C" {
  * LTO_ERR_ARG naming the first such segment; the device-pointer entry points (lto_indirect_dev, the batched solver) cannot look at
  * the times and treat such a segment as an empty span -- callers of those must not pass reversed spans.  time_direction = -1 in the
  * parameters (the backward legs of the reference's direct method and of its trajectory stacking) is the supported way of
- * integrating the time-reversed dynamics. */
+ * integrating the time-reversed dynamics.  The host-buffer entry points also refuse a NaN or infinite t0 / t1; the device-pointer
+ * entry points still do not look at the times (the generic kernel reports such a segment as LTO_ST_NAN, or LTO_ST_HMIN when reversed).
+ * Direct segments (both legs run from ta to t_mid = ta + (tb - ta) / 2), every entry point and kernel:
+ *   - a NaN or infinite ta / tb gives LTO_ST_NAN;
+ *   - tb == ta gives LTO_ST_OK with zero-length legs;
+ *   - tb < ta: LTO_FIXED integrates the legs backwards on the same grid (what the reference's ode7_8 does), status LTO_ST_OK;
+ *     LTO_ADAPTIVE does not integrate such a leg and gives LTO_ST_HMIN. */
 enum { LTO_ST_OK = 0, LTO_ST_NAN = 1, LTO_ST_HMIN = 2, LTO_ST_MAXSTEPS = 3, LTO_ST_BADP = 4 };
 /* return codes */
 enum { LTO_SUCCESS = 0, LTO_ERR_CUDA = -1, LTO_ERR_ARG = -2, LTO_ERR_NODEVICE = -3, LTO_ERR_NOMEM = -4 };

@@ -525,10 +525,13 @@ static int indirect_host(lto_handle* h, const lto_indirect_params* p, long long 
     if (!x0 || !t0 || !defect || (npt == 0 && !t1) || (want_jac && !phi)) return fail(h, LTO_ERR_ARG, "null array argument");
     // Reversed spans (t1 < t0): the reference's solve(ODEProblem(.., (t0, t1))) would integrate backwards; the kernels step forwards
     // only and would hand back x0 and Phi = I.  A wrong answer with status OK is worse than a refused call (ADVICE r1): reject.
+    // The same holds for a NaN time (every comparison in the controllers is false), so non-finite times are refused too.
     for (long long sgm = 0; sgm < n_seg; ++sgm) {
         const long long ia = lto_node_a(sgm, npt);
         const double ta = t0[ia], tb = npt > 0 ? t0[ia + 1] : t1[ia];
-        if (tb < ta) return fail(h, LTO_ERR_ARG, "segment %lld has t1 < t0 (%.17g < %.17g): reversed spans are not supported", sgm, tb, ta);
+        if (!(std::isfinite(ta) && std::isfinite(tb) && tb >= ta))
+            return fail(h, LTO_ERR_ARG, "segment %lld has a non-finite or reversed span (t0 = %.17g, t1 = %.17g): non-finite and reversed spans "
+                        "are not supported", sgm, ta, tb);
     }
     CK(h, cudaSetDevice(h->device));
     const int ND = ndim;

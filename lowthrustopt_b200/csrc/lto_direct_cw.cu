@@ -508,8 +508,8 @@ __device__ __forceinline__ void state_warp_adapt(const DirectArgs& a, long long 
         // ---- drive_ode78 (lto_prop_generic.cuh) / ode78 (ode.jl:477-534)
         const double hmax = (tfinal - t0) / 2.5, hmin = (tfinal - t0) / 1e7;
         double tt = t0, h = (tfinal - t0) / 50.0;
-        int status = 0, nt = 0;
-        bool done = !((tt < tfinal) && (h >= hmin));
+        int status = span_status(t0, tfinal), nt = 0;                      // NaN / infinite / reversed span: flagged, never integrated
+        bool done = status != 0 || !((tt < tfinal) && (h >= hmin));
         while (true) {
             const unsigned slot = g & (NSLOT - 1), use = g / NSLOT;
             double* slotp = recs + (size_t)(t * NSLOT + slot) * C::STEP_DOUBLES * 32;

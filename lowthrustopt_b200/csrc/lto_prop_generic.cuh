@@ -123,10 +123,21 @@ LTO_HD int drive_fixed(RHS& rhs, double* y, double t0, double t1, int nsteps, do
     return st;
 }
 
+// Span rule of the adaptive controllers.  Their loop conditions (t < tfinal, h >= hmin) are false for a NaN end point and for a
+// reversed span, so without this the leg would come back as x0 with status OK, never integrated: a non-finite end point is
+// LTO_ST_NAN, tfinal < t0 is LTO_ST_HMIN (the leg does not reach its end time).  tfinal == t0 stays OK (x0, no attempts).
+LTO_HD bool finite_time(double t) { return fabs(t) <= 1.7976931348623157e308; }   // false for +-inf and NaN
+LTO_HD int span_status(double t0, double tfinal) {
+    if (!(finite_time(t0) && finite_time(tfinal))) return LTO_ST_NAN;
+    return (tfinal < t0) ? LTO_ST_HMIN : LTO_OK;
+}
+
 // ode78 controller (ode.jl:477-534).  NE = number of leading components the norms span.
 template <int NT, class RHS>
 LTO_HD int drive_ode78(RHS& rhs, double* y, double t0, double tfinal, double tol, int ne, int max_attempts,
                        int* nacc, int* natt, double* k, double* ytmp, double* ynew, double* gam) {
+    const int ss = span_status(t0, tfinal);
+    if (ss) { *nacc = 0; *natt = 0; return ss; }
     const double hmax = (tfinal - t0) / 2.5;
     double t = t0;
     const double hmin = (tfinal - t) / 1e7;
@@ -191,6 +202,8 @@ LTO_HD int drive_rk8(RHS& rhs, double* y, double t0, double tfinal, double atol,
     const double span = tfinal - t0;
     int na = 0, nt = 0, status = 0;
     *nacc = 0; *natt = 0;
+    const int ss = span_status(t0, tfinal);          // same span rule as drive_ode78
+    if (ss) return ss;
     // initial step: f0 -> k[0..NT), euler probe -> k[NT..2NT)
     int rs = rhs(y, k);
     if (rs) return rs;
